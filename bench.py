@@ -4,7 +4,7 @@
     full-res 1600x1200 dehaze images/sec at N B200s  (config 3: 1200x1600 image wrap-padded to 1664^2,
     cut into 169 tiles of 128x128, tiles sharded over the ranks, final all_gather of the outputs)
 
-    python bench.py --gpus N --steps K --warmup W [--dtype f32|bf16] [--impl ours|reference]
+    python bench.py --gpus N --steps K --warmup W [--dtype f32|bf16] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one full image.  `value` is measured with the image already resident in HBM, `e2e` through
 the public API from pinned HOST memory (H2D + D2H inside the timed region).  `roofline` is for the
@@ -252,8 +252,13 @@ def main():
                     help="images in flight per rank in the serving pipeline (fullres.TiledPipeline lanes: one CUDA graph and one "
                          "stream each; 1 = one forward at a time)")
     ap.add_argument("--no-train-step", action="store_true", help="skip the config 2 / 4 training-step measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the restored image of the last timed step to DIR/restored.npy (float32, 1 x 3 x 1200 x 1600); "
+                         "the inputs are seeded, so two builds run with the same arguments can be compared output for output")
     args = ap.parse_args()
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs needs --impl ours")
         return run_reference(args)
     args.warmup = max(args.warmup, 3)
 
@@ -344,6 +349,7 @@ def main():
     # N > 1: the rank's tile forward of image i+1 overlaps the all_gather + stitch of image i (fullres.TiledPipeline; same
     # kernels per image, bit-identical output - checked below before anything is timed); N == 1 has no collective to hide
     tpipes = {}
+    last_out = [None]
 
     def step_resident():
         dt = cur_dtype[0]
@@ -351,8 +357,10 @@ def main():
             if dt not in tpipes:
                 tpipes[dt] = fullres.TiledPipeline(model, graphed_lanes(dt), (1, 3, IMG_H, IMG_W), dev, ps=PS,
                                                    dtype=torch.bfloat16 if dt == "bf16" else torch.float32)
-            return tpipes[dt].submit(img_dev, idx)[0]
-        return forward(img_dev)
+            last_out[0] = tpipes[dt].submit(img_dev, idx)[0]
+        else:
+            last_out[0] = forward(img_dev)
+        return last_out[0]
 
     def finish_resident():
         for tp in tpipes.values():
@@ -407,6 +415,8 @@ def main():
             a = step_resident(); finish_resident(); torch.cuda.synchronize()
             assert torch.equal(a, want), "TiledPipeline differs from dehaze_tiled"
     ms_total = timed(step_resident, args.steps, finish=finish_resident)
+    # copied now: a pipeline slot is reused by the later passes
+    restored = last_out[0].float().cpu().numpy() if args.dump_outputs and rank == 0 else None
     launches = lib.lewin_launch_count() - n0
     if args.dtype in graphs:          # graph replay: the captured library launches run once per replay
         launches += graphs[args.dtype].launches_per_replay * args.steps
@@ -583,6 +593,10 @@ def main():
         "train_step": train,
         "kernels": kernels,
     }
+    if args.dump_outputs:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "restored.npy"), restored)
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()

@@ -1,9 +1,8 @@
 """Import the UNMODIFIED reference model (read-only, /root/reference) in the build container.
 
-TEST INFRASTRUCTURE ONLY (see oracle/lewin_oracle.py header).  /root/reference does not
-exist on the GPU box, so nothing that runs there may import this module; it is used by
-``oracle/make_golden.py`` and by the ``-m "not gpu"`` tests that are skipped when the
-reference tree is absent.
+TEST INFRASTRUCTURE ONLY (see oracle/lewin_oracle.py header).  The reference source is not part
+of this repository, so the package, the tests and the benchmark never import this module; only
+``oracle/make_golden.py`` uses it, and the tests read the fixtures it wrote.
 
 The reference needs ``timm.models.layers.{DropPath,to_2tuple,trunc_normal_}``
 (My_model_1.py:10); timm is not installed, so an in-memory shim provides the three

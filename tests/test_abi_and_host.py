@@ -154,25 +154,34 @@ def test_fullres_pad_tile_roundtrip():
     assert cover == list(range(169))
 
 
-@pytest.mark.needs_reference
-def test_patch_reference_model_structure():
-    from oracle import ref_shim
-    if not ref_shim.available():
-        pytest.skip("reference tree not mounted")
+def test_patch_reference_model_structure(golden_dir):
+    """patch() / unpatch() on a block with the reference's class names and module layout: the foreign stand-in of
+    tests/test_gpu_patch.py, whose state_dict must equal the reference's recorded layout of a shifted embed_dim 32 block."""
     import lewin_b200 as L
-    ref = ref_shim.import_reference()
-    blk = ref.LeWinTransformerBlock(dim=32, input_resolution=(128, 128), num_heads=1, win_size=8, shift_size=4,
-                                    token_mlp="leff")
+    from tests.test_gpu_patch import LeWinTransformerBlock
+    pre = "encoderlayer_0.blocks.1."
+    lines = open(os.path.join(golden_dir, "uformer32_state_dict_keys.txt")).read().strip().split("\n")
+    ref = {k[len(pre):]: v for k, v in (l.split(" ", 1) for l in lines) if k.startswith(pre)}
+    torch.manual_seed(0)
+    blk = LeWinTransformerBlock(32, 1, 4).eval()
+    assert {k: f"{tuple(v.shape)} {str(v.dtype).replace('torch.', '')}" for k, v in blk.state_dict().items()} == ref
+    x = torch.randn(1, 256, 32)
+    torch.manual_seed(1)
+    with torch.no_grad():
+        before = blk(x)
     keys = list(blk.state_dict().keys())
     L.patch(blk)
     assert list(blk.state_dict().keys()) == keys
     assert blk.forward.__func__.__name__ == "_block_forward"
     assert blk.attn.forward.__func__.__name__ == "_window_attention_forward"
+    assert blk.mlp.forward.__func__.__name__ == "_leff_forward"
     with pytest.raises(RuntimeError, match="no CPU fallback"):
         blk(torch.zeros(1, 256, 32))
     L.unpatch(blk)
-    out = blk(torch.zeros(1, 256, 32))          # reference forward restored, runs on CPU
-    assert out.shape == (1, 256, 32)
+    torch.manual_seed(1)
+    with torch.no_grad():
+        out = blk(x)                            # the block's own forward restored, runs on CPU
+    assert out.shape == (1, 256, 32) and torch.equal(out, before)
 
 
 def test_rows_needed_cover_each_ranks_tiles():

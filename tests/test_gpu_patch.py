@@ -5,7 +5,8 @@ attribute layout (My_model_1.py:336-415 WindowAttention, :477-534 LeFF, :738-875
 AttentionLayer) whose own forward is the torch restatement of the reference op sequence (oracle/torch_port.py, pinned to the
 reference's golden output by tests/test_oracle_golden.py) including the reference's own `torch.randint(64, (64, 25))` draw.
 patch() knows these modules only by class name - exactly how it meets the unmodified reference (tests/test_abi_and_host.py::
-test_patch_reference_model_structure does the structural half with the real classes where the reference is mounted).
+test_patch_reference_model_structure pins the stand-in's state_dict to the reference's recorded layout and does the structural
+half on the CPU).
 
 Checked: the patched forward runs the sm_100a kernels on the foreign module's OWN parameter objects, consumes the CPU RNG
 stream exactly like the foreign forward (same draw, same position), matches it within 1e-3 (fp32, north_star) with identical
@@ -33,6 +34,13 @@ class AttentionLayer(nn.Module):                       # attribute layout of Pro
         self.n_heads = n_heads
 
 
+class LinearProjection(nn.Module):                     # the reference's qkv module: separate q and kv linears
+    def __init__(self, dim):
+        super().__init__()
+        self.to_q = nn.Linear(dim, dim)
+        self.to_kv = nn.Linear(dim, 2 * dim)
+
+
 class WindowAttention(nn.Module):                      # My_model_1.py:346-398
     def __init__(self, dim, num_heads):
         super().__init__()
@@ -40,7 +48,7 @@ class WindowAttention(nn.Module):                      # My_model_1.py:346-398
         self.relative_position_bias_table = nn.Parameter(torch.randn(225, num_heads) * 0.3)
         self.register_buffer("relative_position_index", torch_port._rel_index().clone())
         self.ProbSpare = AttentionLayer(dim, num_heads)
-        self.qkv = nn.Linear(dim, 3 * dim)             # dead parameters of the reference, kept in its state_dict
+        self.qkv = LinearProjection(dim)               # dead parameters of the reference, kept in its state_dict
         self.proj = nn.Linear(dim, dim)
 
 
