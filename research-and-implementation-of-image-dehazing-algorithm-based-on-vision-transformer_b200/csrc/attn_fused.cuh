@@ -610,13 +610,8 @@ __global__ void __launch_bounds__(THREADS, 1) attn_fused_kernel(const Args a) {
     if (tid < 32) tc::tmem_dealloc<Cf::TMEM_COLS>(*tmem_slot);
 }
 
-inline bool enabled() {
-    static const bool on = [] { const char* e = getenv("LEWIN_NO_FUSED_ATTN"); return !(e && e[0] == '1'); }();
-    return on;
-}
-
 inline bool supported(int C, int nH, long long tokens) {
-    return enabled() && (C == 32 || C == 64) && C == nH * kHeadDim && tokens >= 4 * TM && tokens < (1ll << 31);
+    return (C == 32 || C == 64) && C == nH * kHeadDim && tokens >= 4 * TM && tokens < (1ll << 31);
 }
 
 template <int C>

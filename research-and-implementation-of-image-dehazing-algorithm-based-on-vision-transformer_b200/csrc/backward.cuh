@@ -806,10 +806,10 @@ cudaError_t launch_core_bwd_d(const CoreBwdArgs<T>& a, int num_sms, cudaStream_t
 template <typename T>
 cudaError_t launch_core_bwd(const CoreBwdArgs<T>& a, int num_sms, cudaStream_t stream) {
     const int D = a.C / a.nH;
-    if constexpr (Act<T>::kIsBf16) {
-        if (D == 32 && pcb2::enabled()) return pcb2::launch(a, num_sms, stream);      // register-resident bf16 path
+    if (D == 32) {
+        if constexpr (Act<T>::kIsBf16) return pcb2::launch(a, num_sms, stream);       // register-resident bf16 path
+        else return launch_core_bwd_d<T, 32>(a, num_sms, stream);
     }
-    if (D == 32) return launch_core_bwd_d<T, 32>(a, num_sms, stream);
     if (D == 64) return launch_core_bwd_d<T, 64>(a, num_sms, stream);
     if (D == 128) return launch_core_bwd_d<T, 128>(a, num_sms, stream);
     return cudaErrorInvalidValue;
@@ -884,26 +884,23 @@ template <typename T>
 inline cudaError_t launch_dgrad_gemm(const GemmArgs<T>& g, __nv_bfloat16* wT_bf16, int sms, cudaStream_t st,
                                      __nv_bfloat16* a_scratch = nullptr, bool* scratch_filled = nullptr) {
     if constexpr (Act<T>::kIsBf16) {
-        static const bool on = [] { const char* e = getenv("LEWIN_NO_WSS_DGRAD"); return !(e && e[0] == '1'); }();
-        static const int min_dim = [] { const char* e = getenv("LEWIN_WSS_DGRAD_MIN"); return e ? atoi(e) : 128; }();
-        if (on) {
-            GemmArgs<T> h = g;
-            const bool prepass = (g.mapA || g.a_row_scale) && a_scratch && !g.mean && g.K % 8 == 0 && g.M < (1ll << 31);
-            if (prepass) { h.A = a_scratch; h.lda = g.K; h.mapA = 0; h.a_row_scale = nullptr; }
-            const bool big = wT_bf16 && g.K >= min_dim && g.N >= min_dim && ws::wss_supported(h);   // streamed-W tcgen05 kernel
-            const bool small = !big && ws::plain_supported(h);                                      // resident-W warp-specialised kernel
-            if (big || small) {
-                if (prepass) {
-                    cudaError_t e = launch_scale_gather_rows(g.A, a_scratch, g.a_row_scale, g.M, g.K, g.lda, g.mapA, g.map,
-                                                             g.tokens_per_image, sms, st);
-                    if (e != cudaSuccess) return e;
-                    if (scratch_filled) *scratch_filled = true;   // [M, K] rows with the gather / DropPath scale applied
-                }
-                if (small) return ws::launch_plain(h, sms, st);
-                cudaError_t e = launch_convert_w(g.Wt, wT_bf16, static_cast<long long>(g.N) * g.K, st);
+        constexpr int min_dim = 128;
+        GemmArgs<T> h = g;
+        const bool prepass = (g.mapA || g.a_row_scale) && a_scratch && !g.mean && g.K % 8 == 0 && g.M < (1ll << 31);
+        if (prepass) { h.A = a_scratch; h.lda = g.K; h.mapA = 0; h.a_row_scale = nullptr; }
+        const bool big = wT_bf16 && g.K >= min_dim && g.N >= min_dim && ws::wss_supported(h);   // streamed-W tcgen05 kernel
+        const bool small = !big && ws::plain_supported(h);                                      // resident-W warp-specialised kernel
+        if (big || small) {
+            if (prepass) {
+                cudaError_t e = launch_scale_gather_rows(g.A, a_scratch, g.a_row_scale, g.M, g.K, g.lda, g.mapA, g.map,
+                                                         g.tokens_per_image, sms, st);
                 if (e != cudaSuccess) return e;
-                return ws::wss_launch<EPI_BIAS>(h, wT_bf16, sms, st);
+                if (scratch_filled) *scratch_filled = true;   // [M, K] rows with the gather / DropPath scale applied
             }
+            if (small) return ws::launch_plain(h, sms, st);
+            cudaError_t e = launch_convert_w(g.Wt, wT_bf16, static_cast<long long>(g.N) * g.K, st);
+            if (e != cudaSuccess) return e;
+            return ws::wss_launch<EPI_BIAS>(h, wT_bf16, sms, st);
         }
     }
     return launch_gemm_any<T, EPI_BIAS>(g, st);

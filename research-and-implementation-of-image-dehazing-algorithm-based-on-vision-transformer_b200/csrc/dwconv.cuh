@@ -517,17 +517,12 @@ bool launch_dwconv_bwd_tiled(const T* g2, const T* a2, const T* h1, const T* a1,
     if (H % 8 || W % 8 || Ch % SLAB) return false;
     const int slabs = Ch / SLAB;
     if (W % 16 == 0) {
-        const unsigned grid = static_cast<unsigned>(B) * (H / 8) * (W / 16) * slabs;
-        constexpr int smem16 = 2 * 10 * 18 * 128 + 9 * SLAB * 4 + kGeluTabSize * 2;
-        bool fast = false;
-        if constexpr (Act<T>::kIsBf16) {
-            if (dws::bwd_enabled() && dws::supported(H, W, Ch)) {      // element-wise dGELU + streaming TMA kernel (dwconv_stream.cuh)
-                *err = dws::launch_bwd_data(g2, a2, a1, da1, da2_scratch, w, B, H, W, Ch, num_sms, st);
-                if (*err != cudaSuccess) return true;
-                fast = true;
-            }
-        }
-        if (!fast) {
+        if constexpr (Act<T>::kIsBf16) {      // element-wise dGELU + streaming TMA kernel (dwconv_stream.cuh; dws::supported holds here)
+            *err = dws::launch_bwd_data(g2, a2, a1, da1, da2_scratch, w, B, H, W, Ch, num_sms, st);
+            if (*err != cudaSuccess) return true;
+        } else {
+            const unsigned grid = static_cast<unsigned>(B) * (H / 8) * (W / 16) * slabs;
+            constexpr int smem16 = 2 * 10 * 18 * 128 + 9 * SLAB * 4 + kGeluTabSize * 2;
             cudaFuncSetAttribute(dwconv_bwd_data_kernel<T, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem16);
             dwconv_bwd_data_kernel<T, 16><<<grid, 256, smem16, st>>>(g2, a2, a1, da1, da2_scratch, w, B, H, W, Ch);
         }
@@ -537,8 +532,7 @@ bool launch_dwconv_bwd_tiled(const T* g2, const T* a2, const T* h1, const T* a1,
         CUtensorMap hmap{}, dmap{};
         bool tma_done = false;
         if constexpr (Act<T>::kIsBf16) {
-            static const bool tma_on = [] { const char* e = getenv("LEWIN_NO_TMA"); return !(e && e[0] == '1'); }();
-            if (tma_on && tma::make_nhwc_bf16(&hmap, h1, B, H, W, Ch, 10, 18, SLAB) &&
+            if (tma::make_nhwc_bf16(&hmap, h1, B, H, W, Ch, 10, 18, SLAB) &&
                 tma::make_nhwc_bf16(&dmap, da2_scratch, B, H, W, Ch, 8, 16, SLAB)) {
                 constexpr int smem_tma = wg_smem16 + 128 /*alignment*/ + 16 /*mbarriers*/;
                 cudaFuncSetAttribute(dwconv_bwd_wgrad_kernel<T, 16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_tma);

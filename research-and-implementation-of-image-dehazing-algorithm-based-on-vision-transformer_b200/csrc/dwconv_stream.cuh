@@ -220,8 +220,7 @@ __global__ void __launch_bounds__(THREADS, 2) dwconv_stream_kernel(const Args a,
 // The code was removed in round 2; the conclusion stands: this kernel is bound by the GELU lookups' LSU traffic, not the MACs.
 
 inline bool supported(int H, int W, int Ch) {
-    static const bool on = [] { const char* e = getenv("LEWIN_NO_STREAM_DWCONV"); return !(e && e[0] == '1'); }();
-    return on && H >= 1 && W >= TX && W % 8 == 0 && Ch % SLAB == 0;   // any height; widths that are not a multiple of the tile are cut at the edge (an 8-wide map would waste half of every tile: first-generation kernel)
+    return H >= 1 && W >= TX && W % 8 == 0 && Ch % SLAB == 0;   // any height; widths that are not a multiple of the tile are cut at the edge (an 8-wide map would waste half of every tile: first-generation kernel)
 }
 
 template <bool BWD>
@@ -235,9 +234,8 @@ inline cudaError_t launch_mode(const __nv_bfloat16* x, __nv_bfloat16* out, __nv_
     a.total_tiles = a.spatial_tiles * (Ch / SLAB);
     int grid = 2 * num_sms;
     if (grid > a.total_tiles) grid = a.total_tiles;
-    static const bool tma_on = [] { const char* e = getenv("LEWIN_NO_TMA"); return !(e && e[0] == '1'); }();
     CUtensorMap map{};
-    if (tma_on && tma::make_nhwc_bf16(&map, x, B, H, W, Ch, HY, HX, SLAB)) {
+    if (tma::make_nhwc_bf16(&map, x, B, H, W, Ch, HY, HX, SLAB)) {
         cudaError_t e = cudaFuncSetAttribute(dwconv_stream_kernel<true, BWD>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(SMEM));
         if (e != cudaSuccess) return e;
         dwconv_stream_kernel<true, BWD><<<grid, THREADS, SMEM, stream>>>(a, map);
@@ -282,10 +280,6 @@ __global__ void __launch_bounds__(256) dgelu_mul_kernel(const __nv_bfloat16* __r
     }
 }
 
-inline bool bwd_enabled() {
-    static const bool on = [] { const char* e = getenv("LEWIN_NO_BWD2"); return !(e && e[0] == '1'); }();
-    return on;
-}
 inline cudaError_t launch_bwd_data(const __nv_bfloat16* g2, const __nv_bfloat16* a2, const __nv_bfloat16* a1, __nv_bfloat16* da1,
                                    __nv_bfloat16* da2, const float* w, int B, int H, int W, int Ch, int num_sms, cudaStream_t stream) {
     const long long n8 = static_cast<long long>(B) * H * W * Ch / 8;

@@ -4,11 +4,11 @@
 // attn.py:456 out projection, My_model_1.py:508 LeFF linear1, :529 LeFF linear2) with what surrounds
 // them in the reference folded in:
 //   prologue : LayerNorm (My_model_1.py:839/873) from precomputed row stats, cyclic shift +
-//              window_partition (My_model_1.py:846-852) as row addressing, bf16 rounding points;
+//              window_partition (My_model_1.py:846-852) as row addressing;
 //   epilogue : bias, exact GELU (My_model_1.py:487), DropPath scale + residual (My_model_1.py:872-873),
 //              window_reverse + un-shift (My_model_1.py:861-866) as row addressing.
-// Tensor cores: mma.sync m16n8k8 TF32, 3-pass error-compensated for fp32 activations (fp32-grade
-// accuracy), single pass for bf16 activations (bf16 operands are exact in TF32).
+// Tensor cores: mma.sync m16n8k8 TF32, 3-pass error-compensated (fp32-grade accuracy).  fp32 activations only: the bf16
+// GEMMs run on tcgen05 (gemm_tc.cuh, gemm_ws.cuh).
 #pragma once
 #include "common.cuh"
 
@@ -61,8 +61,10 @@ constexpr size_t gemm_smem_bytes() {
            sizeof(float) * 4 * GEMM_BM;
 }
 
+// T is always float; it stays a template parameter so that the kernel keeps the symbol name the profiles record
 template <typename T, int BN, int EPI>
 __global__ void __launch_bounds__(GEMM_THREADS) gemm_fused_kernel(const GemmArgs<T> g) {
+    static_assert(std::is_same<T, float>::value, "gemm_fused_kernel serves fp32 activations only");
     constexpr int PASSES = Act<T>::kPasses;
     constexpr int NT = BN / 16;    // n8-tiles per warp (warp covers BN/2 columns)
     constexpr int MT = 2;          // m16-tiles per warp (warp covers 32 rows)
@@ -135,10 +137,6 @@ __global__ void __launch_bounds__(GEMM_THREADS) gemm_fused_kernel(const GemmArgs
                     v.y = (v.y - mu) * rs * w.y + b.y;
                     v.z = (v.z - mu) * rs * w.z + b.z;
                     v.w = (v.w - mu) * rs * w.w + b.w;
-                    if (Act<T>::kIsBf16) {   // autocast: LN output (fp32) is cast to bf16 by the linear
-                        v.x = Act<T>::round(v.x); v.y = Act<T>::round(v.y);
-                        v.z = Act<T>::round(v.z); v.w = Act<T>::round(v.w);
-                    }
                 }
             }
             areg[i] = v;
@@ -191,8 +189,8 @@ __global__ void __launch_bounds__(GEMM_THREADS) gemm_fused_kernel(const GemmArgs
 #pragma unroll
             for (int j = 0; j < NT; ++j) {
                 const float* p = Wb + (j * 8 + gq) * GEMM_LDS + ks * 8 + tq;
-                bf[j][0] = Act<T>::round(p[0]);     // autocast casts the weight to bf16
-                bf[j][1] = Act<T>::round(p[4]);
+                bf[j][0] = p[0];
+                bf[j][1] = p[4];
             }
 #pragma unroll
             for (int i = 0; i < MT; ++i)
@@ -220,18 +218,16 @@ __global__ void __launch_bounds__(GEMM_THREADS) gemm_fused_kernel(const GemmArgs
                 const int col = n0 + warp_n * (BN / 2) + j * 8 + 2 * tq;
                 float v0 = acc[i][j][half * 2 + 0];
                 float v1 = acc[i][j][half * 2 + 1];
-                if (g.bias) { v0 += Act<T>::round(g.bias[col]); v1 += Act<T>::round(g.bias[col + 1]); }   // autocast casts the bias too
+                if (g.bias) { v0 += g.bias[col]; v1 += g.bias[col + 1]; }
                 if (EPI == EPI_MUL_GELUGRAD) {
                     const float2 pre = ld2(g.aux + oy + col);
                     v0 *= gelu_erf_grad(pre.x);
                     v1 *= gelu_erf_grad(pre.y);
                 } else if (EPI == EPI_BIAS_GELU) {
-                    if (Act<T>::kIsBf16) { v0 = Act<T>::round(v0); v1 = Act<T>::round(v1); }
                     if (g.Y2) st2(g.Y2 + oy + col, v0, v1);
                     v0 = gelu_erf(v0);
                     v1 = gelu_erf(v1);
                 } else if (EPI == EPI_BIAS_RESID) {
-                    if (Act<T>::kIsBf16) { v0 = Act<T>::round(v0); v1 = Act<T>::round(v1); }
                     float2 rr = ld2(g.R + oy + col);
                     v0 = rr.x + sc * v0;
                     v1 = rr.y + sc * v1;
@@ -293,19 +289,19 @@ __global__ void __launch_bounds__(256) ln_stats_kernel(const T* __restrict__ x, 
     }
 }
 
-template <typename T, int EPI>
-cudaError_t launch_gemm(const GemmArgs<T>& g, cudaStream_t stream) {
+template <int EPI>
+cudaError_t launch_gemm(const GemmArgs<float>& g, cudaStream_t stream) {
     dim3 block(GEMM_THREADS);
     const unsigned gm = static_cast<unsigned>((g.M + GEMM_BM - 1) / GEMM_BM);
     if (g.N % 64 == 0) {
         constexpr size_t smem = gemm_smem_bytes<64>();
-        auto k = gemm_fused_kernel<T, 64, EPI>;
+        auto k = gemm_fused_kernel<float, 64, EPI>;
         cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
         if (e != cudaSuccess) return e;
         k<<<dim3(gm, g.N / 64), block, smem, stream>>>(g);
     } else {
         constexpr size_t smem = gemm_smem_bytes<32>();
-        auto k = gemm_fused_kernel<T, 32, EPI>;
+        auto k = gemm_fused_kernel<float, 32, EPI>;
         cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
         if (e != cudaSuccess) return e;
         k<<<dim3(gm, g.N / 32), block, smem, stream>>>(g);

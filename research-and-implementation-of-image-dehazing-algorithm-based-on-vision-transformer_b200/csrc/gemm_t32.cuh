@@ -39,11 +39,6 @@ constexpr int STG_BUF = 32 * STG_ROW;
 constexpr int NTAB = 8;                       // per-tile row tables in flight (the A loads run up to DA tiles ahead of the convert)
 constexpr int SMEM_MAX = 227 * 1024;
 
-inline bool enabled() {
-    static const bool on = [] { const char* e = getenv("LEWIN_NO_T32_GEMM"); return !(e && e[0] == '1'); }();
-    return on;
-}
-
 #ifdef LEWIN_T32_PROF_BUILD
 // Diagnostic build (-DLEWIN_T32_PROF_BUILD, run with LEWIN_T32_PROF=1): per-role cycle counters, launch i since the last
 // reset counts into slot i % 8:  [0] producer total  [1] producer table barrier  [2] producer wait-for-free-stage
@@ -511,7 +506,7 @@ cudaError_t launch_bn(const GemmArgs<float>& g, int num_sms, cudaStream_t stream
 // forward-pass shapes of the LeWin block: K, N multiples of 32, 16-byte aligned rows, no backward-only prologues
 template <int EPI>
 inline bool supported(const GemmArgs<float>& g) {
-    if (!enabled() || g.a_row_scale || g.aux || g.up2) return false;
+    if (g.a_row_scale || g.aux || g.up2) return false;
     if (EPI != EPI_BIAS && EPI != EPI_BIAS_GELU && EPI != EPI_BIAS_RESID) return false;
     if (EPI == EPI_BIAS_RESID && !g.R) return false;
     if (g.K % 32 || g.N % 32 || g.M <= 0 || g.M >= (1ll << 31)) return false;
@@ -522,9 +517,8 @@ inline bool supported(const GemmArgs<float>& g) {
 
 template <int EPI>
 cudaError_t launch(const GemmArgs<float>& g, int num_sms, cudaStream_t stream) {
-    static const bool wide = [] { const char* e = getenv("LEWIN_T32_NO_BN256"); return !(e && e[0] == '1'); }();
     // tensor-bound shapes (long K): 256-wide tiles halve the A traffic per FLOP; two 96 KB stages
-    if (wide && g.N % 256 == 0 && g.K >= 128 && (g.M + BM - 1) / BM * (g.N / 256) >= num_sms) return launch_bn<256, EPI>(g, num_sms, stream);
+    if (g.N % 256 == 0 && g.K >= 128 && (g.M + BM - 1) / BM * (g.N / 256) >= num_sms) return launch_bn<256, EPI>(g, num_sms, stream);
     if (g.N % 128 == 0) return launch_bn<128, EPI>(g, num_sms, stream);
     if (g.N % 96 == 0) return launch_bn<96, EPI>(g, num_sms, stream);
     if (g.N % 64 == 0) return launch_bn<64, EPI>(g, num_sms, stream);

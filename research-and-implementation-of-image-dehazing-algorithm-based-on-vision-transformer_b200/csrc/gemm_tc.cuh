@@ -754,21 +754,13 @@ cudaError_t launch_gemm_tca_st(const GemmArgs<__nv_bfloat16>& g, const __nv_bflo
     return cudaGetLastError();
 }
 
-template <int BN, int EPI>
-cudaError_t launch_gemm_tca_bn(const GemmArgs<__nv_bfloat16>& g, const __nv_bfloat16* Wb, cudaStream_t stream) {
-    static const int deep = [] { const char* e = getenv("LEWIN_TCA_STAGES"); return e ? atoi(e) : 2; }();
-    if (deep >= 4 && g.K >= 256) return launch_gemm_tca_st<BN, 4, EPI>(g, Wb, stream);
-    if (deep == 3 && g.K >= 192) return launch_gemm_tca_st<BN, 3, EPI>(g, Wb, stream);
-    return launch_gemm_tca_st<BN, 2, EPI>(g, Wb, stream);
-}
-
-// plain-bf16-operand GEMM (K % 64 == 0, no LayerNorm prologue): Wb = bf16 copy of g.Wt
+// plain-bf16-operand GEMM (K % 64 == 0, no LayerNorm prologue): Wb = bf16 copy of g.Wt; two cp.async stages
 template <int EPI>
 cudaError_t launch_gemm_tca(const GemmArgs<__nv_bfloat16>& g, const __nv_bfloat16* Wb, cudaStream_t stream) {
-    if (g.N % 256 == 0) return launch_gemm_tca_bn<256, EPI>(g, Wb, stream);
-    if (g.N % 192 == 0) return launch_gemm_tca_bn<192, EPI>(g, Wb, stream);
-    if (g.N % 128 == 0) return launch_gemm_tca_bn<128, EPI>(g, Wb, stream);
-    return launch_gemm_tca_bn<64, EPI>(g, Wb, stream);
+    if (g.N % 256 == 0) return launch_gemm_tca_st<256, 2, EPI>(g, Wb, stream);
+    if (g.N % 192 == 0) return launch_gemm_tca_st<192, 2, EPI>(g, Wb, stream);
+    if (g.N % 128 == 0) return launch_gemm_tca_st<128, 2, EPI>(g, Wb, stream);
+    return launch_gemm_tca_st<64, 2, EPI>(g, Wb, stream);
 }
 
 template <int BN, int KC, int EPI, int STAGES>
@@ -793,8 +785,7 @@ inline int tc_num_sms() {
 
 template <int BN, int KC, int EPI>
 cudaError_t launch_gemm_tc_inst(const GemmArgs<__nv_bfloat16>& g, cudaStream_t stream) {
-    static const bool persist = [] { const char* e = getenv("LEWIN_NO_PERSIST_GEMM"); return !(e && e[0] == '1'); }();
-    if (persist && g.M >= 4 * TC_BM) {
+    if (g.M >= 4 * TC_BM) {
         if (g.K == KC) return launch_gemm_tcp<BN, KC, 1, EPI>(g, tc_num_sms(), stream);
         if (g.K == 2 * KC) return launch_gemm_tcp<BN, KC, 2, EPI>(g, tc_num_sms(), stream);
     }
@@ -806,11 +797,8 @@ template <int KC, int EPI>
 cudaError_t launch_gemm_tc_kc(const GemmArgs<__nv_bfloat16>& g, cudaStream_t stream) {
     const int N = g.N;
     // wide (192/256-column, 256-thread) tiles measured faster than 128-column / 128-thread tiles on every shape
-    static const bool wide = [] { const char* e = getenv("LEWIN_TC_NARROW"); return !(e && e[0] == '1'); }();
-    if (wide) {
-        if (N % 256 == 0) return launch_gemm_tc_inst<256, KC, EPI>(g, stream);
-        if (N % 192 == 0) return launch_gemm_tc_inst<192, KC, EPI>(g, stream);
-    }
+    if (N % 256 == 0) return launch_gemm_tc_inst<256, KC, EPI>(g, stream);
+    if (N % 192 == 0) return launch_gemm_tc_inst<192, KC, EPI>(g, stream);
     if (N % 128 == 0) return launch_gemm_tc_inst<128, KC, EPI>(g, stream);
     if (N % 96 == 0) return launch_gemm_tc_inst<96, KC, EPI>(g, stream);
     if (N % 64 == 0) return launch_gemm_tc_inst<64, KC, EPI>(g, stream);
@@ -824,21 +812,16 @@ cudaError_t launch_gemm_tc(const GemmArgs<__nv_bfloat16>& g, cudaStream_t stream
     return launch_gemm_tc_kc<32, EPI>(g, stream);
 }
 
-// Dispatch used by the ABI: fp32 activations -> 3xTF32 mma.sync kernel; bf16 activations -> tcgen05 kernel
-// (LEWIN_NO_TCGEN05=1 in the environment selects the mma.sync kernel for A/B comparison).
-inline bool tcgen05_enabled() {
-    static const bool on = [] { const char* e = getenv("LEWIN_NO_TCGEN05"); return !(e && e[0] == '1'); }();
-    return on;
-}
+// Dispatch used by the ABI: bf16 activations -> tcgen05 kernel; fp32 activations -> 3xTF32 on tcgen05 (gemm_t32.cuh) for
+// the forward shapes, the 3xTF32 mma.sync kernel otherwise
 template <typename T, int EPI>
 cudaError_t launch_gemm_any(const GemmArgs<T>& g, cudaStream_t stream) {
     if constexpr (Act<T>::kIsBf16) {
-        if (tcgen05_enabled()) return launch_gemm_tc<EPI>(g, stream);
+        return launch_gemm_tc<EPI>(g, stream);
     } else {
-        // fp32: 3xTF32 on tcgen05 (gemm_t32.cuh) for the forward shapes; mma.sync kernel otherwise
         if (gemm_t32_supported(g, EPI)) return gemm_t32_launch(g, EPI, stream);
+        return launch_gemm<EPI>(g, stream);
     }
-    return launch_gemm<T, EPI>(g, stream);
 }
 
 }  // namespace lewin

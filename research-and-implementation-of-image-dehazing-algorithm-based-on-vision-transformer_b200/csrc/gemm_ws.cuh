@@ -46,11 +46,6 @@ __device__ __forceinline__ void unpack8(const uint4& u, float (&f)[8]) {
 }
 
 
-inline bool enabled() {
-    static const bool on = [] { const char* e = getenv("LEWIN_NO_WS_GEMM"); return !(e && e[0] == '1'); }();
-    return on;
-}
-
 // packed fp32x2 arithmetic (one issue slot for two lanes of work; same IEEE rounding as the scalar instructions)
 __device__ __forceinline__ float2 add2(const float2 a, const float2 b) {
     unsigned long long d;
@@ -565,8 +560,7 @@ cudaError_t launch_inst(const GemmArgs<__nv_bfloat16>& g, int num_sms, cudaStrea
     if (gx < 1) gx = 1;
     if (gx > row_tiles) gx = row_tiles;
     CUtensorMap ymap{};
-    static const bool tma_store = [] { const char* e = getenv("LEWIN_NO_TMA_STORE"); return !(e && e[0] == '1'); }();
-    const int use_ymap = (tma_store && EPI != EPI_BIAS_RESID && !g.mapY && !g.up2 && (g.ldy % 8) == 0 &&
+    const int use_ymap = (EPI != EPI_BIAS_RESID && !g.mapY && !g.up2 && (g.ldy % 8) == 0 &&
                           tma::make_2d_bf16_store32(&ymap, g.Y, g.M, g.N, g.ldy)) ? 1 : 0;
     k<<<dim3(gx, col_tiles), THREADS, smem, stream>>>(g, row_tiles, nkc, S, ymap, use_ymap);
     return cudaGetLastError();
@@ -712,8 +706,7 @@ cudaError_t wss_launch_bn(const GemmArgs<__nv_bfloat16>& g, const __nv_bfloat16*
     int grid = num_sms;
     if (grid > row_tiles * col_tiles) grid = row_tiles * col_tiles;
     CUtensorMap ymap{};
-    static const bool tma_store = [] { const char* e = getenv("LEWIN_NO_TMA_STORE"); return !(e && e[0] == '1'); }();
-    const int use_ymap = (tma_store && EPI != EPI_BIAS_RESID && !g.mapY && !g.up2 && (g.ldy % 8) == 0 &&
+    const int use_ymap = (EPI != EPI_BIAS_RESID && !g.mapY && !g.up2 && (g.ldy % 8) == 0 &&
                           tma::make_2d_bf16_store32(&ymap, g.Y, g.M, g.N, g.ldy)) ? 1 : 0;
     k<<<grid, WssCfg<EPI>::THREADS, smem, stream>>>(g, amap, wmap, row_tiles, col_tiles, g.K / 64, S, ymap, use_ymap);
     return cudaGetLastError();
@@ -721,8 +714,7 @@ cudaError_t wss_launch_bn(const GemmArgs<__nv_bfloat16>& g, const __nv_bfloat16*
 
 // plain bf16 operands, K % 64 == 0, N % 128 == 0, no A-row gather / scale (callers fall back to gemm_tca otherwise)
 inline bool wss_supported(const GemmArgs<__nv_bfloat16>& g) {
-    static const bool on = [] { const char* e = getenv("LEWIN_NO_WSS_GEMM"); return !(e && e[0] == '1'); }();
-    return on && enabled() && !g.mapA && !g.a_row_scale && !g.aux && !g.mean && g.K % 64 == 0 && g.N % 128 == 0 && g.N <= 4096 &&
+    return !g.mapA && !g.a_row_scale && !g.aux && !g.mean && g.K % 64 == 0 && g.N % 128 == 0 && g.N <= 4096 &&
            (g.M >= 4 * TC_BM || g.up2) && (g.lda % 8) == 0 && tma::encode_fn() != nullptr;
 }
 // Tile width by occupancy: the widest BN whose tile count still fills the SMs.  At the deep levels of a small tile shard
@@ -731,9 +723,8 @@ inline bool wss_supported(const GemmArgs<__nv_bfloat16>& g) {
 template <int EPI>
 cudaError_t wss_launch(const GemmArgs<__nv_bfloat16>& g, const __nv_bfloat16* Wb, int num_sms, cudaStream_t stream) {
     const long long row_tiles = (g.M + TC_BM - 1) / TC_BM;
-    static const bool narrow = [] { const char* e = getenv("LEWIN_NO_NARROW_WSS"); return !(e && e[0] == '1'); }();
-    if (g.N % 256 == 0 && (!narrow || row_tiles * (g.N / 256) >= num_sms)) return wss_launch_bn<256, EPI>(g, Wb, num_sms, stream);
-    if (!narrow || row_tiles * (g.N / 128) >= num_sms || g.up2) return wss_launch_bn<128, EPI>(g, Wb, num_sms, stream);
+    if (g.N % 256 == 0 && row_tiles * (g.N / 256) >= num_sms) return wss_launch_bn<256, EPI>(g, Wb, num_sms, stream);
+    if (row_tiles * (g.N / 128) >= num_sms || g.up2) return wss_launch_bn<128, EPI>(g, Wb, num_sms, stream);
     return wss_launch_bn<64, EPI>(g, Wb, num_sms, stream);
 }
 
@@ -744,7 +735,7 @@ cudaError_t wss_launch(const GemmArgs<__nv_bfloat16>& g, const __nv_bfloat16* Wb
 //   EPI_BIAS_RESID      (out, linear2): N = C in {32, 64, 128}, K in {C, 4C}
 template <int EPI>
 inline bool supported(const GemmArgs<__nv_bfloat16>& g, bool ln) {
-    if (!enabled() || g.a_row_scale || g.aux) return false;
+    if (g.a_row_scale || g.aux) return false;
     if (g.M < 4 * TC_BM) return false;
     if (ln) {
         if (!(g.K == 32 || g.K == 64 || g.K == 128)) return false;
@@ -778,7 +769,7 @@ cudaError_t launch(const GemmArgs<__nv_bfloat16>& g, bool ln, int num_sms, cudaS
 // Plain bf16 operand, no LayerNorm, bias-only epilogue (optionally scattered through window_reverse + un-roll): the
 // data-gradient GEMMs dX = dY . W of the C <= 64 levels (N in {32, 64} or the 4C-wide dh2), weights resident in shared memory.
 inline bool plain_supported(const GemmArgs<__nv_bfloat16>& g) {
-    if (!enabled() || g.mapA || g.a_row_scale || g.aux || g.mean || g.up2 || g.Y2 || g.R) return false;
+    if (g.mapA || g.a_row_scale || g.aux || g.mean || g.up2 || g.Y2 || g.R) return false;
     if (g.M < 4 * TC_BM || (g.lda % 8) || (g.ldy % 8)) return false;
     if (g.N == 32) return g.K % 32 == 0 && g.K <= 256;
     if (g.N == 64) return g.K % 64 == 0 && g.K <= 512;

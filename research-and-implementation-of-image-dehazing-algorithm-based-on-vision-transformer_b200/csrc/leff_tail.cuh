@@ -331,13 +331,8 @@ __global__ void __launch_bounds__(THREADS, 1) leff_tail_kernel(const Args a, con
     if (warp == 0) tc::tmem_dealloc<Cf::TMEM_COLS>(tmem0);
 }
 
-inline bool enabled() {
-    static const bool on = [] { const char* e = getenv("LEWIN_NO_LEFF_TAIL"); return !(e && e[0] == '1'); }();
-    return on;
-}
-
 inline bool supported(int C, int hidden, int B, int H, int W) {
-    return enabled() && (C == 32 || C == 64) && hidden == 4 * C && W % TX == 0 && H >= 1 &&
+    return (C == 32 || C == 64) && hidden == 4 * C && W % TX == 0 && H >= 1 &&
            static_cast<long long>(B) * H * W >= 4 * 128 && tma::encode_fn() != nullptr;
 }
 

@@ -8,7 +8,6 @@
 #include "gemm_tc.cuh"
 #include "gemm_ws.cuh"
 #include "probsparse_core.cuh"
-#include "probsparse_core_bf16.cuh"
 #include "probsparse_core_v3.cuh"
 #include "backward.cuh"
 #include "attn_fused_api.h"
@@ -36,16 +35,13 @@ inline int device_info(DeviceInfo* d) {
     return d->cc_major == 10 ? 0 : LEWIN_E_ARCH;
 }
 
-std::atomic<long long> g_launches{0};
+std::atomic<long long> g_launches{0};   // diagnostic only (lewin_launch_count)
 
-inline int async_min_c() {   // channels above which the bf16 GEMMs take the async (cp.async ring) kernel
-    static const int v = [] { const char* e = getenv("LEWIN_ASYNC_MIN_C"); return e ? atoi(e) : 128; }();
-    return v;
-}   // diagnostic only (lewin_launch_count)
+constexpr int kAsyncMinC = 128;   // channels above which the bf16 GEMMs take the streamed-W kernels on pre-converted weights
 
 // Which kernels a forward call will run (shared by the launch code and the kernel-mask queries).
 inline bool ws_level(int C, long long tokens) {     // warp-specialised persistent GEMM (gemm_ws.cuh) serves this level
-    return ws::enabled() && (C == 32 || C == 64 || C == 128) && tokens >= 4 * TC_BM;
+    return (C == 32 || C == 64 || C == 128) && tokens >= 4 * TC_BM;
 }
 struct AttnPlan { bool fused, async_gemm, ws_gemm, ln_stats; };
 inline AttnPlan plan_attn(const LewinAttnFwdArgs* a, bool bf) {
@@ -54,7 +50,7 @@ inline AttnPlan plan_attn(const LewinAttnFwdArgs* a, bool bf) {
     p.fused = bf && attn_fused_supported(a);            // the whole half as one kernel (attn_fused.cuh): inference, C <= 64
     if (p.fused) return p;
     p.ws_gemm = bf && !a->windowed && ws_level(a->C, tokens);
-    p.async_gemm = bf && !p.ws_gemm && a->C > async_min_c() && a->C % 64 == 0 && !getenv("LEWIN_NO_ASYNC_GEMM");
+    p.async_gemm = bf && !p.ws_gemm && a->C > kAsyncMinC && a->C % 64 == 0;
     p.ln_stats = !a->windowed && !p.async_gemm && !p.ws_gemm;
     return p;
 }
@@ -75,6 +71,22 @@ struct KTimer {
         cudaError_t _e = (expr);                         \
         if (_e != cudaSuccess) return static_cast<int>(_e); \
     } while (0)
+
+// One linear of a forward call on the kernel its plan chose.  ws_gemm: the warp-specialised GEMM with resident weights,
+// which computes the LayerNorm statistics itself when the linear has a LayerNorm prologue (g.mean set).  Wb: the streamed-W
+// GEMM on that pre-converted bf16 weight (gemm_tca where wss_supported rules the shape out).  Otherwise the generic dispatch.
+template <int EPI, typename T>
+cudaError_t launch_linear(GemmArgs<T> g, bool ws_gemm, const __nv_bfloat16* Wb, int sms, cudaStream_t st) {
+    if constexpr (Act<T>::kIsBf16) {
+        if (ws_gemm) {
+            const bool ln = g.mean != nullptr;
+            g.mean = nullptr; g.rstd = nullptr;
+            return ws::launch<EPI>(g, ln, sms, st);
+        }
+        if (Wb) return ws::wss_supported(g) ? ws::wss_launch<EPI>(g, Wb, sms, st) : launch_gemm_tca<EPI>(g, Wb, st);
+    }
+    return launch_gemm_any<T, EPI>(g, st);
+}
 
 // ------------------------------------------------------------------ attention forward
 int check_attn(const LewinAttnFwdArgs* a) {
@@ -141,11 +153,9 @@ int attn_fwd(const LewinAttnFwdArgs* a, void* ws, size_t ws_bytes, cudaStream_t 
         CK(launch_ln_stats<T>(x, tokens, C, mean, rstd, stream));
         kt.end(LEWIN_ATTN_K_LNSTATS);
     }
-    bool async_gemm = false;
     __nv_bfloat16* xhat = nullptr; __nv_bfloat16* wqkv_b = nullptr; __nv_bfloat16* wout_b = nullptr;
     if constexpr (Act<T>::kIsBf16) {
-        async_gemm = plan.async_gemm;
-        if (async_gemm) {
+        if (plan.async_gemm) {
             unsigned char* q = ws_gemm;
             xhat = reinterpret_cast<__nv_bfloat16*>(q); q += align_up(static_cast<size_t>(tokens) * C * 2, 256);
             wqkv_b = reinterpret_cast<__nv_bfloat16*>(q);
@@ -170,21 +180,12 @@ int attn_fwd(const LewinAttnFwdArgs* a, void* ws, size_t ws_bytes, cudaStream_t 
         g.tokens_per_image = a->H * a->W;
         kt.begin(LEWIN_ATTN_K_QKV);
         if constexpr (Act<T>::kIsBf16) {
-            if (plan.ws_gemm) {          // LN1 statistics computed inside the GEMM's producer warps
-                g.mean = nullptr; g.rstd = nullptr;
-                CK((ws::launch<EPI_BIAS>(g, true, di.sms, stream)));
-            } else if (async_gemm) {
-                if (!a->windowed) {      // LN1 + roll + partition in one pre-pass; the GEMM then streams plain bf16 rows
-                    CK(launch_ln_apply(static_cast<const __nv_bfloat16*>(a->x), xhat, a->ln_w, a->ln_b, tokens, C, 1, map, stream));
-                    g.A = xhat; g.mapA = 0; g.mean = nullptr; g.rstd = nullptr;
-                }
-                CK(((ws::wss_supported(g) ? ws::wss_launch<EPI_BIAS>(g, wqkv_b, di.sms, stream) : launch_gemm_tca<EPI_BIAS>(g, wqkv_b, stream))));
-            } else {
-                CK((launch_gemm_any<T, EPI_BIAS>(g, stream)));
+            if (plan.async_gemm && !a->windowed) {      // LN1 + roll + partition in one pre-pass; the GEMM then streams plain bf16 rows
+                CK(launch_ln_apply(static_cast<const __nv_bfloat16*>(a->x), xhat, a->ln_w, a->ln_b, tokens, C, 1, map, stream));
+                g.A = xhat; g.mapA = 0; g.mean = nullptr; g.rstd = nullptr;
             }
-        } else {
-            CK((launch_gemm_any<T, EPI_BIAS>(g, stream)));
         }
+        CK(launch_linear<EPI_BIAS>(g, plan.ws_gemm, wqkv_b, di.sms, stream));
         kt.end(LEWIN_ATTN_K_QKV);
     }
     {   // ProbSparse core (attn.py:287-342)
@@ -202,20 +203,7 @@ int attn_fwd(const LewinAttnFwdArgs* a, void* ws, size_t ws_bytes, cudaStream_t 
         c.H = a->H; c.W = a->W; c.nWw = a->W / 8; c.nWin = nWin;
         c.y0 = a->band_mode ? a->band_y0 : 0; c.Hg = a->band_mode ? a->band_Hg : a->H;
         kt.begin(LEWIN_ATTN_K_CORE);
-        if constexpr (Act<T>::kIsBf16) {
-            if (C == a->nH * kHeadDim && pc3::enabled()) {       // head_dim 32: register-resident kernel
-                CoreBf16Args b{};
-                b.qkv = c.qkv; b.ctx = c.ctx; b.top = c.top; b.rpb_table = c.rpb_table; b.rpb_dense = c.rpb_dense;
-                b.index_sample = c.index_sample;
-                b.mask = c.mask; b.nW_mask = c.nW_mask; b.B_ = c.B_; b.nH = c.nH; b.C = c.C; b.use_rpb = c.use_rpb;
-                b.shift = c.shift; b.H = c.H; b.W = c.W; b.nWw = c.nWw; b.nWin = c.nWin; b.y0 = c.y0; b.Hg = c.Hg;
-                CK(pc3::launch(b, di.sms, stream));
-            } else {
-                CK(launch_core_fwd<T>(c, di.sms, stream));
-            }
-        } else {
-            CK(launch_core_fwd<T>(c, di.sms, stream));
-        }
+        CK(launch_core_fwd<T>(c, di.sms, stream));
         kt.end(LEWIN_ATTN_K_CORE);
     }
     {   // out projection (attn.py:456) + window_reverse + un-roll + DropPath scale + residual
@@ -227,25 +215,11 @@ int attn_fwd(const LewinAttnFwdArgs* a, void* ws, size_t ws_bytes, cudaStream_t 
         g.mapA = 0; g.mapY = a->windowed ? 0 : 1; g.map = map;
         g.tokens_per_image = a->H * a->W;
         kt.begin(LEWIN_ATTN_K_OUT);
-        bool done = false;
-        if constexpr (Act<T>::kIsBf16) {
-            if (plan.ws_gemm) {
-                g.R = x; g.drop_scale = a->drop_scale;
-                CK((ws::launch<EPI_BIAS_RESID>(g, false, di.sms, stream)));
-                done = true;
-            } else if (async_gemm) {
-                if (a->windowed) { CK(((ws::wss_supported(g) ? ws::wss_launch<EPI_BIAS>(g, wout_b, di.sms, stream) : launch_gemm_tca<EPI_BIAS>(g, wout_b, stream)))); }
-                else { g.R = x; g.drop_scale = a->drop_scale; CK(((ws::wss_supported(g) ? ws::wss_launch<EPI_BIAS_RESID>(g, wout_b, di.sms, stream) : launch_gemm_tca<EPI_BIAS_RESID>(g, wout_b, stream)))); }
-                done = true;
-            }
-        }
-        if (!done) {
-            if (a->windowed) {
-                CK((launch_gemm_any<T, EPI_BIAS>(g, stream)));
-            } else {
-                g.R = x; g.drop_scale = a->drop_scale;
-                CK((launch_gemm_any<T, EPI_BIAS_RESID>(g, stream)));
-            }
+        if (a->windowed) {
+            CK(launch_linear<EPI_BIAS>(g, plan.ws_gemm, wout_b, di.sms, stream));
+        } else {
+            g.R = x; g.drop_scale = a->drop_scale;
+            CK(launch_linear<EPI_BIAS_RESID>(g, plan.ws_gemm, wout_b, di.sms, stream));
         }
         kt.end(LEWIN_ATTN_K_OUT);
     }
@@ -282,19 +256,7 @@ int core_only_fwd(const LewinCoreFwdArgs* a, void*, size_t, cudaStream_t stream)
     c.B_ = a->B_; c.nH = a->nH; c.C = a->nH * D;
     c.use_rpb = a->use_rpb;
     c.shift = 0; c.H = 8; c.W = 8; c.nWw = 1; c.nWin = 1; c.y0 = 0; c.Hg = 8;
-    bool done = false;
-    if constexpr (Act<T>::kIsBf16) {
-        if (D == kHeadDim && pc3::enabled()) {
-            CoreBf16Args b{};
-            b.qkv = c.qkv; b.ctx = c.ctx; b.top = c.top; b.rpb_table = c.rpb_table; b.rpb_dense = c.rpb_dense;
-            b.index_sample = c.index_sample;
-            b.mask = c.mask; b.nW_mask = c.nW_mask; b.B_ = c.B_; b.nH = c.nH; b.C = c.C; b.use_rpb = c.use_rpb;
-            b.shift = 0; b.H = 8; b.W = 8; b.nWw = 1; b.nWin = 1; b.y0 = 0; b.Hg = 8;
-            CK(pc3::launch(b, di.sms, stream));
-            done = true;
-        }
-    }
-    if (!done) CK(launch_core_fwd<T>(c, di.sms, stream));
+    CK(launch_core_fwd<T>(c, di.sms, stream));
     g_launches.fetch_add(1, std::memory_order_relaxed);
     return 0;
 }
@@ -357,8 +319,7 @@ inline LeffPlan plan_leff(const LewinLeffFwdArgs* a, bool bf) {
     LeffPlan p{};
     const long long tokens = static_cast<long long>(a->B) * a->H * a->W;
     p.ws_gemm = bf && a->fused && a->hidden == 4 * a->C && ws_level(a->C, tokens);
-    p.async_gemm = bf && !p.ws_gemm && a->C > async_min_c() && a->C % 64 == 0 && a->hidden % 64 == 0 &&
-                   !getenv("LEWIN_NO_ASYNC_GEMM");
+    p.async_gemm = bf && !p.ws_gemm && a->C > kAsyncMinC && a->C % 64 == 0 && a->hidden % 64 == 0;
     p.ln_stats = a->fused && !p.async_gemm && !p.ws_gemm;
     p.tail = bf && p.ws_gemm && leff_tail_supported(a);      // dwconv + GELU + linear2 + residual in one kernel (leff_tail.cuh)
     return p;
@@ -396,11 +357,9 @@ int leff_fwd(const LewinLeffFwdArgs* a, void* ws, size_t ws_bytes, cudaStream_t 
     if (!leff_ld_out_ok(a, plan)) return LEWIN_E_SHAPE;
     const long long ldo = a->ld_out > 0 ? a->ld_out : a->C;
     if constexpr (Act<T>::kIsBf16) CK(launch_gelu_tab_init(stream));     // idempotent 8 KB table (common.cuh)
-    bool async_gemm = false;
     __nv_bfloat16* xhat = nullptr; __nv_bfloat16* w1b = nullptr; __nv_bfloat16* w2b = nullptr;
     if constexpr (Act<T>::kIsBf16) {
-        async_gemm = plan.async_gemm;
-        if (async_gemm) {
+        if (plan.async_gemm) {
             unsigned char* q = wsp + 2 * align_up(tokens * sizeof(float), 256);
             xhat = reinterpret_cast<__nv_bfloat16*>(q); q += align_up(static_cast<size_t>(tokens) * C * 2, 256);
             w1b = reinterpret_cast<__nv_bfloat16*>(q);
@@ -428,23 +387,14 @@ int leff_fwd(const LewinLeffFwdArgs* a, void* ws, size_t ws_bytes, cudaStream_t 
         if (a->fused) { g.mean = mean; g.rstd = rstd; g.ln_w = a->ln_w; g.ln_b = a->ln_b; }
         g.tokens_per_image = a->H * a->W;
         kt.begin(LEWIN_LEFF_K_FC1);
-        bool done1 = false;
         if constexpr (Act<T>::kIsBf16) {
-            if (plan.ws_gemm) {          // LN2 statistics computed inside the GEMM's producer warps
-                g.mean = nullptr; g.rstd = nullptr;
-                CK((ws::launch<EPI_BIAS_GELU>(g, true, di.sms, stream)));
-                done1 = true;
-            } else if (async_gemm) {
-                if (a->fused) {
-                    WinMap nomap{a->H, a->W, a->W / 8, (a->H / 8) * (a->W / 8), 0, 0};
-                    CK(launch_ln_apply(static_cast<const __nv_bfloat16*>(a->y), xhat, a->ln_w, a->ln_b, tokens, C, 0, nomap, stream));
-                    g.A = xhat; g.mean = nullptr; g.rstd = nullptr;
-                }
-                CK(((ws::wss_supported(g) ? ws::wss_launch<EPI_BIAS_GELU>(g, w1b, di.sms, stream) : launch_gemm_tca<EPI_BIAS_GELU>(g, w1b, stream))));
-                done1 = true;
+            if (plan.async_gemm && a->fused) {          // LN2 in one pre-pass; the GEMM then streams plain bf16 rows
+                WinMap nomap{a->H, a->W, a->W / 8, (a->H / 8) * (a->W / 8), 0, 0};
+                CK(launch_ln_apply(static_cast<const __nv_bfloat16*>(a->y), xhat, a->ln_w, a->ln_b, tokens, C, 0, nomap, stream));
+                g.A = xhat; g.mean = nullptr; g.rstd = nullptr;
             }
         }
-        if (!done1) CK((launch_gemm_any<T, EPI_BIAS_GELU>(g, stream)));
+        CK(launch_linear<EPI_BIAS_GELU>(g, plan.ws_gemm, w1b, di.sms, stream));
         kt.end(LEWIN_LEFF_K_FC1);
     }
     if (plan.tail) {
@@ -456,15 +406,10 @@ int leff_fwd(const LewinLeffFwdArgs* a, void* ws, size_t ws_bytes, cudaStream_t 
         return 0;
     }
     kt.begin(LEWIN_LEFF_K_DWCONV);
-    bool dw_done = false;
-    if constexpr (Act<T>::kIsBf16) {
-        if (dws::supported(a->H, a->W, Ch)) {     // persistent double-buffered kernel (dwconv_stream.cuh)
-            CK(dws::launch(static_cast<const __nv_bfloat16*>(a->h1), static_cast<__nv_bfloat16*>(a->h2),
-                           save ? static_cast<__nv_bfloat16*>(a->a2) : nullptr, a->w_dw, a->b_dw, a->B, a->H, a->W, Ch, di.sms, stream));
-            dw_done = true;
-        }
-    }
-    if (!dw_done)
+    if (Act<T>::kIsBf16 && dws::supported(a->H, a->W, Ch))      // persistent double-buffered kernel (dwconv_stream.cuh)
+        CK(dws::launch(static_cast<const __nv_bfloat16*>(a->h1), static_cast<__nv_bfloat16*>(a->h2),
+                       save ? static_cast<__nv_bfloat16*>(a->a2) : nullptr, a->w_dw, a->b_dw, a->B, a->H, a->W, Ch, di.sms, stream));
+    else
         CK(launch_dwconv_gelu_auto<T>(static_cast<const T*>(a->h1), static_cast<T*>(a->h2), save ? static_cast<T*>(a->a2) : nullptr,
                                       a->w_dw, a->b_dw, a->B, a->H, a->W, Ch, stream));
     kt.end(LEWIN_LEFF_K_DWCONV);
@@ -476,25 +421,11 @@ int leff_fwd(const LewinLeffFwdArgs* a, void* ws, size_t ws_bytes, cudaStream_t 
         g.M = tokens; g.N = C; g.K = Ch;
         g.tokens_per_image = a->H * a->W;
         kt.begin(LEWIN_LEFF_K_FC2);
-        bool done2 = false;
-        if constexpr (Act<T>::kIsBf16) {
-            if (plan.ws_gemm) {
-                g.R = y; g.drop_scale = a->drop_scale;
-                CK((ws::launch<EPI_BIAS_RESID>(g, false, di.sms, stream)));
-                done2 = true;
-            } else if (async_gemm) {
-                if (a->fused) { g.R = y; g.drop_scale = a->drop_scale; CK(((ws::wss_supported(g) ? ws::wss_launch<EPI_BIAS_RESID>(g, w2b, di.sms, stream) : launch_gemm_tca<EPI_BIAS_RESID>(g, w2b, stream)))); }
-                else { CK(((ws::wss_supported(g) ? ws::wss_launch<EPI_BIAS>(g, w2b, di.sms, stream) : launch_gemm_tca<EPI_BIAS>(g, w2b, stream)))); }
-                done2 = true;
-            }
-        }
-        if (!done2) {
-            if (a->fused) {
-                g.R = y; g.drop_scale = a->drop_scale;
-                CK((launch_gemm_any<T, EPI_BIAS_RESID>(g, stream)));
-            } else {
-                CK((launch_gemm_any<T, EPI_BIAS>(g, stream)));
-            }
+        if (a->fused) {
+            g.R = y; g.drop_scale = a->drop_scale;
+            CK(launch_linear<EPI_BIAS_RESID>(g, plan.ws_gemm, w2b, di.sms, stream));
+        } else {
+            CK(launch_linear<EPI_BIAS>(g, plan.ws_gemm, w2b, di.sms, stream));
         }
         kt.end(LEWIN_LEFF_K_FC2);
     }

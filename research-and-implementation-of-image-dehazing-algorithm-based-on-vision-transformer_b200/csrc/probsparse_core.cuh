@@ -301,14 +301,5 @@ cudaError_t launch_core_fwd_d(const CoreFwdArgs<T>& a, int num_sms, cudaStream_t
     k<<<grid, CORE_THREADS, smem, stream>>>(a);
     return cudaGetLastError();
 }
-// head_dim = C / nH in {32, 64, 128}
-template <typename T>
-cudaError_t launch_core_fwd(const CoreFwdArgs<T>& a, int num_sms, cudaStream_t stream) {
-    const int D = a.C / a.nH;
-    if (D == 32) return launch_core_fwd_d<T, 32>(a, num_sms, stream);
-    if (D == 64) return launch_core_fwd_d<T, 64>(a, num_sms, stream);
-    if (D == 128) return launch_core_fwd_d<T, 128>(a, num_sms, stream);
-    return cudaErrorInvalidValue;
-}
 
 }  // namespace lewin

@@ -1,5 +1,5 @@
 // Shared pieces of the bf16 ProbSparse core kernels (probsparse_core_v3.cuh forward, probsparse_core_bwd_v2.cuh backward;
-// reference ProbSparse/attn.py:287-342): ldmatrix / mma.sync.m16n8k16 wrappers and the argument struct.
+// reference ProbSparse/attn.py:287-342): ldmatrix / mma.sync.m16n8k16 wrappers.
 #pragma once
 #include <cuda_fp16.h>
 
@@ -30,13 +30,5 @@ __device__ __forceinline__ uint32_t pack2(float a, float b) {
     return *reinterpret_cast<uint32_t*>(&h);
 }
 }  // namespace pc
-
-struct CoreBf16Args {
-    const __nv_bfloat16* qkv; __nv_bfloat16* ctx; uint8_t* top;
-    const float* rpb_table; const float* rpb_dense; const int32_t* index_sample;   // [64, 25] (attn.py:91)
-    const float* mask; int nW_mask;
-    int B_, nH, C, use_rpb, shift, H, W, nWw, nWin;
-    int y0, Hg;           // row band of a taller image: see CoreFwdArgs
-};
 
 }  // namespace lewin

@@ -345,11 +345,6 @@ __global__ void __launch_bounds__(THREADS, 3) core_bwd_v2_kernel(const CoreBwdAr
     }
 }
 
-inline bool enabled() {
-    static const bool on = [] { const char* e = getenv("LEWIN_NO_CORE_BWD2"); return !(e && e[0] == '1'); }();
-    return on;
-}
-
 inline cudaError_t launch(const CoreBwdArgs<__nv_bfloat16>& a, int num_sms, cudaStream_t stream) {
     auto k = core_bwd_v2_kernel;
     const size_t smem = sizeof(Smem);

@@ -1,6 +1,6 @@
 // ProbSparse window-attention core, forward, bf16 — register-resident restatement (ProbSparse/attn.py:287-342).
 //
-// Same algorithm, rounding points and selection rule as probsparse_core_bf16_kernel; restructured around the measured
+// Same algorithm, rounding points and selection rule as probsparse_core_fwd_kernel (probsparse_core.cuh); restructured around the measured
 // bound of that kernel (instruction issue + 7 block barriers per (window, head) item, ~7500 warp-instructions per item):
 //   * q | k | v of the NEXT item are prefetched with cp.async into a second shared-memory buffer while the current one is
 //     processed (the item's DRAM latency is never exposed);
@@ -22,6 +22,8 @@ namespace lewin {
 namespace pc3 {
 
 constexpr int THREADS = 128;
+constexpr int CTAS = 5;                                 // resident CTAs per SM the register budget is compiled for (96 registers;
+                                                        // 6 CTAs at 80 registers measured 1.6 % slower: the kernel is issue-bound)
 constexpr int LD = 40;                                  // bf16 row stride of the q/k/v tiles (80 B: conflict-free ldmatrix)
 constexpr int TILE = kTok * LD;                         // elements per q / k / v tile
 
@@ -37,8 +39,7 @@ struct Smem {
     alignas(16) __nv_bfloat16 ostage[4][8 * kHeadDim];              // per-warp staging of the 8 selected context rows
 };
 
-template <int CTAS>   // resident CTAs per SM the register budget is compiled for (5: 96 registers, 6: 80 registers)
-__global__ void __launch_bounds__(THREADS, CTAS) probsparse_core_v3_kernel(const CoreBf16Args a) {
+__global__ void __launch_bounds__(THREADS, CTAS) probsparse_core_v3_kernel(const CoreFwdArgs<__nv_bfloat16> a) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     Smem& s = *reinterpret_cast<Smem*>(smem_raw);
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -331,14 +332,8 @@ __global__ void __launch_bounds__(THREADS, CTAS) probsparse_core_v3_kernel(const
     cp_async_wait<0>();
 }
 
-inline bool enabled() {
-    static const bool on = [] { const char* e = getenv("LEWIN_NO_CORE_V3"); return !(e && e[0] == '1'); }();
-    return on;
-}
-
-template <int CTAS>
-inline cudaError_t launch_c(const CoreBf16Args& a, int num_sms, cudaStream_t stream) {
-    auto k = probsparse_core_v3_kernel<CTAS>;
+inline cudaError_t launch(const CoreFwdArgs<__nv_bfloat16>& a, int num_sms, cudaStream_t stream) {
+    auto k = probsparse_core_v3_kernel;
     const size_t smem = sizeof(Smem);
     cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
     if (e != cudaSuccess) return e;
@@ -350,10 +345,18 @@ inline cudaError_t launch_c(const CoreBf16Args& a, int num_sms, cudaStream_t str
     return cudaGetLastError();
 }
 
-inline cudaError_t launch(const CoreBf16Args& a, int num_sms, cudaStream_t stream) {
-    static const int ctas = [] { const char* e = getenv("LEWIN_CORE_CTAS"); return e ? atoi(e) : 5; }();   // 6 CTAs (80 registers) measured 1.6 % slower: the kernel is issue-bound
-    return ctas == 5 ? launch_c<5>(a, num_sms, stream) : launch_c<6>(a, num_sms, stream);
-}
-
 }  // namespace pc3
+
+// head_dim = C / nH in {32, 64, 128}; bf16 at head_dim 32 runs the register-resident kernel above
+template <typename T>
+cudaError_t launch_core_fwd(const CoreFwdArgs<T>& a, int num_sms, cudaStream_t stream) {
+    const int D = a.C / a.nH;
+    if (D == 32) {
+        if constexpr (Act<T>::kIsBf16) return pc3::launch(a, num_sms, stream);
+        else return launch_core_fwd_d<T, 32>(a, num_sms, stream);
+    }
+    if (D == 64) return launch_core_fwd_d<T, 64>(a, num_sms, stream);
+    if (D == 128) return launch_core_fwd_d<T, 128>(a, num_sms, stream);
+    return cudaErrorInvalidValue;
+}
 }  // namespace lewin

@@ -201,8 +201,7 @@ __global__ void __launch_bounds__(THREADS) wgrad_bf16_kernel(const WgradArgs<__n
 }
 
 inline bool supported(const WgradArgs<__nv_bfloat16>& g) {
-    static const bool on = [] { const char* e = getenv("LEWIN_NO_WGRAD2"); return !(e && e[0] == '1'); }();
-    return on && !g.dy_aux && g.N % 32 == 0 && g.K % 32 == 0 && g.M < (1ll << 31);
+    return !g.dy_aux && g.N % 32 == 0 && g.K % 32 == 0 && g.M < (1ll << 31);
 }
 
 template <int NT, int KT, int WARPS_N>

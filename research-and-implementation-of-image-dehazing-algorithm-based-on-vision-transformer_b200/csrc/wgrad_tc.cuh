@@ -32,11 +32,6 @@ constexpr int BLK = TOK * 128;                // bytes of one [64 tokens x 64 fe
 constexpr int STG_LD = 33;                    // transpose tile row stride (floats)
 constexpr int SMEM_MAX = 227 * 1024;
 
-inline bool enabled() {
-    static const bool on = [] { const char* e = getenv("LEWIN_NO_WGRAD_TC"); return !(e && e[0] == '1'); }();
-    return on;
-}
-
 // MN-major SWIZZLE_128B descriptor: LBO = 8 KB (next 64-feature block), SBO = 1 KB (next 8-token group)
 __device__ __forceinline__ uint64_t make_desc_mn(uint32_t smem_addr) {
     return static_cast<uint64_t>((smem_addr >> 4) & 0x3FFF) | (static_cast<uint64_t>(BLK >> 4) << 16) |
@@ -159,7 +154,7 @@ __global__ void __launch_bounds__(THREADS, 1) wgrad_tc_kernel(const WgradArgs<__
 }
 
 inline bool supported(const WgradArgs<__nv_bfloat16>& g) {
-    if (!enabled() || g.mapDY || g.mapX || g.dy_row_scale || g.mean || g.dy_aux) return false;
+    if (g.mapDY || g.mapX || g.dy_row_scale || g.mean || g.dy_aux) return false;
     if (g.N % 32 || g.K % 32 || (g.K > 256 && g.K % 256) || g.M < 1024 || g.M >= (1ll << 31)) return false;
     if (!(g.K % 256 == 0 || g.K == 32 || g.K == 64 || g.K == 96 || g.K == 128 || g.K == 192)) return false;
     if ((g.lddy % 8) || (g.ldx % 8)) return false;

@@ -70,8 +70,7 @@ class Vgg19(nn.Module):
     # ---- B200 path: every conv + ReLU pair with Cin >= 64 (12 of the 13) as one implicit-GEMM tcgen05 kernel, forward and data
     #      gradient (ops.conv3x3_relu -> lewin_conv3x3_fwd_bf16); conv1_1 (3 input channels) and the max-pools stay on torch
     def _own_kernels(self, X):
-        import os
-        if not X.is_cuda or os.environ.get("LEWIN_VGG_CUDNN") == "1":
+        if not X.is_cuda:
             return False
         if any(p.requires_grad for p in self.parameters()):
             return False                                  # the kernel path has no weight gradient (the reference freezes VGG too)

@@ -11,7 +11,6 @@ lewin_leff(y, ...)   LeFF half (My_model_1.py:873) or, with ``fused=False``, LeF
 """
 from __future__ import annotations
 
-import os
 import threading
 import weakref
 
@@ -138,9 +137,6 @@ class TopRecorder:
         TopRecorder.active = None
 
 
-_WEIGHT_IMAGES_ON = os.environ.get("LEWIN_NO_WEIGHT_CACHE", "0") != "1"      # knob for scripts/diff_paths.py
-
-
 class _WeightImages:
     """bf16 images of constant fp32 weights for the C >= 256 GEMMs (the ABI's optional w*_bf16 fields).
 
@@ -238,7 +234,7 @@ def _attn_forward(x, ln_w, ln_b, w_qkv, b_qkv, w_out, b_out, rpb_table, rpb_dens
         qkv = torch.empty((tokens, 3 * C), dtype=x.dtype, device=dev)
         cbuf = torch.empty((tokens, C), dtype=x.dtype, device=dev)
     a.qkv, a.ctx = _ptr(qkv), _ptr(cbuf)
-    if dt == "bf16" and C >= 256 and not need_grad and _WEIGHT_IMAGES_ON:      # constants of an inference call: convert once
+    if dt == "bf16" and C >= 256 and not need_grad:      # constants of an inference call: convert once
         wq_b, wo_b = _bf16_image(w_qkv_), _bf16_image(w_out_)
         a.w_qkv_bf16, a.w_out_bf16 = _ptr(wq_b), _ptr(wo_b)
     if KernelTimer.active is not None:
@@ -328,7 +324,7 @@ def _leff_forward(y, ln_w, ln_b, w1, b1, w_dw, b_dw, w2, b2, drop_scale, geom, o
         y=_ptr(y), out=_ptr(out), ln_w=_ptr(ln_w_), ln_b=_ptr(ln_b_), w1=_ptr(w1_), b1=_ptr(b1_),
         w_dw=_ptr(wdw_), b_dw=_ptr(bdw_), w2=_ptr(w2_), b2=_ptr(b2_), drop_scale=_ptr(ds_),
         h1=_ptr(h1), h2=_ptr(h2), a1=_ptr(a1), a2=_ptr(a2))
-    if dt == "bf16" and C >= 256 and not need_grad and _WEIGHT_IMAGES_ON:
+    if dt == "bf16" and C >= 256 and not need_grad:
         w1_b, w2_b = _bf16_image(w1_), _bf16_image(w2_)
         a.w1_bf16, a.w2_bf16 = _ptr(w1_b), _ptr(w2_b)
     if out_view is not None and not need_grad and lib.lewin_leff_fwd_supports_ld_out(a, _lib.DTYPE_TAG[dt]):
@@ -497,10 +493,7 @@ def probsparse_core(qkv, *, num_heads, index_sample, rpb_table=None, rpb_dense=N
 
 def upsample_supported(x, Cin, Cout, tokens):
     """The 2x2 / stride-2 transposed convolution runs as a token GEMM on the streamed-W tcgen05 kernel (bf16, no autograd)."""
-    import os
-    return (x.is_cuda and x.dtype == torch.bfloat16 and Cin % 64 == 0 and Cout % 32 == 0 and tokens >= 1 and
-            os.environ.get("LEWIN_NO_WS_GEMM") != "1" and os.environ.get("LEWIN_NO_WSS_GEMM") != "1" and
-            os.environ.get("LEWIN_NO_UPSAMPLE_GEMM") != "1")
+    return x.is_cuda and x.dtype == torch.bfloat16 and Cin % 64 == 0 and Cout % 32 == 0 and tokens >= 1
 
 
 def lewin_upsample(x, weight, bias, *, B, H, W, out=None):
@@ -523,14 +516,9 @@ def lewin_upsample(x, weight, bias, *, B, H, W, out=None):
     return out
 
 
-def conv_igemm_enabled():
-    import os
-    return os.environ.get("LEWIN_NO_CONV_IGEMM") != "1"
-
-
 def downsample_supported(x, Cin, W):
     """Downsample's 4x4 / stride-2 convolution runs as an implicit GEMM on tcgen05 (bf16, no autograd)."""
-    return (conv_igemm_enabled() and x.is_cuda and x.dtype == torch.bfloat16 and (Cin == 32 or (Cin % 64 == 0 and Cin <= 512)) and
+    return (x.is_cuda and x.dtype == torch.bfloat16 and (Cin == 32 or (Cin % 64 == 0 and Cin <= 512)) and
             W % 16 == 0)
 
 
@@ -557,7 +545,7 @@ def lewin_downsample(x, weight, bias, *, B, H, W, pad_h=True, out=None):
 
 def conv3x3_supported(x, Cin, Cout):
     """x: NCHW tensor in channels_last memory format, bf16, on the GPU; Cin, Cout multiples of 64 up to 512; W % 8 == 0."""
-    return (conv_igemm_enabled() and x.is_cuda and x.dtype == torch.bfloat16 and x.dim() == 4 and Cin % 64 == 0 and Cin <= 512 and
+    return (x.is_cuda and x.dtype == torch.bfloat16 and x.dim() == 4 and Cin % 64 == 0 and Cin <= 512 and
             Cout % 64 == 0 and Cout <= 512 and x.shape[3] % 8 == 0 and x.is_contiguous(memory_format=torch.channels_last))
 
 
@@ -610,7 +598,7 @@ def conv3x3_relu(x, w_fwd, w_bwd, bias):
 
 
 def output_proj_supported(x, Cin, Cout, W):
-    return (conv_igemm_enabled() and x.is_cuda and x.dtype == torch.bfloat16 and Cin % 64 == 0 and Cin <= 256 and 1 <= Cout <= 8)
+    return x.is_cuda and x.dtype == torch.bfloat16 and Cin % 64 == 0 and Cin <= 256 and 1 <= Cout <= 8
 
 
 def lewin_output_proj(x, weight, bias, *, B, H, W, residual=None, pad_h=True):

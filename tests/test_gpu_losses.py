@@ -70,7 +70,7 @@ def test_contrast_loss_on_own_kernels_matches_the_cudnn_path(monkeypatch):
     n_own = sum("conv_igemm_kernel" in k for k in names)
     # features[0:30] hold 13 convolutions; all but the 3-channel conv1_1: 12 layers x (a pass + p|n pass) forward, 12 data gradients
     assert n_own == 12 * 2 + 12, n_own
-    monkeypatch.setenv("LEWIN_VGG_CUDNN", "1")
+    monkeypatch.setattr(crit.vgg, "_own_kernels", lambda X: False)      # the cuDNN path
     l2, ap2, an2, g2 = run()
     assert abs(l1 - l2) < 2e-2 * abs(l2) and abs(ap1 - ap2) < 2e-2 * abs(ap2) and abs(an1 - an2) < 2e-2 * abs(an2), (l1, l2)
     # the gradient of an L1 loss through 13 bf16 layers is noisy in either implementation (sign(fa - fp) flips wherever two
