@@ -137,7 +137,8 @@ int lewin_attn_fwd_bf16(const LewinAttnFwdArgs* a, void* workspace, size_t works
 
 /* Backward of the attention half (autograd of the same reference lines; gradient paths in
  * SURVEY.md section 3.4).  Gradients of parameters are ACCUMULATED (+=) into fp32 buffers the
- * caller zero-initialises, dx is written. */
+ * caller zero-initialises, dx is written.  Shapes as the forward's (C % 32 == 0, C <= 1024,
+ * head_dim = C / nH in {32, 64, 128}) with nH <= 16; anything else returns LEWIN_E_SHAPE. */
 typedef struct {
     LewinAttnFwdArgs fwd;          /* same tensors as the forward call (x, params, qkv, ctx, top, ...) */
     const void* dy;                /* same shape/dtype as y */
@@ -244,6 +245,8 @@ int lewin_leff_fwd_supports_ld_out(const LewinLeffFwdArgs* a, int dtype);
 int lewin_leff_fwd_f32 (const LewinLeffFwdArgs* a, void* workspace, size_t workspace_bytes, lewin_stream_t stream);
 int lewin_leff_fwd_bf16(const LewinLeffFwdArgs* a, void* workspace, size_t workspace_bytes, lewin_stream_t stream);
 
+/* Backward of the LeFF half: parameter gradients ACCUMULATED into zero-initialised fp32 buffers, dy written.
+ * C % 32 == 0, hidden % 32 == 0, C <= 1024 (as the forward); anything else returns LEWIN_E_SHAPE. */
 typedef struct {
     LewinLeffFwdArgs fwd;
     const void* dout;              /* gradient of `out` */

@@ -319,11 +319,109 @@ __global__ void __launch_bounds__(256, MAXV == 1 ? 3 : 1) ln_bwd_kernel(const T*
     }
 }
 
+// The same LayerNorm backward for fp32 rows of 516 ... 1024 channels (embed_dim 64: C = 1024 at the bottleneck).  ln_bwd_kernel
+// would need 32 elements of x, dz and dres per lane plus per-lane d(gamma) / d(beta) partials for 32 columns, which spills;
+// here a CTA stages LNW_ROWS rows of x and dz in shared memory (4 KB each per row at C = 1024), one warp per row reduces the
+// row statistics from there, and then thread t owns columns [4t, 4t + 4) of every staged row: dx is written and dres read
+// as whole coalesced rows, and d(gamma) / d(beta) live in 8 registers per thread until one atomic per column per CTA.
+constexpr int LNW_ROWS = 8;           // rows per tile = warps per CTA (one row's statistics per warp)
+constexpr int LNW_THREADS = 256;      // x 4 columns = the widest row
+
+__global__ void __launch_bounds__(LNW_THREADS) ln_bwd_wide_kernel(const float* __restrict__ dz, const float* __restrict__ x,
+                                                                  const float* __restrict__ dres, float* __restrict__ dx,
+                                                                  const float* __restrict__ gamma, float* __restrict__ dgamma,
+                                                                  float* __restrict__ dbeta, long long rows, int C) {
+    extern __shared__ __align__(16) float lnw_smem[];
+    float* xs = lnw_smem;                         // [LNW_ROWS][C]
+    float* ds = lnw_smem + LNW_ROWS * C;          // [LNW_ROWS][C]
+    __shared__ float s_mu[LNW_ROWS], s_rs[LNW_ROWS], s_s1[LNW_ROWS], s_s2[LNW_ROWS];
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int cpr = C / 4;                        // 16-byte chunks per row
+    const int k = tid * 4;                        // this thread's columns
+    const bool own = tid < cpr;
+    const float4 gm = own ? ld4(gamma + k) : make_float4(0.f, 0.f, 0.f, 0.f);
+    float4 ga = make_float4(0.f, 0.f, 0.f, 0.f), ba = make_float4(0.f, 0.f, 0.f, 0.f);
+
+    for (long long r0 = static_cast<long long>(blockIdx.x) * LNW_ROWS; r0 < rows; r0 += static_cast<long long>(gridDim.x) * LNW_ROWS) {
+        const int nr = rows - r0 < LNW_ROWS ? static_cast<int>(rows - r0) : LNW_ROWS;
+        __syncthreads();                          // the previous tile's column pass is done with xs / ds
+        for (int c = tid; c < nr * cpr; c += LNW_THREADS) {
+            const long long o = r0 * C + static_cast<long long>(c) * 4;
+            *reinterpret_cast<float4*>(xs + c * 4) = ld4(x + o);
+            *reinterpret_cast<float4*>(ds + c * 4) = ld4(dz + o);
+        }
+        __syncthreads();
+        if (warp < nr) {                          // row statistics: two-pass mean / biased variance, then <dxhat> and <dxhat, xhat>
+            const float* xr = xs + warp * C;
+            const float* dr = ds + warp * C;
+            float s = 0.f;
+            for (int c = lane; c < cpr; c += 32) {
+                const float4 v = *reinterpret_cast<const float4*>(xr + c * 4);
+                s += (v.x + v.y) + (v.z + v.w);
+            }
+            const float mu = group_sum<32>(s) / C;
+            float q = 0.f;
+            for (int c = lane; c < cpr; c += 32) {
+                const float4 v = *reinterpret_cast<const float4*>(xr + c * 4);
+                const float a = v.x - mu, b = v.y - mu, e = v.z - mu, f = v.w - mu;
+                q += (a * a + b * b) + (e * e + f * f);
+            }
+            const float rs = rsqrtf(group_sum<32>(q) / C + 1e-5f);
+            float s1 = 0.f, s2 = 0.f;
+            for (int c = lane; c < cpr; c += 32) {
+                const float4 v = *reinterpret_cast<const float4*>(xr + c * 4);
+                const float4 d = *reinterpret_cast<const float4*>(dr + c * 4);
+                const float4 g = ld4(gamma + c * 4);
+                const float d0 = d.x * g.x, d1 = d.y * g.y, d2 = d.z * g.z, d3 = d.w * g.w;
+                s1 += (d0 + d1) + (d2 + d3);
+                s2 += (d0 * (v.x - mu) + d1 * (v.y - mu)) + (d2 * (v.z - mu) + d3 * (v.w - mu));
+            }
+            s1 = group_sum<32>(s1);
+            s2 = group_sum<32>(s2);
+            if (lane == 0) { s_mu[warp] = mu; s_rs[warp] = rs; s_s1[warp] = s1 / C; s_s2[warp] = s2 * rs / C; }
+        }
+        __syncthreads();
+        if (own) {
+            for (int r = 0; r < nr; ++r) {
+                const float mu = s_mu[r], rs = s_rs[r], s1 = s_s1[r], s2 = s_s2[r];
+                const float4 v = *reinterpret_cast<const float4*>(xs + r * C + k);
+                const float4 d = *reinterpret_cast<const float4*>(ds + r * C + k);
+                const long long o = (r0 + r) * C + k;
+                const float4 res = dres ? ld4(dres + o) : make_float4(0.f, 0.f, 0.f, 0.f);
+                const float h0 = (v.x - mu) * rs, h1 = (v.y - mu) * rs, h2 = (v.z - mu) * rs, h3 = (v.w - mu) * rs;   // xhat
+                ga.x += d.x * h0; ga.y += d.y * h1; ga.z += d.z * h2; ga.w += d.w * h3;
+                ba.x += d.x; ba.y += d.y; ba.z += d.z; ba.w += d.w;
+                st4(dx + o, make_float4(res.x + rs * (d.x * gm.x - s1 - h0 * s2), res.y + rs * (d.y * gm.y - s1 - h1 * s2),
+                                        res.z + rs * (d.z * gm.z - s1 - h2 * s2), res.w + rs * (d.w * gm.w - s1 - h3 * s2)));
+            }
+        }
+    }
+    if (own) {
+        atomicAdd(dgamma + k, ga.x); atomicAdd(dgamma + k + 1, ga.y); atomicAdd(dgamma + k + 2, ga.z); atomicAdd(dgamma + k + 3, ga.w);
+        atomicAdd(dbeta + k, ba.x); atomicAdd(dbeta + k + 1, ba.y); atomicAdd(dbeta + k + 2, ba.z); atomicAdd(dbeta + k + 3, ba.w);
+    }
+}
+
+inline cudaError_t launch_ln_bwd_wide(const float* dz, const float* x, const float* dres, float* dx, const float* gamma,
+                                      float* dgamma, float* dbeta, long long rows, int C, int num_sms, cudaStream_t st) {
+    const int smem = 2 * LNW_ROWS * C * static_cast<int>(sizeof(float));     // 64 KB at C = 1024: three CTAs per SM
+    cudaError_t e = cudaFuncSetAttribute(ln_bwd_wide_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+    if (e != cudaSuccess) return e;
+    long long blocks = (rows + LNW_ROWS - 1) / LNW_ROWS;
+    const long long cap = static_cast<long long>(num_sms) * 3;
+    if (blocks > cap) blocks = cap;
+    ln_bwd_wide_kernel<<<static_cast<unsigned>(blocks), LNW_THREADS, smem, st>>>(dz, x, dres, dx, gamma, dgamma, dbeta, rows, C);
+    return cudaGetLastError();
+}
+
 template <typename T>
 cudaError_t launch_ln_bwd(const T* dz, const T* x, const T* dres, T* dx, const float* gamma, float* dgamma,
                           float* dbeta, long long rows, int C, int num_sms, cudaStream_t st) {
     constexpr int EPL = 16 / sizeof(T);
     const int chunks = C / EPL;
+    if constexpr (!Act<T>::kIsBf16) {
+        if (C <= 1024 && chunks > 128) return launch_ln_bwd_wide(dz, x, dres, dx, gamma, dgamma, dbeta, rows, C, num_sms, st);
+    }
     auto go = [&](auto gtag, auto vtag) -> cudaError_t {
         constexpr int G = decltype(gtag)::value, MAXV = decltype(vtag)::value;
         long long blocks = (rows + 8 * (32 / G) - 1) / (8 * (32 / G));
@@ -913,7 +1011,7 @@ int attn_bwd(const LewinAttnBwdArgs* a, void* ws, size_t ws_bytes, cudaStream_t 
     if (!f.x || !f.w_qkv || !f.w_out || !f.qkv || !f.ctx || !f.top) return LEWIN_E_NULL;
     if (!a->d_w_qkv || !a->d_b_qkv || !a->d_w_out || !a->d_b_out) return LEWIN_E_NULL;
     if (!f.windowed && (!f.ln_w || !f.ln_b || !a->d_ln_w || !a->d_ln_b)) return LEWIN_E_NULL;
-    if (f.H % 8 || f.W % 8 || f.C % 32 || !head_dim_ok(f.C, f.nH) || f.C > 512 || f.nH > 16) return LEWIN_E_SHAPE;
+    if (f.H % 8 || f.W % 8 || f.C % 32 || !head_dim_ok(f.C, f.nH) || f.C > 1024 || f.nH > 16) return LEWIN_E_SHAPE;
     int sms = 0;
     if (int rc = bw_device(&sms)) return rc;
     const int dtype = Act<T>::kIsBf16 ? LEWIN_DTYPE_BF16 : LEWIN_DTYPE_F32;
@@ -1032,7 +1130,7 @@ int leff_bwd(const LewinLeffBwdArgs* a, void* ws, size_t ws_bytes, cudaStream_t 
     if (!f.y || !f.w1 || !f.w_dw || !f.w2 || !f.h1 || !f.h2 || !f.a1 || !f.a2) return LEWIN_E_NULL;
     if (!a->d_w1 || !a->d_b1 || !a->d_w_dw || !a->d_b_dw || !a->d_w2 || !a->d_b2) return LEWIN_E_NULL;
     if (f.fused && (!f.ln_w || !f.ln_b || !a->d_ln_w || !a->d_ln_b)) return LEWIN_E_NULL;
-    if (f.C % 32 || f.hidden % 32 || f.C > 512) return LEWIN_E_SHAPE;
+    if (f.C % 32 || f.hidden % 32 || f.C > 1024) return LEWIN_E_SHAPE;
     int sms = 0;
     if (int rc = bw_device(&sms)) return rc;
     const int dtype = Act<T>::kIsBf16 ? LEWIN_DTYPE_BF16 : LEWIN_DTYPE_F32;

@@ -2,13 +2,13 @@
 
 Sweep: window 8 (N = 64 tokens, u = U = 25), heads 1..16 at head_dim 32 (C = 32 * heads, what the reference's
 Uformer_ProbSparse produces at embed_dim 32) over 64..1024 windows, plus head_dim = embed_dim 64 and 128 (My_model_1.py:962
-makes head_dim = embed_dim; C = heads * head_dim up to 512, the widest level the backward is built for) over 64 / 256 / 1024
-windows; shift 0 / 4, bf16 and f32; forward and
+makes head_dim = embed_dim; C = heads * head_dim up to 1024, the bottleneck of the embed_dim 64 model: 16 heads of 64, and
+8 heads of 128) over 64 / 256 / 1024 windows; shift 0 / 4, bf16 and f32; forward and
 forward+backward microseconds per block (attention half + LeFF half through the C ABI, `ops.lewin_attn` / `ops.lewin_leff`),
 CUDA events over `--iters` calls after 3 warm-up calls, x ~ N(0, 1) seed 0, weights N(0, C^-1/2), index_sample from
 torch.manual_seed(0); torch.randint(64, (64, 25)).  Also prints the fraction of the block's roofline time (SURVEY 8d: fully
 fused ideal = max(algorithmic FLOPs / sustained bf16 TFLOP/s, 4 C s bytes per token / HBM GB/s)).
-Usage (GPU box):  python scripts/op_microbench.py [--iters 20] [--out gpurun_out/op_microbench.json]
+Usage (GPU box):  python scripts/op_microbench.py [--iters 20] [--channels 1024] [--out FILE]
 """
 import argparse
 import json
@@ -23,6 +23,7 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--iters", type=int, default=20)
     ap.add_argument("--head-dim-32-only", action="store_true", help="skip the head_dim 64 / 128 rows")
+    ap.add_argument("--channels", type=int, nargs="*", help="only the rows of these widths C")
     ap.add_argument("--out", default=os.path.join(ROOT, "gpurun_out", "op_microbench.json"))
     args = ap.parse_args()
     import torch
@@ -39,7 +40,9 @@ def main():
         tdt = torch.bfloat16 if dtype == "bf16" else torch.float32
         sweep = [(32, h, (64, 128, 256, 512, 1024)) for h in (1, 2, 4, 8, 16)]
         if not args.head_dim_32_only:
-            sweep += [(hd, h, (64, 256, 1024)) for hd in (64, 128) for h in (1, 2, 4, 8) if hd * h <= 512]
+            sweep += [(hd, h, (64, 256, 1024)) for hd in (64, 128) for h in (1, 2, 4, 8, 16) if hd * h <= 1024]
+        if args.channels:
+            sweep = [t for t in sweep if t[0] * t[1] in args.channels]
         for head_dim, heads, window_counts in sweep:
             C = head_dim * heads
             for windows in window_counts:
@@ -117,7 +120,7 @@ def main():
                     ideal_us = max(flops / (tf * 1e12), tokens * 4 * C * s / (hbm * 1e9)) * 1e6
                     rows.append(dict(dtype=dtype, heads=heads, head_dim=head_dim, C=C, windows=windows, H=H, W=W, shift=shift, fwd_us=f_us,
                                      fwd_bwd_us=fb_us, fwd_us_eager=f_eager, fwd_bwd_us_eager=fb_eager, launch=launch, fwd_tflops=flops / f_us / 1e6, ideal_fwd_us=ideal_us))
-                    print(f"{dtype} heads={heads:2d} head_dim={head_dim:3d} C={C:3d} windows={windows:4d} ({H}x{W}) shift={shift}: fwd {f_us:8.1f} us  "
+                    print(f"{dtype} heads={heads:2d} head_dim={head_dim:3d} C={C:4d} windows={windows:4d} ({H}x{W}) shift={shift}: fwd {f_us:8.1f} us  "
                           f"fwd+bwd {fb_us:8.1f} us (eager {f_eager:7.1f} / {fb_eager:7.1f})  {flops / f_us / 1e6:7.1f} TFLOP/s fwd  "
                           f"(fused-ideal {ideal_us:6.1f} us)", flush=True)
     os.makedirs(os.path.dirname(args.out), exist_ok=True)

@@ -2,7 +2,9 @@
 restored = clamp(model(input), 0, 1), loss = Charbonnier(eps 1e-3) + ContrastLoss(VGG19, random init: no weight file
 offline), AdamW 2e-4 / wd 0.02; My_train.py:221-250) on the sm_100a LeWin ops; under torchrun the model is wrapped with
 parallel.wrap_ddp (NCCL gradient all-reduce).  `contrast=False` drops the VGG term (the LeWin path alone).
-Prints one JSON line (rank 0)."""
+Prints one JSON line (rank 0).
+Usage:  python scripts/train_step.py [batch] [--embed-dim 32|64]   (embed_dim 64: C = 64 ... 1024, 16 heads of 64 at the bottleneck)"""
+import argparse
 import json
 import os
 import sys
@@ -11,7 +13,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 
 
-def run(batch=32, steps=10, warmup=3, dtype="bf16", graph=True, contrast=True):
+def run(batch=32, steps=10, warmup=3, dtype="bf16", graph=True, contrast=True, embed_dim=32):
     import torch
     import torch.distributed as dist
     import lewin_b200 as L
@@ -23,7 +25,7 @@ def run(batch=32, steps=10, warmup=3, dtype="bf16", graph=True, contrast=True):
         os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
         dist.init_process_group("nccl", device_id=dev)
     torch.manual_seed(1234)
-    model = L.Uformer(img_size=128, embed_dim=32, win_size=8, token_projection="linear", token_mlp="leff").to(dev).train()
+    model = L.Uformer(img_size=128, embed_dim=embed_dim, win_size=8, token_projection="linear", token_mlp="leff").to(dev).train()
     crit = None
     if contrast:
         from lewin_b200.losses import ContrastLoss
@@ -49,7 +51,7 @@ def run(batch=32, steps=10, warmup=3, dtype="bf16", graph=True, contrast=True):
     if world > 1:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
     res = dict(step_ms=float(ms.item()), patches_per_s=batch * world / (float(ms.item()) / 1e3), batch_per_gpu=batch, n_gpus=world,
-               dtype=dtype, loss=ts.loss(),
+               embed_dim=embed_dim, dtype=dtype, loss=ts.loss(),
                loss_terms="Charbonnier + ContrastLoss (VGG19 random init, p / n passes batched under no_grad, channels-last bf16)"
                if contrast else "Charbonnier only",
                optimizer="AdamW(2e-4, wd 0.02)", parallelism="ddp" if world > 1 else "single", launch=ts.launch_mode,
@@ -58,6 +60,10 @@ def run(batch=32, steps=10, warmup=3, dtype="bf16", graph=True, contrast=True):
 
 
 if __name__ == "__main__":
-    r, rank = run(batch=int(sys.argv[1]) if len(sys.argv) > 1 else 32)
+    ap = argparse.ArgumentParser()
+    ap.add_argument("batch", type=int, nargs="?", default=32)
+    ap.add_argument("--embed-dim", type=int, default=32, choices=(32, 64))
+    args = ap.parse_args()
+    r, rank = run(batch=args.batch, embed_dim=args.embed_dim)
     if rank == 0:
         print(json.dumps(r), flush=True)
