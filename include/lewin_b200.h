@@ -39,7 +39,7 @@ extern "C" {
 typedef struct CUstream_st* lewin_stream_t; /* == cudaStream_t */
 typedef struct CUevent_st*  lewin_event_t;  /* == cudaEvent_t  */
 
-#define LEWIN_ABI_VERSION 5
+#define LEWIN_ABI_VERSION 6
 
 /* error codes (negative) */
 #define LEWIN_E_NULL      (-1)  /* a required pointer is NULL */
@@ -69,10 +69,19 @@ typedef struct CUevent_st*  lewin_event_t;  /* == cudaEvent_t  */
  *       into the load / store addressing.
  *   windowed == 1 (strict drop-in at WindowAttention.forward): x, y are [B_, 64, C] windows
  *       (B_ = B * (H/8) * (W/8), batch-major); no LN, no roll, no residual.
- * Mask: `mask` (nullable) is a dense fp32 [nW_mask, 64, 64] added to the post-softmax
- * probabilities of window (w mod nW_mask) exactly as attn.py:236-261; if `analytic_shift_mask`
- * != 0 and shift > 0 the shift mask of My_model_1.py:803-836 is evaluated in registers instead
- * of being materialised (the two may be combined).
+ * Masks are added to the post-softmax probabilities exactly as attn.py:236-261, in one fp32 add
+ * after the relative-position bias:
+ *   - `mask` (nullable) is a dense fp32 [nW_mask, 64, 64], window w takes slice (w mod nW_mask);
+ *   - if `analytic_shift_mask` != 0 and shift > 0, the shift mask of My_model_1.py:803-836 is
+ *     evaluated from window coordinates instead of being materialised (combinable with `mask`);
+ *   - `token_mask` (nullable, fused block half only) is the input mask of My_model_1.py:791-798
+ *     as one fp32 value per token: the caller's F.interpolate(mask, size=(H, W)) as [Bm, H, W],
+ *     image b using mask (b mod Bm).  For query token i and key token j of a window the term is
+ *     -100 where the fp32 product m_i * m_j != 0, else 0, and is combined with the analytic
+ *     shift mask before the single add, so the result equals the dense [B*nW, 64, 64] mask the
+ *     reference builds.  Window (wy, wx) reads m[wy*8 + r/8, wx*8 + r%8] for its row r: the
+ *     unshifted frame, as the reference partitions the mask (not the pixel a rolled token came
+ *     from).  Not combinable with `mask`, `windowed` or `band_mode` (LEWIN_E_SHAPE); B % Bm == 0.
  * ---------------------------------------------------------------------------------------- */
 typedef struct {
     int32_t B, H, W, C, nH;        /* head_dim = C / nH (d_keys = d_model // n_heads, attn.py:370-372) in {32, 64, 128};
@@ -122,6 +131,11 @@ typedef struct {
      * torch.roll would bring in).  The cyclic shift then applies to the columns only, and the analytic shift mask
      * (My_model_1.py:803-836) takes its row regions at shifted-frame row band_y0 + (row in the band).  band_mode = 0: whole image. */
     int32_t band_mode, band_y0, band_Hg, reserved2;
+
+    /* Input mask per token (see the mask paragraph above): [Bm, H, W] fp32, 16-byte aligned, or NULL.  Saved for and read
+     * again by lewin_attn_bwd_*. */
+    const float* token_mask;
+    int32_t Bm, reserved3;
 } LewinAttnFwdArgs;
 
 #define LEWIN_ATTN_K_LNSTATS 0

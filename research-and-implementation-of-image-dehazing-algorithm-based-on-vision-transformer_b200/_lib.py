@@ -30,6 +30,7 @@ class LewinAttnFwdArgs(C.Structure):
         ("timing", c_ptr),
         ("w_qkv_bf16", c_ptr), ("w_out_bf16", c_ptr),
         ("band_mode", C.c_int32), ("band_y0", C.c_int32), ("band_Hg", C.c_int32), ("reserved2", C.c_int32),
+        ("token_mask", c_ptr), ("Bm", C.c_int32), ("reserved3", C.c_int32),
     ]
 
 
@@ -136,7 +137,7 @@ EXPORTS = (
     "lewin_output_proj_fwd_bf16", "lewin_output_proj_fwd_workspace_bytes",
 )
 
-ABI_VERSION = 5
+ABI_VERSION = 6
 DTYPE_TAG = {"f32": 0, "bf16": 1}
 
 _lib = None

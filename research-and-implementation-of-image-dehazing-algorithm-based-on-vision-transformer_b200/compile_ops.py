@@ -30,11 +30,12 @@ def _req(t, like):
 def attn_fwd(x: Tensor, ln_w: Optional[Tensor], ln_b: Optional[Tensor], w_qkv: Tensor, b_qkv: Tensor, w_out: Tensor,
              b_out: Tensor, rpb_table: Optional[Tensor], rpb_dense: Optional[Tensor], index_sample: Tensor,
              mask: Optional[Tensor], drop_scale: Optional[Tensor], B: int, H: int, W: int, num_heads: int, shift: int,
-             windowed: bool, use_rpb: bool, analytic_shift_mask: bool, save: bool) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
+             windowed: bool, use_rpb: bool, analytic_shift_mask: bool, save: bool, token_mask: Optional[Tensor] = None
+             ) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
     """-> (y, top u8 [B_, nH, 25], qkv [tokens, 3C], ctx [tokens, C]); qkv / ctx are empty unless ``save``."""
     geom = (B, H, W, num_heads, shift, windowed, use_rpb, analytic_shift_mask, save)
     y, top, saved = ops._attn_forward(x, ln_w, ln_b, w_qkv, b_qkv, w_out, b_out, rpb_table, rpb_dense, index_sample, mask,
-                                      drop_scale, geom)
+                                      drop_scale, geom, token_mask)
     if not save:
         return y, top, x.new_empty((0,)), x.new_empty((0,))
     qkv, cbuf = saved[12], saved[13]
@@ -43,7 +44,7 @@ def attn_fwd(x: Tensor, ln_w: Optional[Tensor], ln_b: Optional[Tensor], w_qkv: T
 
 @attn_fwd.register_fake
 def _(x, ln_w, ln_b, w_qkv, b_qkv, w_out, b_out, rpb_table, rpb_dense, index_sample, mask, drop_scale, B, H, W, num_heads,
-      shift, windowed, use_rpb, analytic_shift_mask, save):
+      shift, windowed, use_rpb, analytic_shift_mask, save, token_mask=None):
     C = x.shape[-1]
     tokens = B * H * W
     y = torch.empty_like(x, memory_format=torch.contiguous_format)
@@ -57,13 +58,14 @@ def _(x, ln_w, ln_b, w_qkv, b_qkv, w_out, b_out, rpb_table, rpb_dense, index_sam
 def attn_bwd(dy: Tensor, x: Tensor, ln_w: Optional[Tensor], ln_b: Optional[Tensor], w_qkv: Tensor, b_qkv: Tensor,
              w_out: Tensor, b_out: Tensor, rpb_table: Optional[Tensor], rpb_dense: Optional[Tensor], index_sample: Tensor,
              mask: Optional[Tensor], drop_scale: Optional[Tensor], qkv: Tensor, ctx: Tensor, top: Tensor, B: int, H: int,
-             W: int, num_heads: int, shift: int, windowed: bool, use_rpb: bool, analytic_shift_mask: bool
-             ) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor, Tensor, Tensor, Tensor]:
+             W: int, num_heads: int, shift: int, windowed: bool, use_rpb: bool, analytic_shift_mask: bool,
+             token_mask: Optional[Tensor] = None) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor, Tensor, Tensor, Tensor]:
     """-> (dx, d_ln_w, d_ln_b, d_w_qkv, d_b_qkv, d_w_out, d_b_out, d_rpb); d_rpb has the shape of whichever bias was given."""
     geom = (B, H, W, num_heads, shift, windowed, use_rpb, analytic_shift_mask, True)
     f = ops._f32c
     saved = (x.contiguous(), f(ln_w), f(ln_b), f(w_qkv), f(b_qkv), f(w_out), f(b_out), f(rpb_table), f(rpb_dense),
-             ops.prepare_index_sample(index_sample, x.device), f(mask), f(drop_scale), qkv, ctx, top)
+             ops.prepare_index_sample(index_sample, x.device), f(mask), f(drop_scale), qkv, ctx, top,
+             ops._token_mask(token_mask, B, H, W, x.device))
     dx, d_ln_w, d_ln_b, d_wq, d_bq, d_wo, d_bo, d_tab, d_dense = ops._attn_backward(saved, geom, dy, separate_grads=True)
     d_rpb = d_tab if d_tab is not None else d_dense
     z = dx.new_empty((0,), dtype=torch.float32)
@@ -72,7 +74,7 @@ def attn_bwd(dy: Tensor, x: Tensor, ln_w: Optional[Tensor], ln_b: Optional[Tenso
 
 @attn_bwd.register_fake
 def _(dy, x, ln_w, ln_b, w_qkv, b_qkv, w_out, b_out, rpb_table, rpb_dense, index_sample, mask, drop_scale, qkv, ctx, top,
-      B, H, W, num_heads, shift, windowed, use_rpb, analytic_shift_mask):
+      B, H, W, num_heads, shift, windowed, use_rpb, analytic_shift_mask, token_mask=None):
     def g(t):
         return x.new_empty((0,) if t is None else tuple(t.shape), dtype=torch.float32)
     return (torch.empty_like(x, memory_format=torch.contiguous_format), g(ln_w), g(ln_b), g(w_qkv), g(b_qkv), g(w_out),
@@ -80,7 +82,8 @@ def _(dy, x, ln_w, ln_b, w_qkv, b_qkv, w_out, b_out, rpb_table, rpb_dense, index
 
 
 def _attn_setup(ctx, inputs, output):
-    (x, ln_w, ln_b, w_qkv, b_qkv, w_out, b_out, rpb_table, rpb_dense, index_sample, mask, drop_scale, *geom) = inputs
+    (x, ln_w, ln_b, w_qkv, b_qkv, w_out, b_out, rpb_table, rpb_dense, index_sample, mask, drop_scale, *rest) = inputs
+    geom, token_mask = rest[:9], (rest[9] if len(rest) > 9 else None)
     if not geom[-1]:
         ctx.geom = None              # an inference call reached autograd: refused in the backward, with the reason
         return
@@ -88,21 +91,21 @@ def _attn_setup(ctx, inputs, output):
     ctx.geom = tuple(geom[:-1])
     ctx.have = (ln_w is not None, rpb_table is not None, rpb_dense is not None)
     ctx.save_for_backward(x, ln_w, ln_b, w_qkv, b_qkv, w_out, b_out, rpb_table, rpb_dense, index_sample, mask, drop_scale,
-                          qkv, cbuf, top)
+                          qkv, cbuf, top, token_mask)
 
 
 def _attn_backward(ctx, dy, _dtop, _dqkv, _dctx):
     if ctx.geom is None:
         raise RuntimeError("lewin_b200::attn_fwd was called with save=False but its output needs a gradient")
     (x, ln_w, ln_b, w_qkv, b_qkv, w_out, b_out, rpb_table, rpb_dense, index_sample, mask, drop_scale, qkv, cbuf,
-     top) = ctx.saved_tensors
+     top, token_mask) = ctx.saved_tensors
     dx, d_ln_w, d_ln_b, d_wq, d_bq, d_wo, d_bo, d_rpb = torch.ops.lewin_b200.attn_bwd(
         dy, x, ln_w, ln_b, w_qkv, b_qkv, w_out, b_out, rpb_table, rpb_dense, index_sample, mask, drop_scale, qkv, cbuf, top,
-        *ctx.geom)
+        *ctx.geom, token_mask)
     has_ln, has_tab, has_dense = ctx.have
     return (dx, d_ln_w if has_ln else None, d_ln_b if has_ln else None, d_wq, d_bq, d_wo, d_bo,
             d_rpb if has_tab else None, d_rpb if (has_dense and not has_tab) else None,
-            None, None, None) + (None,) * 9
+            None, None, None) + (None,) * 10
 
 
 torch.library.register_autograd(f"{_NS}::attn_fwd", _attn_backward, setup_context=_attn_setup)
@@ -176,11 +179,11 @@ torch.library.register_autograd(f"{_NS}::leff_fwd", _leff_backward, setup_contex
 
 # --------------------------------------------------------------------------------- what ops.lewin_attn / lewin_leff call
 def lewin_attn(x, *, B, H, W, num_heads, shift, ln_w, ln_b, w_qkv, b_qkv, w_out, b_out, rpb_table, rpb_dense, index_sample,
-               mask, drop_scale, windowed, use_rpb, analytic_shift_mask, need):
+               mask, drop_scale, windowed, use_rpb, analytic_shift_mask, need, token_mask=None):
     index_sample = ops.prepare_index_sample(index_sample, x.device)
     y, top, _qkv, _ctx = torch.ops.lewin_b200.attn_fwd(
         x, ln_w, ln_b, w_qkv, b_qkv, w_out, b_out, rpb_table, rpb_dense, index_sample, mask, drop_scale, int(B), int(H), int(W),
-        int(num_heads), int(shift), bool(windowed), bool(use_rpb), bool(analytic_shift_mask), bool(need))
+        int(num_heads), int(shift), bool(windowed), bool(use_rpb), bool(analytic_shift_mask), bool(need), token_mask)
     return y, top
 
 

@@ -16,8 +16,8 @@
 //   -> LayerNorm in registers (same lane partition and summation order as gemm_ws's producers) -> swizzled UMMA A tile
 //   -> tcgen05.mma  [128 x C] x [C x 3C]  -> TMEM  -> + bias -> bf16 q | k | v tiles (XOR-swizzled 64-byte rows)
 //   -> ProbSparse core on mma.sync fragments, 4 warps per (window, head) item: the arithmetic of probsparse_core_v3.cuh
-//      (S = Q K^T, sparsity measure from the sample multiplicities, rank-count top-25, softmax -> +rpb -> +shift mask ->
-//      softmax, P.V, mean(V) fill), context rows written straight into the swizzled A tile of the second GEMM
+//      (S = Q K^T, sparsity measure from the sample multiplicities, rank-count top-25, softmax -> +rpb -> +shift / input
+//      mask -> softmax, P.V, mean(V) fill), context rows written straight into the swizzled A tile of the second GEMM
 //   -> tcgen05.mma  [128 x C] x [C x C]  -> TMEM  -> + bias, DropPath scale, + residual (x rows re-read through L2)
 //   -> per-warp staging -> row-cooperative coalesced stores through window_reverse + un-roll.
 //
@@ -53,6 +53,8 @@ struct Args {
     int tiles;                                // ceil(windows / 2)
     int tokens_per_image;
     WinMap map;
+    const float* tmask;                       // input mask per token [Bm, H, W] or null (LewinAttnFwdArgs::token_mask)
+    int Bm;
 };
 
 struct SetScratch {                           // per 4-warp set (one (window, head) item at a time)
@@ -61,8 +63,10 @@ struct SetScratch {                           // per 4-warp set (one (window, he
     int tok_of[32];
     alignas(8) int region[kTok];
     int mixed;
-    int pad[3];
+    int tm_live;                              // some token of the window has a non-zero input-mask value
+    int pad[2];
     alignas(16) __nv_bfloat16 vmean[kHeadDim];
+    alignas(16) float tm[kTok];               // input mask of the window's tokens (a.tmask)
 };
 
 template <int C>
@@ -117,7 +121,9 @@ __device__ __forceinline__ void bar_sync(int id, int n) { asm volatile("bar.sync
 // 8 consecutive rows of one chunk column hit 8 different bank groups -> conflict-free ldmatrix and row-per-lane stores)
 __device__ __forceinline__ uint32_t core_off(int row, int ch) { return static_cast<uint32_t>(row * 64 + ((ch ^ ((row >> 1) & 3)) << 4)); }
 
-template <int C>
+// TMASK: the call has an input mask per token (a.tmask).  A template parameter rather than a runtime branch: the kernel runs at
+// its register limit, and the unmasked instantiation keeps the code it had before the input mask existed.
+template <int C, bool TMASK>
 __global__ void __launch_bounds__(THREADS, 1) attn_fused_kernel(const Args a) {
     using Cf = Cfg<C>;
     constexpr int NH = Cf::NH, KC = Cf::KC, G = Cf::G, RPP = Cf::RPP, NP = Cf::NP;
@@ -411,6 +417,14 @@ __global__ void __launch_bounds__(THREADS, 1) attn_fused_kernel(const Args a) {
                     }
                     if (lane == 0) s.mixed = (a.mask_y0 + wy * 8 + 8 > a.mask_Hg - 8) || (wx * 8 + 8 > a.map.W - 8);
                 }
+                if (TMASK && sw == 1) {                          // input mask of this window's tokens (read in phase 3 only)
+                    const float m0 = window_token_mask(a.tmask, a.Bm, a.map.H, a.map.W, a.map.nWw, a.map.nWin, wg, lane);
+                    const float m1 = window_token_mask(a.tmask, a.Bm, a.map.H, a.map.W, a.map.nWw, a.map.nWin, wg, lane + 32);
+                    s.tm[lane] = m0;
+                    s.tm[lane + 32] = m1;
+                    const bool live = __any_sync(0xffffffffu, m0 != 0.f || m1 != 0.f);
+                    if (lane == 0) s.tm_live = live;
+                }
             }
             bar_sync(3 + 2 * g + set, 128);                        // [S2] slots assigned
             // ---- phase 3: slots 8*sw..+7 = rows 0..7 of this warp's m16 tile (rows 8..15 are dummies)
@@ -466,7 +480,23 @@ __global__ void __launch_bounds__(THREADS, 1) attn_fused_kernel(const Args a) {
 #pragma unroll
                     for (int j = 0; j < 8; ++j) { acc[j][0] += tb[-j * 15]; acc[j][1] += tb[-j * 15 - 1]; }
                 }
-                if (a.shift > 0 && s.mixed) {
+                if (TMASK && s.tm_live) {                         // input + shift mask, one add (== the dense sum)
+                    const float mr = s.tm[r];
+                    const bool sh = a.shift > 0 && s.mixed;
+                    const int rr = s.region[r];
+#pragma unroll
+                    for (int j = 0; j < 8; ++j) {
+                        const float2 mc = *reinterpret_cast<const float2*>(s.tm + j * 8 + 2 * tq);
+                        float m0 = token_mask_term(mr, mc.x), m1 = token_mask_term(mr, mc.y);
+                        if (sh) {
+                            const int2 rc = *reinterpret_cast<const int2*>(s.region + j * 8 + 2 * tq);
+                            m0 += (rc.x != rr) ? -100.0f : 0.f;
+                            m1 += (rc.y != rr) ? -100.0f : 0.f;
+                        }
+                        acc[j][0] += m0;
+                        acc[j][1] += m1;
+                    }
+                } else if (a.shift > 0 && s.mixed) {
                     const int rr = s.region[r];
 #pragma unroll
                     for (int j = 0; j < 8; ++j) {
@@ -614,9 +644,9 @@ inline bool supported(int C, int nH, long long tokens) {
     return (C == 32 || C == 64) && C == nH * kHeadDim && tokens >= 4 * TM && tokens < (1ll << 31);
 }
 
-template <int C>
+template <int C, bool TMASK>
 inline cudaError_t launch_c(const Args& a, int num_sms, cudaStream_t stream) {
-    auto k = attn_fused_kernel<C>;
+    auto k = attn_fused_kernel<C, TMASK>;
     cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg<C>::SMEM);
     if (e != cudaSuccess) return e;
     int grid = (a.tiles + GROUPS - 1) / GROUPS;
@@ -626,8 +656,8 @@ inline cudaError_t launch_c(const Args& a, int num_sms, cudaStream_t stream) {
 }
 
 inline cudaError_t launch(int C, const Args& a, int num_sms, cudaStream_t stream) {
-    if (C == 32) return launch_c<32>(a, num_sms, stream);
-    if (C == 64) return launch_c<64>(a, num_sms, stream);
+    if (C == 32) return a.tmask ? launch_c<32, true>(a, num_sms, stream) : launch_c<32, false>(a, num_sms, stream);
+    if (C == 64) return a.tmask ? launch_c<64, true>(a, num_sms, stream) : launch_c<64, false>(a, num_sms, stream);
     return cudaErrorInvalidValue;
 }
 

@@ -603,6 +603,7 @@ struct CoreBwdSmem {
     int tok_of[32];
     int slot_of[kTok];
     int region[kTok];
+    float tm[kTok];               // input mask of the window's tokens (a.tmask)
 };
 
 template <typename T, int D>
@@ -649,6 +650,7 @@ __global__ void __launch_bounds__(CORE_THREADS) probsparse_core_bwd_kernel(const
                 int cb = x < a.W - 8 ? 0 : (x < a.W - a.shift ? 1 : 2);
                 s.region[tid] = rb * 3 + cb;
             }
+            if (a.tmask && tid < kTok) s.tm[tid] = window_token_mask(a.tmask, a.Bm, a.H, a.W, a.nWw, a.nWin, wg, tid);
         }
         __syncthreads();
         if (tid < 32) {
@@ -730,7 +732,17 @@ __global__ void __launch_bounds__(CORE_THREADS) probsparse_core_bwd_kernel(const
                 const float* mrow = a.mask + (static_cast<long long>(wg % a.nW_mask) * kTok + r) * kTok;
                 p0 += mrow[lane]; p1v += mrow[lane + 32];
             }
-            if (a.shift > 0) {
+            if (a.tmask) {                       // input + shift mask, one add (as the forward)
+                const float mr = s.tm[r];
+                float m0 = token_mask_term(mr, s.tm[lane]), m1 = token_mask_term(mr, s.tm[lane + 32]);
+                if (a.shift > 0) {
+                    const int rr = s.region[r];
+                    m0 += (s.region[lane] != rr) ? -100.0f : 0.f;
+                    m1 += (s.region[lane + 32] != rr) ? -100.0f : 0.f;
+                }
+                p0 += m0;
+                p1v += m1;
+            } else if (a.shift > 0) {
                 const int rr = s.region[r];
                 p0 += (s.region[lane] != rr) ? -100.0f : 0.f;
                 p1v += (s.region[lane + 32] != rr) ? -100.0f : 0.f;
@@ -1004,6 +1016,14 @@ inline cudaError_t launch_dgrad_gemm(const GemmArgs<T>& g, __nv_bfloat16* wT_bf1
     return launch_gemm_any<T, EPI_BIAS>(g, st);
 }
 
+// LewinAttnFwdArgs::token_mask: the fused block half of a whole image only, never with the dense mask, Bm divides B
+inline int check_token_mask(const LewinAttnFwdArgs* a) {
+    if (!a->token_mask) return 0;
+    if (a->windowed || a->band_mode || a->mask || a->Bm <= 0 || a->B % a->Bm) return LEWIN_E_SHAPE;
+    if (reinterpret_cast<uintptr_t>(a->token_mask) & 15u) return LEWIN_E_ALIGN;
+    return 0;
+}
+
 template <typename T>
 int attn_bwd(const LewinAttnBwdArgs* a, void* ws, size_t ws_bytes, cudaStream_t st) {
     if (!a || !a->dy || !a->dx) return LEWIN_E_NULL;
@@ -1012,6 +1032,7 @@ int attn_bwd(const LewinAttnBwdArgs* a, void* ws, size_t ws_bytes, cudaStream_t 
     if (!a->d_w_qkv || !a->d_b_qkv || !a->d_w_out || !a->d_b_out) return LEWIN_E_NULL;
     if (!f.windowed && (!f.ln_w || !f.ln_b || !a->d_ln_w || !a->d_ln_b)) return LEWIN_E_NULL;
     if (f.H % 8 || f.W % 8 || f.C % 32 || !head_dim_ok(f.C, f.nH) || f.C > 1024 || f.nH > 16) return LEWIN_E_SHAPE;
+    if (int rc = check_token_mask(&f)) return rc;
     int sms = 0;
     if (int rc = bw_device(&sms)) return rc;
     const int dtype = Act<T>::kIsBf16 ? LEWIN_DTYPE_BF16 : LEWIN_DTYPE_F32;
@@ -1080,6 +1101,7 @@ int attn_bwd(const LewinAttnBwdArgs* a, void* ws, size_t ws_bytes, cudaStream_t 
         c.B_ = B_; c.nH = f.nH; c.C = C; c.use_rpb = f.use_rpb;
         c.shift = (f.analytic_shift_mask && !f.windowed) ? f.shift : 0;
         c.H = f.H; c.W = f.W; c.nWw = f.W / 8; c.nWin = nWin;
+        c.tmask = f.token_mask; c.Bm = f.token_mask ? f.Bm : 1;
         BCK(launch_core_bwd<T>(c, sms, st));
     }
     {   // dW_qkv += dqkv^T LN1(x)[window order] ; db_qkv += colsum(dqkv)

@@ -353,4 +353,16 @@ struct WinMap {
     }
 };
 
+// ---------------------------------------------------------------- input mask per token (LewinAttnFwdArgs::token_mask)
+// Value of token n of global window wg (batch-major) in the [Bm, H, W] level mask: image b takes mask b mod Bm, and the window
+// is partitioned in the UNSHIFTED frame (My_model_1.py:791-798 partitions the mask, not the rolled tokens).
+__device__ __forceinline__ float window_token_mask(const float* __restrict__ tm, int Bm, int H, int W, int nWw, int nWin, int wg, int n) {
+    const int b = wg / nWin, w = wg - b * nWin;
+    const int wy = w / nWw, wx = w - wy * nWw;
+    return tm[(static_cast<long long>(b % Bm) * H + wy * 8 + (n >> 3)) * W + wx * 8 + (n & 7)];
+}
+// Input-mask term of query token i and key token j: -100 where the fp32 product m_i * m_j is non-zero (NaN and inf included,
+// products that underflow to zero excluded), exactly as the reference's masked_fill(mask != 0, -100) on that product
+__device__ __forceinline__ float token_mask_term(float mi, float mj) { return __fmul_rn(mi, mj) != 0.f ? -100.0f : 0.f; }
+
 }  // namespace lewin

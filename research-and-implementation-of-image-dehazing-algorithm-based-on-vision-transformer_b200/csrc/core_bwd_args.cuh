@@ -16,6 +16,7 @@ struct CoreBwdArgs {
     const float* mask; int nW_mask;
     int B_, nH, C, use_rpb;
     int shift, H, W, nWw, nWin;
+    const float* tmask; int Bm;   // input mask per token [Bm, H, W] or null (CoreFwdArgs::tmask)
 };
 
 }  // namespace lewin

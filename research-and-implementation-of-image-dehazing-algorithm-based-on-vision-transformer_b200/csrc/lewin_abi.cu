@@ -105,6 +105,7 @@ int check_attn(const LewinAttnFwdArgs* a) {
     if (a->windowed && (a->shift != 0 || a->analytic_shift_mask)) return LEWIN_E_SHAPE;
     if (a->mask && a->nW_mask <= 0) return LEWIN_E_SHAPE;
     if (a->mask && ((a->B * (a->H / 8) * (a->W / 8)) % a->nW_mask)) return LEWIN_E_SHAPE;
+    if (int rc = check_token_mask(a)) return rc;
     const void* ps[] = {a->x, a->y, a->ln_w, a->ln_b, a->w_qkv, a->b_qkv, a->w_out, a->b_out, a->qkv, a->ctx, a->mask,
                         a->w_qkv_bf16, a->w_out_bf16};
     for (const void* p : ps)
@@ -202,6 +203,7 @@ int attn_fwd(const LewinAttnFwdArgs* a, void* ws, size_t ws_bytes, cudaStream_t 
         c.shift = (a->analytic_shift_mask && !a->windowed) ? a->shift : 0;
         c.H = a->H; c.W = a->W; c.nWw = a->W / 8; c.nWin = nWin;
         c.y0 = a->band_mode ? a->band_y0 : 0; c.Hg = a->band_mode ? a->band_Hg : a->H;
+        c.tmask = a->token_mask; c.Bm = a->token_mask ? a->Bm : 1;
         kt.begin(LEWIN_ATTN_K_CORE);
         CK(launch_core_fwd<T>(c, di.sms, stream));
         kt.end(LEWIN_ATTN_K_CORE);

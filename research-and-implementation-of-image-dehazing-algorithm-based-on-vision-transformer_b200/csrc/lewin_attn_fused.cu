@@ -28,6 +28,7 @@ int attn_fused_launch(const LewinAttnFwdArgs* a, int num_sms, cudaStream_t strea
     k.map = WinMap{a->H, a->W, a->W / 8, nWin, a->shift, a->band_mode ? 0 : a->shift};
     k.mask_y0 = a->band_mode ? a->band_y0 : 0;
     k.mask_Hg = a->band_mode ? a->band_Hg : a->H;
+    k.tmask = a->token_mask; k.Bm = a->token_mask ? a->Bm : 1;
     return static_cast<int>(af::launch(a->C, k, num_sms, stream));
 }
 

@@ -32,6 +32,9 @@ struct CoreFwdArgs {
     // image Hg rows tall (y0 = 0, Hg = H unless the map is a row band of a taller image)
     int shift, H, W, nWw, nWin;
     int y0, Hg;
+    // input mask per token [Bm, H, W] (LewinAttnFwdArgs::token_mask) or null; its term and the shift mask's are one add
+    const float* tmask;
+    int Bm;
 };
 
 constexpr int CORE_THREADS = 128;
@@ -54,6 +57,7 @@ struct CoreSmem {
     int slot_of[kTok];            // token -> slot (or -1)
     int tok_of[32];               // slot -> token
     int region[kTok];
+    float tm[kTok];               // input mask of the window's tokens (a.tmask)
 };
 
 // cnt[n][m] = #{t : idx[n, t] == m} (the reference's K_sample gather, attn.py:88-104, as a multiplicity matrix), built in
@@ -112,6 +116,7 @@ __global__ void __launch_bounds__(CORE_THREADS) probsparse_core_fwd_kernel(const
                 int cb = x < a.W - 8 ? 0 : (x < a.W - a.shift ? 1 : 2);
                 s.region[tid] = rb * 3 + cb;
             }
+            if (a.tmask && tid < kTok) s.tm[tid] = window_token_mask(a.tmask, a.Bm, a.H, a.W, a.nWw, a.nWin, wg, tid);
         }
         __syncthreads();
 
@@ -232,7 +237,17 @@ __global__ void __launch_bounds__(CORE_THREADS) probsparse_core_fwd_kernel(const
                 p0 += mrow[lane];
                 p1 += mrow[lane + 32];
             }
-            if (a.shift > 0) {
+            if (a.tmask) {                                       // input + shift mask, one add (== the dense sum)
+                const float mr = s.tm[r];
+                float m0 = token_mask_term(mr, s.tm[lane]), m1 = token_mask_term(mr, s.tm[lane + 32]);
+                if (a.shift > 0) {
+                    const int rr = s.region[r];
+                    m0 += (s.region[lane] != rr) ? -100.0f : 0.f;
+                    m1 += (s.region[lane + 32] != rr) ? -100.0f : 0.f;
+                }
+                p0 += m0;
+                p1 += m1;
+            } else if (a.shift > 0) {
                 const int rr = s.region[r];
                 p0 += (s.region[lane] != rr) ? -100.0f : 0.f;
                 p1 += (s.region[lane + 32] != rr) ? -100.0f : 0.f;

@@ -31,8 +31,12 @@ struct Smem {
     alignas(8) int region[kTok];
     int mixed;
     float tacc[16 * 225];                               // d(rpb table) partials per head
+    alignas(16) float tm[kTok];                         // input mask of the window's tokens (a.tmask)
+    int tm_live[2];                                     // per staging warp: some token has a non-zero input-mask value
 };
 
+// TMASK: the call has an input mask per token (a.tmask); a template parameter, as in probsparse_core_v3_kernel
+template <bool TMASK>
 __global__ void __launch_bounds__(THREADS, 3) core_bwd_v2_kernel(const CoreBwdArgs<__nv_bfloat16> a) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     Smem& s = *reinterpret_cast<Smem*>(smem_raw);
@@ -85,11 +89,17 @@ __global__ void __launch_bounds__(THREADS, 3) core_bwd_v2_kernel(const CoreBwdAr
             s.region[tid] = rb * 3 + cb;
             if (tid == 0) s.mixed = (wy * 8 + 8 > a.H - 8) || (wx * 8 + 8 > a.W - 8);
         }
+        if (TMASK && tid < kTok) {
+            const float m = window_token_mask(a.tmask, a.Bm, a.H, a.W, a.nWw, a.nWin, wg, tid);
+            s.tm[tid] = m;
+            const bool live = __any_sync(0xffffffffu, m != 0.f);
+            if (lane == 0) s.tm_live[warp] = live;
+        }
         // membership mask of the selected tokens (uniform in the warp)
         unsigned long long selmask = my_sel >= 0 ? (1ull << my_sel) : 0ull;
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) selmask |= __shfl_xor_sync(0xffffffffu, selmask, o);
-        const bool need_tbl_sync = (a.use_rpb && a.rpb_table) || a.shift > 0;
+        const bool need_tbl_sync = (a.use_rpb && a.rpb_table) || a.shift > 0 || TMASK;
         if (need_tbl_sync) __syncthreads();                                     // [B2] bias table / region of this item visible
 
         const int my_tok = __shfl_sync(0xffffffffu, my_sel, (warp * 8 + gq) & 31);          // token of my fragment row (-1: dummy)
@@ -165,7 +175,23 @@ __global__ void __launch_bounds__(THREADS, 3) core_bwd_v2_kernel(const CoreBwdAr
 #pragma unroll
                 for (int j = 0; j < 8; ++j) { const float2 m2 = *reinterpret_cast<const float2*>(mk + j * 8); x[j][0] += m2.x; x[j][1] += m2.y; }
             }
-            if (a.shift > 0 && s.mixed) {
+            if (TMASK && (s.tm_live[0] | s.tm_live[1])) {                  // input + shift mask, one add (as the forward)
+                const float mr = s.tm[r];
+                const bool sh = a.shift > 0 && s.mixed;
+                const int rr = s.region[r];
+#pragma unroll
+                for (int j = 0; j < 8; ++j) {
+                    const float2 mc = *reinterpret_cast<const float2*>(s.tm + j * 8 + 2 * tq);
+                    float m0 = token_mask_term(mr, mc.x), m1 = token_mask_term(mr, mc.y);
+                    if (sh) {
+                        const int2 rc = *reinterpret_cast<const int2*>(s.region + j * 8 + 2 * tq);
+                        m0 += (rc.x != rr) ? -100.0f : 0.f;
+                        m1 += (rc.y != rr) ? -100.0f : 0.f;
+                    }
+                    x[j][0] += m0;
+                    x[j][1] += m1;
+                }
+            } else if (a.shift > 0 && s.mixed) {
                 const int rr = s.region[r];
 #pragma unroll
                 for (int j = 0; j < 8; ++j) {
@@ -346,7 +372,7 @@ __global__ void __launch_bounds__(THREADS, 3) core_bwd_v2_kernel(const CoreBwdAr
 }
 
 inline cudaError_t launch(const CoreBwdArgs<__nv_bfloat16>& a, int num_sms, cudaStream_t stream) {
-    auto k = core_bwd_v2_kernel;
+    auto k = a.tmask ? core_bwd_v2_kernel<true> : core_bwd_v2_kernel<false>;
     const size_t smem = sizeof(Smem);
     cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
     if (e != cudaSuccess) return e;

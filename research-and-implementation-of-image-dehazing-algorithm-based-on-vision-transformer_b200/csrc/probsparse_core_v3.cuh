@@ -37,8 +37,13 @@ struct Smem {
     int mixed;                                          // window crosses a shift-mask region border
     alignas(16) __nv_bfloat16 vmean[kHeadDim];
     alignas(16) __nv_bfloat16 ostage[4][8 * kHeadDim];              // per-warp staging of the 8 selected context rows
+    alignas(16) float tm[kTok];                         // input mask of the window's tokens (a.tmask)
+    int tm_live[2];                                     // per staging warp: some token has a non-zero mask value
 };
 
+// TMASK: the call has an input mask per token (a.tmask).  A template parameter rather than a runtime branch, so that the
+// unmasked instantiation is the issue-bound code it was before the input mask existed.
+template <bool TMASK>
 __global__ void __launch_bounds__(THREADS, CTAS) probsparse_core_v3_kernel(const CoreFwdArgs<__nv_bfloat16> a) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     Smem& s = *reinterpret_cast<Smem*>(smem_raw);
@@ -115,6 +120,12 @@ __global__ void __launch_bounds__(THREADS, CTAS) probsparse_core_v3_kernel(const
                     s.mixed = (a.y0 + wy0 * 8 + 8 > a.Hg - 8) || (wx0 * 8 + 8 > a.W - 8);
                 }
             }
+        }
+        if (TMASK && tid < kTok) {
+            const float m = window_token_mask(a.tmask, a.Bm, a.H, a.W, a.nWw, a.nWin, wg, tid);
+            s.tm[tid] = m;
+            const bool live = __any_sync(0xffffffffu, m != 0.f);        // all-zero windows: every product is zero
+            if (lane == 0) s.tm_live[warp] = live;
         }
 
         // ================= phase 1: S = Q K^T for rows 16*warp..+15, sparsity measure M (attn.py:71-117)
@@ -252,7 +263,23 @@ __global__ void __launch_bounds__(THREADS, CTAS) probsparse_core_v3_kernel(const
 #pragma unroll
                 for (int j = 0; j < 8; ++j) { const float2 m2 = *reinterpret_cast<const float2*>(mk + j * 8); acc[j][0] += m2.x; acc[j][1] += m2.y; }
             }
-            if (a.shift > 0 && s.mixed) {
+            if (TMASK && (s.tm_live[0] | s.tm_live[1])) {                  // input + shift mask, one add (== the dense sum)
+                const float mr = s.tm[r];
+                const bool sh = a.shift > 0 && s.mixed;
+                const int rr = s.region[r];
+#pragma unroll
+                for (int j = 0; j < 8; ++j) {
+                    const float2 mc = *reinterpret_cast<const float2*>(s.tm + j * 8 + 2 * tq);
+                    float m0 = token_mask_term(mr, mc.x), m1 = token_mask_term(mr, mc.y);
+                    if (sh) {
+                        const int2 rc = *reinterpret_cast<const int2*>(s.region + j * 8 + 2 * tq);
+                        m0 += (rc.x != rr) ? -100.0f : 0.f;
+                        m1 += (rc.y != rr) ? -100.0f : 0.f;
+                    }
+                    acc[j][0] += m0;
+                    acc[j][1] += m1;
+                }
+            } else if (a.shift > 0 && s.mixed) {
                 const int rr = s.region[r];
 #pragma unroll
                 for (int j = 0; j < 8; ++j) {
@@ -333,7 +360,7 @@ __global__ void __launch_bounds__(THREADS, CTAS) probsparse_core_v3_kernel(const
 }
 
 inline cudaError_t launch(const CoreFwdArgs<__nv_bfloat16>& a, int num_sms, cudaStream_t stream) {
-    auto k = probsparse_core_v3_kernel;
+    auto k = a.tmask ? probsparse_core_v3_kernel<true> : probsparse_core_v3_kernel<false>;
     const size_t smem = sizeof(Smem);
     cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
     if (e != cudaSuccess) return e;

@@ -274,31 +274,6 @@ class LeFF(nn.Module):
 
 
 # ------------------------------------------------------------------------------ LeWin block
-def input_attn_mask(mask, H, W, win_size, dtype=torch.float32):
-    """Host-side restatement of My_model_1.py:791-798 (only reached from test_in_any_resolution.py:106)."""
-    m = torch.nn.functional.interpolate(mask, size=(H, W)).permute(0, 2, 3, 1)
-    B = m.shape[0]
-    mw = m.view(B, H // win_size, win_size, W // win_size, win_size, 1).permute(0, 1, 3, 2, 4, 5)
-    mw = mw.reshape(-1, win_size * win_size)
-    am = mw.unsqueeze(2) * mw.unsqueeze(1)
-    return am.masked_fill(am != 0, -100.0).masked_fill(am == 0, 0.0).to(dtype)
-
-
-def dense_shift_mask(H, W, win_size, shift, device, dtype=torch.float32):
-    """Materialised shift mask, My_model_1.py:803-836 (used only when an input mask must be combined)."""
-    img = torch.zeros((1, H, W, 1), device=device)
-    sl = (slice(0, -win_size), slice(-win_size, -shift), slice(-shift, None))
-    cnt = 0
-    for h in sl:
-        for w in sl:
-            img[:, h, w, :] = cnt
-            cnt += 1
-    mw = img.view(1, H // win_size, win_size, W // win_size, win_size, 1).permute(0, 1, 3, 2, 4, 5)
-    mw = mw.reshape(-1, win_size * win_size)
-    d = mw.unsqueeze(1) - mw.unsqueeze(2)
-    return d.masked_fill(d != 0, -100.0).masked_fill(d == 0, 0.0).to(dtype)
-
-
 def lewin_block_forward(blk, x, mask=None, index_sample=None, out=None):
     """LeWinTransformerBlock.forward (My_model_1.py:785-875) on the sm_100a ops.
 
@@ -314,13 +289,11 @@ def lewin_block_forward(blk, x, mask=None, index_sample=None, out=None):
         index_sample = draw_index_sample(64, 64)            # same point in the RNG stream as attn.py:91
     dt = _act_dtype(x)
     x = x.to(dt)
-    dense = None
-    analytic = True
+    token_mask = None
     if mask is not None:                                    # input-mask path (test_in_any_resolution.py:106)
-        dense = input_attn_mask(mask, H, W, blk.win_size)
-        if blk.shift_size > 0:
-            dense = dense + dense_shift_mask(H, W, blk.win_size, blk.shift_size, x.device)
-            analytic = False
+        # My_model_1.py:791-792: the nearest-resized level mask, one value per token; the window partition and the pairwise
+        # product (:793-798) are evaluated inside the attention kernels, together with the analytic shift mask
+        token_mask = torch.nn.functional.interpolate(mask, size=(H, W))[:, 0]
     dp = blk.drop_path
     s0 = dp.sample_scale(x) if isinstance(dp, DropPath) else _foreign_droppath_scale(dp, x)
     if hasattr(ps, "qkv_weights"):
@@ -331,8 +304,8 @@ def lewin_block_forward(blk, x, mask=None, index_sample=None, out=None):
         x, B=B, H=H, W=W, num_heads=blk.num_heads, shift=blk.shift_size,
         ln_w=blk.norm1.weight, ln_b=blk.norm1.bias, w_qkv=w_qkv, b_qkv=b_qkv,
         w_out=ps.out_projection.weight, b_out=ps.out_projection.bias,
-        rpb_table=blk.attn.relative_position_bias_table, index_sample=index_sample, mask=dense,
-        drop_scale=s0, windowed=False, use_rpb=_use_rpb(), analytic_shift_mask=analytic)
+        rpb_table=blk.attn.relative_position_bias_table, index_sample=index_sample, token_mask=token_mask,
+        drop_scale=s0, windowed=False, use_rpb=_use_rpb(), analytic_shift_mask=True)
     s1 = dp.sample_scale(y) if isinstance(dp, DropPath) else _foreign_droppath_scale(dp, y)
     mlp = blk.mlp
     return ops.lewin_leff(

@@ -197,10 +197,22 @@ def _bf16_image(w):
     return weight_images.get(w)
 
 
-def _attn_forward(x, ln_w, ln_b, w_qkv, b_qkv, w_out, b_out, rpb_table, rpb_dense, index_sample, mask, drop_scale, geom):
+def _token_mask(token_mask, B, H, W, device):
+    """The input mask per token as it crosses the ABI: contiguous fp32 [Bm, H, W] on the activations' device, Bm | B."""
+    if token_mask is None:
+        return None
+    tm = token_mask.to(device=device, dtype=torch.float32).contiguous()
+    if tm.dim() != 3 or tuple(tm.shape[1:]) != (H, W) or tm.shape[0] < 1 or B % tm.shape[0]:
+        raise RuntimeError(f"lewin_b200.lewin_attn: token_mask must be [Bm, {H}, {W}] with Bm dividing B = {B}, "
+                           f"got {tuple(token_mask.shape)}")
+    return tm
+
+
+def _attn_forward(x, ln_w, ln_b, w_qkv, b_qkv, w_out, b_out, rpb_table, rpb_dense, index_sample, mask, drop_scale, geom,
+                  token_mask=None):
     """One lewin_attn_fwd_* call.  Returns (y, top, saved): ``saved`` is what the backward call needs (the fp32 parameter
-    tensors as they crossed the ABI, the int32 sample indices, q|k|v, ctx, top).  Shared by the autograd.Function below and
-    the torch.library ops of compile_ops.py."""
+    tensors as they crossed the ABI, the int32 sample indices, q|k|v, ctx, top, the token mask).  Shared by the
+    autograd.Function below and the torch.library ops of compile_ops.py."""
     B, H, W, nH, shift, windowed, use_rpb, analytic, need_grad = geom[:9]
     band = geom[9] if len(geom) > 9 else None          # (y0, Hg): row band of a taller image (forward only)
     lib = _lib.load()
@@ -215,6 +227,7 @@ def _attn_forward(x, ln_w, ln_b, w_qkv, b_qkv, w_out, b_out, rpb_table, rpb_dens
     params = [_f32c(t) for t in (ln_w, ln_b, w_qkv, b_qkv, w_out, b_out, rpb_table, rpb_dense, mask, drop_scale)]
     ln_w_, ln_b_, w_qkv_, b_qkv_, w_out_, b_out_, tab_, dense_, mask_, ds_ = params
     idx = prepare_index_sample(index_sample, dev)
+    tm = _token_mask(token_mask, B, H, W, dev)
     a = _lib.LewinAttnFwdArgs(
         B=B, H=H, W=W, C=C, nH=nH, shift=shift, windowed=int(windowed), use_rpb=int(use_rpb),
         analytic_shift_mask=int(analytic), nW_mask=0 if mask_ is None else mask_.shape[0],
@@ -222,7 +235,7 @@ def _attn_forward(x, ln_w, ln_b, w_qkv, b_qkv, w_out, b_out, rpb_table, rpb_dens
         x=_ptr(x), y=_ptr(y), ln_w=_ptr(ln_w_), ln_b=_ptr(ln_b_), w_qkv=_ptr(w_qkv_), b_qkv=_ptr(b_qkv_),
         w_out=_ptr(w_out_), b_out=_ptr(b_out_), rpb_table=_ptr(tab_), rpb_dense=_ptr(dense_),
         index_sample=_ptr(idx), mask=_ptr(mask_), drop_scale=_ptr(ds_),
-        qkv=None, ctx=None, top=_ptr(top))
+        qkv=None, ctx=None, top=_ptr(top), token_mask=_ptr(tm), Bm=0 if tm is None else tm.shape[0])
     if band is not None:
         if need_grad:
             raise RuntimeError("lewin_b200.lewin_attn: row-band mode is forward only")
@@ -248,13 +261,13 @@ def _attn_forward(x, ln_w, ln_b, w_qkv, b_qkv, w_out, b_out, rpb_table, rpb_dens
         _lib.check(fn(a, ws.data_ptr(), ws.numel(), _stream()), f"lewin_attn_fwd_{dt}")
     if TopRecorder.active is not None:
         TopRecorder.active.tops.append(top)
-    return y, top, (x, ln_w_, ln_b_, w_qkv_, b_qkv_, w_out_, b_out_, tab_, dense_, idx, mask_, ds_, qkv, cbuf, top)
+    return y, top, (x, ln_w_, ln_b_, w_qkv_, b_qkv_, w_out_, b_out_, tab_, dense_, idx, mask_, ds_, qkv, cbuf, top, tm)
 
 
 def _attn_backward(saved, geom, dy, separate_grads=False):
     """One lewin_attn_bwd_* call on the tensors _attn_forward saved -> (dx, d_ln_w, d_ln_b, d_w_qkv, d_b_qkv, d_w_out, d_b_out,
     d_rpb_table, d_rpb_dense); entries of absent parameters are None."""
-    (x, ln_w, ln_b, w_qkv, b_qkv, w_out, b_out, tab, dense, idx, mask, ds, qkv, cbuf, top) = saved
+    (x, ln_w, ln_b, w_qkv, b_qkv, w_out, b_out, tab, dense, idx, mask, ds, qkv, cbuf, top, tm) = saved
     B, H, W, nH, shift, windowed, use_rpb, analytic, _ = geom[:9]
     lib = _lib.load()
     dt = _dtype_tag(x)
@@ -271,7 +284,7 @@ def _attn_backward(saved, geom, dy, separate_grads=False):
         x=_ptr(x), y=None, ln_w=_ptr(ln_w), ln_b=_ptr(ln_b), w_qkv=_ptr(w_qkv), b_qkv=_ptr(b_qkv),
         w_out=_ptr(w_out), b_out=_ptr(b_out), rpb_table=_ptr(tab), rpb_dense=_ptr(dense),
         index_sample=_ptr(idx), mask=_ptr(mask), drop_scale=_ptr(ds),
-        qkv=_ptr(qkv), ctx=_ptr(cbuf), top=_ptr(top))
+        qkv=_ptr(qkv), ctx=_ptr(cbuf), top=_ptr(top), token_mask=_ptr(tm), Bm=0 if tm is None else tm.shape[0])
     a = _lib.LewinAttnBwdArgs(
         fwd=fwd, dy=_ptr(dy), dx=_ptr(dx), d_ln_w=_ptr(d_ln_w), d_ln_b=_ptr(d_ln_b),
         d_w_qkv=_ptr(d_w_qkv), d_b_qkv=_ptr(d_b_qkv), d_w_out=_ptr(d_w_out), d_b_out=_ptr(d_b_out),
@@ -288,9 +301,9 @@ def _attn_backward(saved, geom, dy, separate_grads=False):
 class _AttnFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, ln_w, ln_b, w_qkv, b_qkv, w_out, b_out, rpb_table, rpb_dense, index_sample, mask,
-                drop_scale, geom):
+                drop_scale, geom, token_mask=None):
         y, top, saved = _attn_forward(x, ln_w, ln_b, w_qkv, b_qkv, w_out, b_out, rpb_table, rpb_dense, index_sample, mask,
-                                      drop_scale, geom)
+                                      drop_scale, geom, token_mask)
         ctx.geom = geom
         ctx.save_for_backward(*saved)
         ctx.mark_non_differentiable(top)
@@ -298,7 +311,7 @@ class _AttnFn(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, dy, _dtop):
-        return _attn_backward(ctx.saved_tensors, ctx.geom, dy) + (None, None, None, None)
+        return _attn_backward(ctx.saved_tensors, ctx.geom, dy) + (None, None, None, None, None)
 
 
 def _leff_forward(y, ln_w, ln_b, w1, b1, w_dw, b_dw, w2, b2, drop_scale, geom, out_view=None):
@@ -390,8 +403,11 @@ class _LeffFn(torch.autograd.Function):
 
 def lewin_attn(x, *, B, H, W, num_heads, shift, ln_w, ln_b, w_qkv, b_qkv, w_out, b_out,
                rpb_table=None, rpb_dense=None, index_sample, mask=None, drop_scale=None,
-               windowed=False, use_rpb=True, analytic_shift_mask=True, return_top=False, band=None):
+               windowed=False, use_rpb=True, analytic_shift_mask=True, return_top=False, band=None, token_mask=None):
     """Attention half of a LeWin block.  Returns y (same shape as x) [and the selected top-u indices].
+    token_mask: the input mask as one value per token, [Bm, H, W] with Bm | B (image b uses mask b mod Bm): the nearest-resized
+    mask of My_model_1.py:791-798, evaluated inside the kernels in place of the dense [B*nW, 64, 64] mask the reference builds
+    (fused block half only; combined with the analytic shift mask).
     band=(y0, Hg): x is a band of H rows, already in shifted-frame row order, of an image Hg rows tall whose shifted-frame
     row y0 is the band's first row (canvas-mode row sharding, fullres / canvas_bands; forward only)."""
     need = torch.is_grad_enabled() and any(
@@ -403,10 +419,11 @@ def lewin_attn(x, *, B, H, W, num_heads, shift, ln_w, ln_b, w_qkv, b_qkv, w_out,
         y, top = compile_ops.lewin_attn(x, B=B, H=H, W=W, num_heads=num_heads, shift=shift, ln_w=ln_w, ln_b=ln_b, w_qkv=w_qkv,
                                         b_qkv=b_qkv, w_out=w_out, b_out=b_out, rpb_table=rpb_table, rpb_dense=rpb_dense,
                                         index_sample=index_sample, mask=mask, drop_scale=drop_scale, windowed=windowed,
-                                        use_rpb=use_rpb, analytic_shift_mask=analytic_shift_mask, need=need)
+                                        use_rpb=use_rpb, analytic_shift_mask=analytic_shift_mask, need=need,
+                                        token_mask=token_mask)
         return (y, top) if return_top else y
     y, top = _AttnFn.apply(x, ln_w, ln_b, w_qkv, b_qkv, w_out, b_out, rpb_table, rpb_dense, index_sample, mask,
-                           drop_scale, geom)
+                           drop_scale, geom, token_mask)
     return (y, top) if return_top else y
 
 
