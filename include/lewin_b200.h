@@ -39,7 +39,7 @@ extern "C" {
 typedef struct CUstream_st* lewin_stream_t; /* == cudaStream_t */
 typedef struct CUevent_st*  lewin_event_t;  /* == cudaEvent_t  */
 
-#define LEWIN_ABI_VERSION 6
+#define LEWIN_ABI_VERSION 7
 
 /* error codes (negative) */
 #define LEWIN_E_NULL      (-1)  /* a required pointer is NULL */
@@ -152,7 +152,14 @@ int lewin_attn_fwd_bf16(const LewinAttnFwdArgs* a, void* workspace, size_t works
 /* Backward of the attention half (autograd of the same reference lines; gradient paths in
  * SURVEY.md section 3.4).  Gradients of parameters are ACCUMULATED (+=) into fp32 buffers the
  * caller zero-initialises, dx is written.  Shapes as the forward's (C % 32 == 0, C <= 1024,
- * head_dim = C / nH in {32, 64, 128}) with nH <= 16; anything else returns LEWIN_E_SHAPE. */
+ * head_dim = C / nH in {32, 64, 128}) with nH <= 16; anything else returns LEWIN_E_SHAPE.
+ *
+ * `deterministic` (all three backward structs): 0 = parameter gradients are summed with fp32 atomics, whose order varies from
+ * run to run.  1 = every parameter gradient of the call is a fixed-order sum: each reduction unit stores its partial into its
+ * own slot of a workspace slab, and one reduction launch at the end of the call sums the slots in order and adds the result
+ * ONCE into the caller's buffer (still accumulated).  The slot counts depend on the shape alone, so the bits are the same on
+ * any sm_100 device.  The data gradients (dx / dy / dqkv) are the same in both modes.  The *_workspace_bytes queries read the
+ * flag (the slabs are included with 1).  torch.use_deterministic_algorithms(True) sets it from the Python layer. */
 typedef struct {
     LewinAttnFwdArgs fwd;          /* same tensors as the forward call (x, params, qkv, ctx, top, ...) */
     const void* dy;                /* same shape/dtype as y */
@@ -163,6 +170,8 @@ typedef struct {
     float* d_rpb_table;            /* [225, nH] (when fwd.rpb_table is given) */
     float* d_rpb_dense;            /* [nH, 64, 64] gradient w.r.t. the gathered bias (when fwd.rpb_dense is given: the
                                       relative_position_bias argument of AttentionLayer.forward, attn.py:385), or NULL */
+    int32_t deterministic;         /* 1: fixed-order parameter-gradient sums (see above) */
+    int32_t reserved;
 } LewinAttnBwdArgs;
 
 int lewin_attn_bwd_f32 (const LewinAttnBwdArgs* a, void* workspace, size_t workspace_bytes, lewin_stream_t stream);
@@ -192,13 +201,16 @@ size_t lewin_probsparse_core_fwd_workspace_bytes(const LewinCoreFwdArgs* a, int 
 
 /* Backward of ProbAttention.forward (what autograd derives from attn.py:287-342, SURVEY.md section 3.4) for the
  * selection saved by the forward (`fwd.top`, required): dqkv [B_*64, 3C] is WRITTEN (dq is zero on the lazy rows),
- * the bias gradients are ACCUMULATED into fp32 buffers the caller zero-initialises (either may be NULL). */
+ * the bias gradients are ACCUMULATED into fp32 buffers the caller zero-initialises (either may be NULL).  The workspace is
+ * empty unless `deterministic` is 1. */
 typedef struct {
     LewinCoreFwdArgs fwd;          /* same qkv / rpb / mask / top as the forward call (index_sample, ctx unused) */
     const void* dctx;              /* [B_*64, C] gradient of the returned context */
     void*       dqkv;              /* [B_*64, 3C] */
     float*      d_rpb_table;       /* [225, nH], used when fwd.rpb_table is given */
     float*      d_rpb_dense;       /* [nH, 64, 64], used when fwd.rpb_dense is given */
+    int32_t     deterministic;     /* 1: fixed-order bias-gradient sums (see LewinAttnBwdArgs) */
+    int32_t     reserved;
 } LewinCoreBwdArgs;
 
 int lewin_probsparse_core_bwd_f32 (const LewinCoreBwdArgs* a, void* workspace, size_t workspace_bytes, lewin_stream_t stream);
@@ -259,7 +271,8 @@ int lewin_leff_fwd_supports_ld_out(const LewinLeffFwdArgs* a, int dtype);
 int lewin_leff_fwd_f32 (const LewinLeffFwdArgs* a, void* workspace, size_t workspace_bytes, lewin_stream_t stream);
 int lewin_leff_fwd_bf16(const LewinLeffFwdArgs* a, void* workspace, size_t workspace_bytes, lewin_stream_t stream);
 
-/* Backward of the LeFF half: parameter gradients ACCUMULATED into zero-initialised fp32 buffers, dy written.
+/* Backward of the LeFF half: parameter gradients ACCUMULATED into zero-initialised fp32 buffers (with `deterministic` = 1 as
+ * fixed-order sums, see LewinAttnBwdArgs), dy written.
  * C % 32 == 0, hidden % 32 == 0, C <= 1024 (as the forward); anything else returns LEWIN_E_SHAPE. */
 typedef struct {
     LewinLeffFwdArgs fwd;
@@ -269,6 +282,8 @@ typedef struct {
     float* d_w1;   float* d_b1;
     float* d_w_dw; float* d_b_dw;
     float* d_w2;   float* d_b2;
+    int32_t deterministic;         /* 1: fixed-order parameter-gradient sums (see LewinAttnBwdArgs) */
+    int32_t reserved;
 } LewinLeffBwdArgs;
 
 int lewin_leff_bwd_f32 (const LewinLeffBwdArgs* a, void* workspace, size_t workspace_bytes, lewin_stream_t stream);

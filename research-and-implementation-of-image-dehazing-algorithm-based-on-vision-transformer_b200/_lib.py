@@ -40,6 +40,7 @@ class LewinAttnBwdArgs(C.Structure):
         ("dy", c_ptr), ("dx", c_ptr),
         ("d_ln_w", c_ptr), ("d_ln_b", c_ptr), ("d_w_qkv", c_ptr), ("d_b_qkv", c_ptr),
         ("d_w_out", c_ptr), ("d_b_out", c_ptr), ("d_rpb_table", c_ptr), ("d_rpb_dense", c_ptr),
+        ("deterministic", C.c_int32), ("reserved", C.c_int32),
     ]
 
 
@@ -56,6 +57,7 @@ class LewinCoreBwdArgs(C.Structure):
     _fields_ = [
         ("fwd", LewinCoreFwdArgs),
         ("dctx", c_ptr), ("dqkv", c_ptr), ("d_rpb_table", c_ptr), ("d_rpb_dense", c_ptr),
+        ("deterministic", C.c_int32), ("reserved", C.c_int32),
     ]
 
 
@@ -78,6 +80,7 @@ class LewinLeffBwdArgs(C.Structure):
         ("dout", c_ptr), ("dy", c_ptr),
         ("d_ln_w", c_ptr), ("d_ln_b", c_ptr), ("d_w1", c_ptr), ("d_b1", c_ptr),
         ("d_w_dw", c_ptr), ("d_b_dw", c_ptr), ("d_w2", c_ptr), ("d_b2", c_ptr),
+        ("deterministic", C.c_int32), ("reserved", C.c_int32),
     ]
 
 
@@ -137,7 +140,7 @@ EXPORTS = (
     "lewin_output_proj_fwd_bf16", "lewin_output_proj_fwd_workspace_bytes",
 )
 
-ABI_VERSION = 6
+ABI_VERSION = 7
 DTYPE_TAG = {"f32": 0, "bf16": 1}
 
 _lib = None

@@ -7,6 +7,14 @@
 //   dwconv_bwd_kernel     depthwise 3x3 backward (data + weight + bias) with both GELU derivatives fused
 //   probsparse_core_bwd   dq, dk, dv and d(rpb table) of the ProbSparse core for the saved top-u selection
 //   transpose_kernel      W -> W^T staging for the data-gradient GEMMs (gemm_fused_kernel)
+//   det_reduce_kernel     deterministic mode: the per-unit partial slabs of one backward call, summed in slot order
+//
+// Deterministic mode (LewinAttnBwdArgs::deterministic etc.): every kernel above that adds into a parameter gradient has a
+// DET = true instantiation in which each reduction unit (a token split of a weight-gradient tile, a CTA of a persistent
+// kernel) stores its partial into its own slot of a workspace slab with the gradient's extent; inside a CTA partials are
+// merged in warp order, never through atomics.  The slot counts are functions of the shape alone (grids sized for a fixed
+// 148 SMs), so the workspace is host arithmetic and the bits do not depend on the device's SM count.  DET = false is the
+// default code, unchanged.
 #pragma once
 #include "../../include/lewin_b200.h"
 #include "common.cuh"
@@ -48,7 +56,7 @@ inline cudaError_t launch_transpose(const float* src, float* dst, int R, int Cc,
 constexpr int WG_BM = 32;             // tokens per stage
 constexpr int WG_THREADS = 256;
 
-template <typename T, int TILE>       // TILE = 64 or 32: dW tile is TILE x TILE
+template <typename T, int TILE, bool DET = false>       // TILE = 64 or 32: dW tile is TILE x TILE.  DET: slabs [splits][N, K]
 __global__ void __launch_bounds__(WG_THREADS) wgrad_kernel(const WgradArgs<T> g) {
     constexpr int PASSES = Act<T>::kPasses;
     constexpr int LD = TILE + 8;                  // (8t + g) % 32 distinct -> conflict-free transposed fragment loads
@@ -157,6 +165,21 @@ __global__ void __launch_bounds__(WG_THREADS) wgrad_kernel(const WgradArgs<T> g)
                 for (int j = 0; j < NT; ++j) mma_x<PASSES>(acc[i][j], af[i], bf[j]);
         }
     }
+    if constexpr (DET) {
+        float* dW = g.dW + static_cast<long long>(blockIdx.z) * g.N * g.K;
+#pragma unroll
+        for (int i = 0; i < MT; ++i)
+#pragma unroll
+            for (int j = 0; j < NT; ++j)
+#pragma unroll
+                for (int half = 0; half < 2; ++half) {
+                    const int n = n0 + wn * WN + i * 16 + gq + half * 8;
+                    const int k = k0 + wk * WK + j * 8 + 2 * tq;
+                    *reinterpret_cast<float2*>(dW + static_cast<long long>(n) * g.K + k) = make_float2(acc[i][j][half * 2], acc[i][j][half * 2 + 1]);
+                }
+        if (g.db && blockIdx.y == 0 && tid < TILE) g.db[static_cast<long long>(blockIdx.z) * g.N + n0 + tid] = bsum;
+        return;
+    }
 #pragma unroll
     for (int i = 0; i < MT; ++i)
 #pragma unroll
@@ -171,11 +194,12 @@ __global__ void __launch_bounds__(WG_THREADS) wgrad_kernel(const WgradArgs<T> g)
     if (g.db && blockIdx.y == 0 && tid < TILE) atomicAdd(g.db + n0 + tid, bsum);
 }
 
+// det: g.dW / g.db are slabs of det_wgrad_splits(M, N, K) slots, whichever kernel runs
 template <typename T>
-cudaError_t launch_wgrad(WgradArgs<T> g, int num_sms, cudaStream_t st) {
+cudaError_t launch_wgrad(WgradArgs<T> g, int num_sms, bool det, cudaStream_t st) {
     if constexpr (Act<T>::kIsBf16) {
-        if (wgrad_tc_supported(g)) return wgrad_tc_launch(g, num_sms, st);   // plain operands, C >= 128: tcgen05 (wgrad_tc.cuh)
-        if (wg2::supported(g)) return wg2::launch(g, num_sms, st);      // pipelined bf16 path (wgrad_bf16.cuh)
+        if (wgrad_tc_supported(g)) return wgrad_tc_launch(g, num_sms, det, st);   // plain operands, C >= 128: tcgen05 (wgrad_tc.cuh)
+        if (wg2::supported(g)) return det ? wg2::launch<true>(g, num_sms, st) : wg2::launch<false>(g, num_sms, st);   // wgrad_bf16.cuh
     }
     const int tile = (g.N % 64 == 0 && g.K % 64 == 0) ? 64 : 32;
     const long long tiles = static_cast<long long>(g.N / tile) * (g.K / tile);
@@ -185,11 +209,17 @@ cudaError_t launch_wgrad(WgradArgs<T> g, int num_sms, cudaStream_t st) {
     if (want < 1) want = 1;
     long long rps = (g.M + want - 1) / want;
     rps = (rps + WG_BM - 1) / WG_BM * WG_BM;
+    if (det) rps = det_wgrad_rows_per_split(g.M, g.N, g.K);
     const unsigned splits = static_cast<unsigned>((g.M + rps - 1) / rps);
     g.rows_per_split = rps;
     dim3 grid(g.N / tile, g.K / tile, splits);
-    if (tile == 64) wgrad_kernel<T, 64><<<grid, WG_THREADS, 0, st>>>(g);
-    else wgrad_kernel<T, 32><<<grid, WG_THREADS, 0, st>>>(g);
+    if (det) {
+        if (tile == 64) wgrad_kernel<T, 64, true><<<grid, WG_THREADS, 0, st>>>(g);
+        else wgrad_kernel<T, 32, true><<<grid, WG_THREADS, 0, st>>>(g);
+    } else {
+        if (tile == 64) wgrad_kernel<T, 64><<<grid, WG_THREADS, 0, st>>>(g);
+        else wgrad_kernel<T, 32><<<grid, WG_THREADS, 0, st>>>(g);
+    }
     return cudaGetLastError();
 }
 
@@ -197,7 +227,9 @@ cudaError_t launch_wgrad(WgradArgs<T> g, int num_sms, cudaStream_t st) {
 // dx[row] = dres[row] + LNbwd(dz[row]; x[row], gamma);  dgamma += sum dz * xhat;  dbeta += sum dz.
 // G lanes per row with 16-byte loads (a warp streams 32/G rows at once), grid-stride over rows, per-lane register
 // partials for dgamma / dbeta reduced through shuffles + shared memory, one global atomic per column per block.
-template <typename T, int G, int MAXV>
+// DET: the warps add into shared memory one after another in warp order, and the block stores its column sums into slab
+// blockIdx.x of [gridDim.x][C].
+template <typename T, int G, int MAXV, bool DET = false>
 __global__ void __launch_bounds__(256, MAXV == 1 ? 3 : 1) ln_bwd_kernel(const T* __restrict__ dz, const T* __restrict__ x,
                                                      const T* __restrict__ dres, T* __restrict__ dx,
                                                      const float* __restrict__ gamma, float* __restrict__ dgamma,
@@ -301,21 +333,45 @@ __global__ void __launch_bounds__(256, MAXV == 1 ? 3 : 1) ln_bwd_kernel(const T*
     __shared__ float sg[1024], sb[1024];
     for (int i = threadIdx.x; i < C; i += blockDim.x) { sg[i] = 0.f; sb[i] = 0.f; }
     __syncthreads();
+    if constexpr (DET) {
+#pragma unroll 1
+        for (int w = 0; w < 8; ++w) {               // 256 threads: 8 warps, in order; the same per-column shuffles as below
+            if ((threadIdx.x >> 5) == w) {
 #pragma unroll
-    for (int i = 0; i < MAXV; ++i) {
-        const int k = (gl + i * G) * EPL;
+                for (int i = 0; i < MAXV; ++i) {
+                    const int k = (gl + i * G) * EPL;
 #pragma unroll
-        for (int j = 0; j < EPL; ++j) {
-            float gv = gacc[i][j], bv = bacc[i][j];
+                    for (int j = 0; j < EPL; ++j) {
+                        float gv = gacc[i][j], bv = bacc[i][j];
 #pragma unroll
-            for (int o = G; o < 32; o <<= 1) { gv += __shfl_xor_sync(0xffffffffu, gv, o); bv += __shfl_xor_sync(0xffffffffu, bv, o); }
-            if (sub == 0 && k < C) { atomicAdd(&sg[k + j], gv); atomicAdd(&sb[k + j], bv); }
+                        for (int o = G; o < 32; o <<= 1) { gv += __shfl_xor_sync(0xffffffffu, gv, o); bv += __shfl_xor_sync(0xffffffffu, bv, o); }
+                        if (sub == 0 && k < C) { sg[k + j] += gv; sb[k + j] += bv; }
+                    }
+                }
+            }
+            __syncthreads();
         }
-    }
-    __syncthreads();
-    for (int i = threadIdx.x; i < C; i += blockDim.x) {
-        atomicAdd(dgamma + i, sg[i]);
-        atomicAdd(dbeta + i, sb[i]);
+        for (int i = threadIdx.x; i < C; i += blockDim.x) {
+            dgamma[static_cast<long long>(blockIdx.x) * C + i] = sg[i];
+            dbeta[static_cast<long long>(blockIdx.x) * C + i] = sb[i];
+        }
+    } else {
+#pragma unroll
+        for (int i = 0; i < MAXV; ++i) {
+            const int k = (gl + i * G) * EPL;
+#pragma unroll
+            for (int j = 0; j < EPL; ++j) {
+                float gv = gacc[i][j], bv = bacc[i][j];
+#pragma unroll
+                for (int o = G; o < 32; o <<= 1) { gv += __shfl_xor_sync(0xffffffffu, gv, o); bv += __shfl_xor_sync(0xffffffffu, bv, o); }
+                if (sub == 0 && k < C) { atomicAdd(&sg[k + j], gv); atomicAdd(&sb[k + j], bv); }
+            }
+        }
+        __syncthreads();
+        for (int i = threadIdx.x; i < C; i += blockDim.x) {
+            atomicAdd(dgamma + i, sg[i]);
+            atomicAdd(dbeta + i, sb[i]);
+        }
     }
 }
 
@@ -327,6 +383,7 @@ __global__ void __launch_bounds__(256, MAXV == 1 ? 3 : 1) ln_bwd_kernel(const T*
 constexpr int LNW_ROWS = 8;           // rows per tile = warps per CTA (one row's statistics per warp)
 constexpr int LNW_THREADS = 256;      // x 4 columns = the widest row
 
+template <bool DET = false>      // DET: the per-CTA column sums are stored into slab blockIdx.x of [gridDim.x][C]
 __global__ void __launch_bounds__(LNW_THREADS) ln_bwd_wide_kernel(const float* __restrict__ dz, const float* __restrict__ x,
                                                                   const float* __restrict__ dres, float* __restrict__ dx,
                                                                   const float* __restrict__ gamma, float* __restrict__ dgamma,
@@ -396,38 +453,59 @@ __global__ void __launch_bounds__(LNW_THREADS) ln_bwd_wide_kernel(const float* _
             }
         }
     }
+    if constexpr (DET) {
+        if (own) {
+            st4(dgamma + static_cast<long long>(blockIdx.x) * C + k, ga);
+            st4(dbeta + static_cast<long long>(blockIdx.x) * C + k, ba);
+        }
+        return;
+    }
     if (own) {
         atomicAdd(dgamma + k, ga.x); atomicAdd(dgamma + k + 1, ga.y); atomicAdd(dgamma + k + 2, ga.z); atomicAdd(dgamma + k + 3, ga.w);
         atomicAdd(dbeta + k, ba.x); atomicAdd(dbeta + k + 1, ba.y); atomicAdd(dbeta + k + 2, ba.z); atomicAdd(dbeta + k + 3, ba.w);
     }
 }
 
+// lanes per row of ln_bwd_kernel for C channels of elem_bytes each (0: the fp32 wide kernel)
+inline int ln_bwd_lanes(int C, int elem_bytes) {
+    const int chunks = C / (16 / elem_bytes);
+    if (elem_bytes == 4 && chunks > 128) return 0;
+    return chunks <= 4 ? 4 : chunks <= 8 ? 8 : chunks <= 16 ? 16 : 32;
+}
+// CTAs of the LayerNorm backward (in deterministic mode with sms = 148: the slabs of d(gamma) / d(beta))
+inline long long ln_bwd_grid(long long rows, int C, int elem_bytes, int sms) {
+    const int G = ln_bwd_lanes(C, elem_bytes);
+    const long long per = G == 0 ? LNW_ROWS : 8 * (32 / G);
+    long long blocks = (rows + per - 1) / per;
+    const long long cap = static_cast<long long>(sms) * (G == 0 ? 3 : 8);
+    return blocks > cap ? cap : blocks;
+}
+
 inline cudaError_t launch_ln_bwd_wide(const float* dz, const float* x, const float* dres, float* dx, const float* gamma,
-                                      float* dgamma, float* dbeta, long long rows, int C, int num_sms, cudaStream_t st) {
+                                      float* dgamma, float* dbeta, long long rows, int C, int num_sms, bool det, cudaStream_t st) {
     const int smem = 2 * LNW_ROWS * C * static_cast<int>(sizeof(float));     // 64 KB at C = 1024: three CTAs per SM
-    cudaError_t e = cudaFuncSetAttribute(ln_bwd_wide_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+    auto k = det ? ln_bwd_wide_kernel<true> : ln_bwd_wide_kernel<false>;
+    cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
     if (e != cudaSuccess) return e;
-    long long blocks = (rows + LNW_ROWS - 1) / LNW_ROWS;
-    const long long cap = static_cast<long long>(num_sms) * 3;
-    if (blocks > cap) blocks = cap;
-    ln_bwd_wide_kernel<<<static_cast<unsigned>(blocks), LNW_THREADS, smem, st>>>(dz, x, dres, dx, gamma, dgamma, dbeta, rows, C);
+    const long long blocks = ln_bwd_grid(rows, C, 4, det ? 148 : num_sms);
+    k<<<static_cast<unsigned>(blocks), LNW_THREADS, smem, st>>>(dz, x, dres, dx, gamma, dgamma, dbeta, rows, C);
     return cudaGetLastError();
 }
 
+// det: dgamma / dbeta are slabs of ln_bwd_grid(rows, C, sizeof(T), 148) slots
 template <typename T>
 cudaError_t launch_ln_bwd(const T* dz, const T* x, const T* dres, T* dx, const float* gamma, float* dgamma,
-                          float* dbeta, long long rows, int C, int num_sms, cudaStream_t st) {
+                          float* dbeta, long long rows, int C, int num_sms, bool det, cudaStream_t st) {
     constexpr int EPL = 16 / sizeof(T);
     const int chunks = C / EPL;
     if constexpr (!Act<T>::kIsBf16) {
-        if (C <= 1024 && chunks > 128) return launch_ln_bwd_wide(dz, x, dres, dx, gamma, dgamma, dbeta, rows, C, num_sms, st);
+        if (C <= 1024 && chunks > 128) return launch_ln_bwd_wide(dz, x, dres, dx, gamma, dgamma, dbeta, rows, C, num_sms, det, st);
     }
     auto go = [&](auto gtag, auto vtag) -> cudaError_t {
         constexpr int G = decltype(gtag)::value, MAXV = decltype(vtag)::value;
-        long long blocks = (rows + 8 * (32 / G) - 1) / (8 * (32 / G));
-        const long long cap = static_cast<long long>(num_sms) * 8;
-        if (blocks > cap) blocks = cap;
-        ln_bwd_kernel<T, G, MAXV><<<static_cast<unsigned>(blocks), 256, 0, st>>>(dz, x, dres, dx, gamma, dgamma, dbeta, rows, C);
+        const long long blocks = ln_bwd_grid(rows, C, sizeof(T), det ? 148 : num_sms);
+        if (det) ln_bwd_kernel<T, G, MAXV, true><<<static_cast<unsigned>(blocks), 256, 0, st>>>(dz, x, dres, dx, gamma, dgamma, dbeta, rows, C);
+        else ln_bwd_kernel<T, G, MAXV><<<static_cast<unsigned>(blocks), 256, 0, st>>>(dz, x, dres, dx, gamma, dgamma, dbeta, rows, C);
         return cudaGetLastError();
     };
     using std::integral_constant;
@@ -444,8 +522,9 @@ cudaError_t launch_ln_bwd(const T* dz, const T* x, const T* dres, T* dx, const f
 // Inputs: g2 = d(h2) (gradient after the second GELU), a2 (pre-GELU conv output), h1 (conv input), a1 (pre-GELU
 // linear1 output).  Outputs: da1 = (conv^T(da2)) * gelu'(a1) with da2 = g2 * gelu'(a2);  dWdw, dbdw accumulated.
 // Block = 32 channel-groups (128 channels) x 8 pixel lanes; persistent over (b, slab, strip) work items so that the
-// weight-gradient partials stay in registers and are flushed once per block.
-template <typename T>
+// weight-gradient partials stay in registers and are flushed once per block.  DET: a flush stores into slab blockIdx.x of
+// [gridDim.x][Ch, 9] / [gridDim.x][Ch] (a CTA flushes each channel slab at most once; the caller zeroes the slabs).
+template <typename T, bool DET = false>
 __global__ void __launch_bounds__(256) dwconv_bwd_kernel(const T* __restrict__ g2, const T* __restrict__ a2,
                                                          const T* __restrict__ h1, const T* __restrict__ a1,
                                                          T* __restrict__ da1, const float* __restrict__ w,
@@ -487,8 +566,13 @@ __global__ void __launch_bounds__(256) dwconv_bwd_kernel(const T* __restrict__ g
             for (int p = 0; p < 8; ++p) s += red[p][cg][j];
             const int c = slab * 128 + cg * 4 + (j < 36 ? j / 9 : j - 36);
             if (c < Ch) {
-                if (j < 36) atomicAdd(dw + c * 9 + (j % 9), s);
-                else atomicAdd(dbias + c, s);
+                if constexpr (DET) {
+                    if (j < 36) dw[(static_cast<long long>(blockIdx.x) * Ch + c) * 9 + (j % 9)] = s;
+                    else dbias[static_cast<long long>(blockIdx.x) * Ch + c] = s;
+                } else {
+                    if (j < 36) atomicAdd(dw + c * 9 + (j % 9), s);
+                    else atomicAdd(dbias + c, s);
+                }
             }
         }
 #pragma unroll
@@ -575,13 +659,18 @@ __global__ void __launch_bounds__(256) dwconv_bwd_kernel(const T* __restrict__ g
     if (cur_slab >= 0) flush(cur_slab);
 }
 
+inline long long dwconv_bwd_grid(int B, int H, int W, int Ch, int sms) {
+    const long long items = static_cast<long long>(B) * ((Ch + 127) / 128) * ((W + 7) / 8) * ((H + 15) / 16);
+    const long long grid = static_cast<long long>(sms) * 8;
+    return grid > items ? items : grid;
+}
+
 template <typename T>
 cudaError_t launch_dwconv_bwd(const T* g2, const T* a2, const T* h1, const T* a1, T* da1, const float* w, float* dw,
-                              float* dbias, int B, int H, int W, int Ch, int num_sms, cudaStream_t st) {
-    const long long items = static_cast<long long>(B) * ((Ch + 127) / 128) * ((W + 7) / 8) * ((H + 15) / 16);
-    long long grid = static_cast<long long>(num_sms) * 8;
-    if (grid > items) grid = items;
-    dwconv_bwd_kernel<T><<<static_cast<unsigned>(grid), 256, 0, st>>>(g2, a2, h1, a1, da1, w, dw, dbias, B, H, W, Ch);
+                              float* dbias, int B, int H, int W, int Ch, int num_sms, bool det, cudaStream_t st) {
+    const long long grid = dwconv_bwd_grid(B, H, W, Ch, det ? 148 : num_sms);
+    if (det) dwconv_bwd_kernel<T, true><<<static_cast<unsigned>(grid), 256, 0, st>>>(g2, a2, h1, a1, da1, w, dw, dbias, B, H, W, Ch);
+    else dwconv_bwd_kernel<T><<<static_cast<unsigned>(grid), 256, 0, st>>>(g2, a2, h1, a1, da1, w, dw, dbias, B, H, W, Ch);
     return cudaGetLastError();
 }
 
@@ -606,12 +695,19 @@ struct CoreBwdSmem {
     float tm[kTok];               // input mask of the window's tokens (a.tmask)
 };
 
-template <typename T, int D>
+// DET (deterministic mode): dynamic shared memory also holds the fp32 dA rows of the item's slots (CoreBwdDetDa); each
+// relative-position entry of the table sums them in slot order, the table partials are stored into slab blockIdx.x of
+// [gridDim.x][225, nH], and d(rpb dense) is added with plain stores into slab blockIdx.x of [gridDim.x][nH, 64, 64] (zeroed by
+// the caller).
+struct CoreBwdDetDa { float da[32 * P_LD]; };
+
+template <typename T, int D, bool DET = false>
 __global__ void __launch_bounds__(CORE_THREADS) probsparse_core_bwd_kernel(const CoreBwdArgs<T> a) {
     constexpr int PASSES = Act<T>::kPasses;
     constexpr int QK_LD = CoreLd<D>::QK;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     CoreBwdSmem<D>& s = *reinterpret_cast<CoreBwdSmem<D>*>(smem_raw);
+    float* const dab = reinterpret_cast<CoreBwdDetDa*>(smem_raw + sizeof(CoreBwdSmem<D>))->da;      // DET only
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int gq = lane >> 2, tq = lane & 3;
     const int C3 = 3 * a.C;
@@ -796,15 +892,25 @@ __global__ void __launch_bounds__(CORE_THREADS) probsparse_core_bwd_kernel(const
             const float q0 = r2[lane], q1 = r2[lane + 32];
             float dot = group_sum<32>(g0 * q0 + g1 * q1);
             const float da0 = q0 * (g0 - dot), da1 = q1 * (g1 - dot);
-            if (want_tab && a.rpb_table) {
-                const int ry = r >> 3, rx = r & 7;
-                atomicAdd(&s.tacc[h * 225 + (ry - (lane >> 3) + 7) * 15 + (rx - (lane & 7) + 7)], da0);
-                atomicAdd(&s.tacc[h * 225 + (ry - ((lane + 32) >> 3) + 7) * 15 + (rx - (lane & 7) + 7)], da1);
-            }
-            if (want_dense) {       // gradient w.r.t. the gathered bias [nH, 64, 64] (AttentionLayer.forward's argument, attn.py:385)
-                float* drow = a.d_rpb_dense + (static_cast<long long>(h) * kTok + r) * kTok;
-                atomicAdd(drow + lane, da0);
-                atomicAdd(drow + lane + 32, da1);
+            if constexpr (DET) {
+                if (want_tab && a.rpb_table) { dab[slot * P_LD + lane] = da0; dab[slot * P_LD + lane + 32] = da1; }
+                if (want_dense) {
+                    float* drow = a.d_rpb_dense + static_cast<long long>(blockIdx.x) * a.nH * kTok * kTok +
+                                  (static_cast<long long>(h) * kTok + r) * kTok;
+                    drow[lane] += da0;
+                    drow[lane + 32] += da1;
+                }
+            } else {
+                if (want_tab && a.rpb_table) {
+                    const int ry = r >> 3, rx = r & 7;
+                    atomicAdd(&s.tacc[h * 225 + (ry - (lane >> 3) + 7) * 15 + (rx - (lane & 7) + 7)], da0);
+                    atomicAdd(&s.tacc[h * 225 + (ry - ((lane + 32) >> 3) + 7) * 15 + (rx - (lane & 7) + 7)], da1);
+                }
+                if (want_dense) {       // gradient w.r.t. the gathered bias [nH, 64, 64] (AttentionLayer.forward's argument, attn.py:385)
+                    float* drow = a.d_rpb_dense + (static_cast<long long>(h) * kTok + r) * kTok;
+                    atomicAdd(drow + lane, da0);
+                    atomicAdd(drow + lane + 32, da1);
+                }
             }
             const float p0 = r1[lane], p1v = r1[lane + 32];
             dot = group_sum<32>(da0 * p0 + da1 * p1v);
@@ -812,6 +918,20 @@ __global__ void __launch_bounds__(CORE_THREADS) probsparse_core_bwd_kernel(const
             rd[lane + 32] = p1v * (da1 - dot) * scale;
         }
         __syncthreads();
+        if constexpr (DET) {
+            if (want_tab && a.rpb_table) {     // entry e = (dy + 7) * 15 + (dx + 7) takes, per slot in order, the key at (ry - dy, rx - dx)
+                for (int e = tid; e < 225; e += CORE_THREADS) {
+                    const int ey = e / 15 - 7, ex = e % 15 - 7;
+                    float sum = 0.f;
+                    for (int sl = 0; sl < kTopU; ++sl) {
+                        const int t = s.tok_of[sl];
+                        const int ly = (t >> 3) - ey, lx = (t & 7) - ex;
+                        if (ly >= 0 && ly < 8 && lx >= 0 && lx < 8) sum += dab[sl * P_LD + ly * 8 + lx];
+                    }
+                    s.tacc[h * 225 + e] += sum;
+                }
+            }
+        }
 
         T* obase = a.dqkv + static_cast<long long>(wg) * kTok * C3 + h * D;
         // ---- dq[top] = dS K  (32 x D x 64): warp -> m-tile (warp&1), D/16 n-tiles ; other rows zero
@@ -894,35 +1014,166 @@ __global__ void __launch_bounds__(CORE_THREADS) probsparse_core_bwd_kernel(const
         for (int i = tid; i < a.nH * 225; i += CORE_THREADS) {
             const int h = i / 225, rel = i - h * 225;
             const float v = s.tacc[i];
-            if (v != 0.f) atomicAdd(a.d_rpb_table + rel * a.nH + h, v);
+            if constexpr (DET) a.d_rpb_table[static_cast<long long>(blockIdx.x) * a.nH * 225 + rel * a.nH + h] = v;
+            else if (v != 0.f) atomicAdd(a.d_rpb_table + rel * a.nH + h, v);
         }
     }
 }
 
+template <int D>
+inline size_t core_bwd_smem(bool det) { return sizeof(CoreBwdSmem<D>) + (det ? sizeof(CoreBwdDetDa) : 0); }
+inline size_t core_bwd_smem(int D, bool det) {
+    return D == 32 ? core_bwd_smem<32>(det) : D == 64 ? core_bwd_smem<64>(det) : core_bwd_smem<128>(det);
+}
+// CTAs of the core backward for head_dim D (in deterministic mode with sms = 148: the slabs of the bias gradients)
+inline long long core_bwd_grid(long long items, int D, bool bf16, int sms, bool det) {
+    if (D == 32 && bf16) return pcb2::grid(items, sms, det);
+    const size_t smem = core_bwd_smem(D, det);
+    const int resident = static_cast<int>((227 * 1024) / (smem + 1024));
+    const long long cap = static_cast<long long>(sms) * (resident < 1 ? 1 : resident > 2 ? 2 : resident) * 2;
+    return items < cap ? items : cap;
+}
+
 template <typename T, int D>
-cudaError_t launch_core_bwd_d(const CoreBwdArgs<T>& a, int num_sms, cudaStream_t stream) {
-    auto k = probsparse_core_bwd_kernel<T, D>;
-    const size_t smem = sizeof(CoreBwdSmem<D>);
+cudaError_t launch_core_bwd_d(const CoreBwdArgs<T>& a, int num_sms, bool det, cudaStream_t stream) {
+    auto k = det ? probsparse_core_bwd_kernel<T, D, true> : probsparse_core_bwd_kernel<T, D>;
+    const size_t smem = core_bwd_smem<D>(det);
     cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
     if (e != cudaSuccess) return e;
-    long long items = static_cast<long long>(a.B_) * a.nH;
-    const int resident = static_cast<int>((227 * 1024) / (smem + 1024));
-    long long cap = static_cast<long long>(num_sms) * (resident < 1 ? 1 : resident > 2 ? 2 : resident) * 2;
-    unsigned grid = static_cast<unsigned>(items < cap ? items : cap);
+    const long long items = static_cast<long long>(a.B_) * a.nH;
+    const unsigned grid = static_cast<unsigned>(core_bwd_grid(items, D, Act<T>::kIsBf16, det ? 148 : num_sms, det));
     k<<<grid, CORE_THREADS, smem, stream>>>(a);
     return cudaGetLastError();
 }
 
+// det: a.d_rpb_table / a.d_rpb_dense are slabs of core_bwd_grid(.., 148, true) slots
 template <typename T>
-cudaError_t launch_core_bwd(const CoreBwdArgs<T>& a, int num_sms, cudaStream_t stream) {
+cudaError_t launch_core_bwd(const CoreBwdArgs<T>& a, int num_sms, bool det, cudaStream_t stream) {
     const int D = a.C / a.nH;
     if (D == 32) {
-        if constexpr (Act<T>::kIsBf16) return pcb2::launch(a, num_sms, stream);       // register-resident bf16 path
-        else return launch_core_bwd_d<T, 32>(a, num_sms, stream);
+        if constexpr (Act<T>::kIsBf16) return pcb2::launch(a, num_sms, det, stream);       // register-resident bf16 path
+        else return launch_core_bwd_d<T, 32>(a, num_sms, det, stream);
     }
-    if (D == 64) return launch_core_bwd_d<T, 64>(a, num_sms, stream);
-    if (D == 128) return launch_core_bwd_d<T, 128>(a, num_sms, stream);
+    if (D == 64) return launch_core_bwd_d<T, 64>(a, num_sms, det, stream);
+    if (D == 128) return launch_core_bwd_d<T, 128>(a, num_sms, det, stream);
     return cudaErrorInvalidValue;
+}
+
+// ------------------------------------------------------------------------------ deterministic-mode reduction
+// One launch per backward call: gradient e of the table gets dst[i] += sum over slots s = 0, 1, ... of slab[s * len + i], the
+// sum formed in slot order.  blockIdx.y = table entry.
+constexpr int kDetMaxSums = 8;
+struct DetSum { const float* slab; float* dst; long long slots, len; };
+struct DetTable { DetSum e[kDetMaxSums]; int n; };
+
+__global__ void __launch_bounds__(256) det_reduce_kernel(const DetTable t) {
+    const DetSum d = t.e[blockIdx.y];
+    for (long long i = static_cast<long long>(blockIdx.x) * 256 + threadIdx.x; i < d.len; i += static_cast<long long>(gridDim.x) * 256) {
+        const float* p = d.slab + i;
+        float sum = 0.f;
+#pragma unroll 8
+        for (long long s = 0; s < d.slots; ++s) sum += p[s * d.len];
+        d.dst[i] += sum;
+    }
+}
+
+// The slabs of one backward call, in the order the call registers them: the workspace query (base == nullptr) and the launch
+// run the same registration code, so slot counts and offsets have a single source.
+struct DetSlabs {
+    unsigned char* base = nullptr;
+    size_t bytes = 0;
+    DetTable t{};
+    bool zero[kDetMaxSums] = {};          // the slab has elements no unit stores: cleared before the kernels run
+    bool overflow = false;                // more slabs than the reduction table holds: clear() refuses, nothing is launched
+    float* add(float* dst, long long slots, long long len, bool holes = false) {
+        if (t.n == kDetMaxSums) { overflow = true; return nullptr; }
+        float* p = base ? reinterpret_cast<float*>(base + bytes) : nullptr;
+        t.e[t.n] = DetSum{p, dst, slots, len};
+        zero[t.n] = holes;
+        ++t.n;
+        bytes += bw_align(static_cast<size_t>(slots) * static_cast<size_t>(len) * sizeof(float));
+        return p;
+    }
+    cudaError_t clear(cudaStream_t st) const {      // called before the first kernel of the call
+        if (overflow) return cudaErrorInvalidValue;
+        for (int i = 0; i < t.n; ++i)
+            if (zero[i]) {
+                cudaError_t e = cudaMemsetAsync(const_cast<float*>(t.e[i].slab), 0, static_cast<size_t>(t.e[i].slots) * t.e[i].len * sizeof(float), st);
+                if (e != cudaSuccess) return e;
+            }
+        return cudaSuccess;
+    }
+    cudaError_t reduce(cudaStream_t st) const {
+        if (t.n == 0) return cudaSuccess;
+        long long len = 0;
+        for (int i = 0; i < t.n; ++i) len = t.e[i].len > len ? t.e[i].len : len;
+        long long gx = (len + 255) / 256;
+        if (gx > 148 * 8) gx = 148 * 8;
+        det_reduce_kernel<<<dim3(static_cast<unsigned>(gx), t.n), 256, 0, st>>>(t);
+        return cudaGetLastError();
+    }
+};
+
+// slabs of the attention-half backward, in launch order
+struct AttnDet { float *w_out, *b_out, *rpb_table, *rpb_dense, *w_qkv, *b_qkv, *ln_w, *ln_b; };
+inline AttnDet attn_bwd_det(const LewinAttnBwdArgs* a, int dtype, DetSlabs& d) {
+    const LewinAttnFwdArgs& f = a->fwd;
+    const long long tokens = static_cast<long long>(f.B) * f.H * f.W;
+    const long long C = f.C;
+    const int es = dtype == LEWIN_DTYPE_BF16 ? 2 : 4;
+    AttnDet r{};
+    const long long so = det_wgrad_splits(tokens, f.C, f.C);
+    r.w_out = d.add(a->d_w_out, so, C * C);
+    r.b_out = d.add(a->d_b_out, so, C);
+    const long long items = tokens / kTok * f.nH;
+    const long long sc = core_bwd_grid(items, f.C / f.nH, es == 2, 148, true);
+    if (a->d_rpb_table && f.use_rpb && f.rpb_table) r.rpb_table = d.add(a->d_rpb_table, sc, 225ll * f.nH);
+    if (a->d_rpb_dense && f.use_rpb) r.rpb_dense = d.add(a->d_rpb_dense, sc, f.nH * 4096ll, true);
+    const long long sq = det_wgrad_splits(tokens, 3 * f.C, f.C);
+    r.w_qkv = d.add(a->d_w_qkv, sq, 3 * C * C);
+    r.b_qkv = d.add(a->d_b_qkv, sq, 3 * C);
+    if (!f.windowed) {
+        const long long sl = ln_bwd_grid(tokens, f.C, es, 148);
+        r.ln_w = d.add(a->d_ln_w, sl, C);
+        r.ln_b = d.add(a->d_ln_b, sl, C);
+    }
+    return r;
+}
+
+// slabs of the LeFF-half backward, in launch order
+struct LeffDet { float *w2, *b2, *w_dw, *b_dw, *w1, *b1, *ln_w, *ln_b; };
+inline LeffDet leff_bwd_det(const LewinLeffBwdArgs* a, int dtype, DetSlabs& d) {
+    const LewinLeffFwdArgs& f = a->fwd;
+    const long long tokens = static_cast<long long>(f.B) * f.H * f.W;
+    const long long C = f.C, Ch = f.hidden;
+    const int es = dtype == LEWIN_DTYPE_BF16 ? 2 : 4;
+    LeffDet r{};
+    const long long s2 = det_wgrad_splits(tokens, f.C, f.hidden);
+    r.w2 = d.add(a->d_w2, s2, C * Ch);
+    r.b2 = d.add(a->d_b2, s2, C);
+    const bool tiled = dwconv_bwd_tiled_ok(f.H, f.W, f.hidden, es);
+    const long long sd = tiled ? dwconv_bwd_wgrad_gx(f.B, f.H, f.W, f.hidden, es, 148) : dwconv_bwd_grid(f.B, f.H, f.W, f.hidden, 148);
+    r.w_dw = d.add(a->d_w_dw, sd, Ch * 9, !tiled);
+    r.b_dw = d.add(a->d_b_dw, sd, Ch, !tiled);
+    const long long s1 = det_wgrad_splits(tokens, f.hidden, f.C);
+    r.w1 = d.add(a->d_w1, s1, Ch * C);
+    r.b1 = d.add(a->d_b1, s1, Ch);
+    if (f.fused) {
+        const long long sl = ln_bwd_grid(tokens, f.C, es, 148);
+        r.ln_w = d.add(a->d_ln_w, sl, C);
+        r.ln_b = d.add(a->d_ln_b, sl, C);
+    }
+    return r;
+}
+
+// slabs of the core-only backward
+inline float* core_bwd_det(const LewinCoreBwdArgs* a, int dtype, DetSlabs& d) {
+    const LewinCoreFwdArgs& f = a->fwd;
+    const int D = f.head_dim > 0 ? f.head_dim : kHeadDim;
+    const long long sc = core_bwd_grid(static_cast<long long>(f.B_) * f.nH, D, dtype == LEWIN_DTYPE_BF16, 148, true);
+    if (a->d_rpb_table && f.use_rpb && f.rpb_table) return d.add(a->d_rpb_table, sc, 225ll * f.nH);
+    if (a->d_rpb_dense && f.use_rpb && !f.rpb_table) return d.add(a->d_rpb_dense, sc, f.nH * 4096ll, true);
+    return nullptr;
 }
 
 // ------------------------------------------------------------------------------ host orchestration
@@ -940,7 +1191,7 @@ inline int bw_device(int* sms) {
     return cc == 10 ? 0 : LEWIN_E_ARCH;
 }
 
-inline size_t attn_bwd_ws(const LewinAttnBwdArgs* a, int dtype) {
+inline size_t attn_bwd_ws_base(const LewinAttnBwdArgs* a, int dtype) {
     const LewinAttnFwdArgs& f = a->fwd;
     const size_t tokens = static_cast<size_t>(f.B) * f.H * f.W;
     const size_t es = dtype == LEWIN_DTYPE_BF16 ? 2 : 4;
@@ -949,6 +1200,16 @@ inline size_t attn_bwd_ws(const LewinAttnBwdArgs* a, int dtype) {
            bw_align(tokens * C * es) + bw_align(C * C * 4) + bw_align(3 * C * C * 4) +
            (dtype == LEWIN_DTYPE_BF16 ? bw_align(3 * C * C * 2) + bw_align(C * C * 2) + bw_align(tokens * C * 2) : 0);
            // bf16: images of W_qkv^T / W_out^T and the scaled, window-ordered dy rows for the streamed-W GEMMs
+}
+// + the partial slabs of deterministic mode after the rest
+inline size_t attn_bwd_ws(const LewinAttnBwdArgs* a, int dtype) {
+    size_t n = attn_bwd_ws_base(a, dtype);
+    if (a->deterministic) {
+        DetSlabs d;
+        attn_bwd_det(a, dtype, d);
+        n += d.bytes;
+    }
+    return n;
 }
 
 // Data-gradient GEMM dX = dY . W (W^T staged as the [N, K] operand).  bf16 at the C >= 256 levels: the forward's
@@ -1037,6 +1298,12 @@ int attn_bwd(const LewinAttnBwdArgs* a, void* ws, size_t ws_bytes, cudaStream_t 
     if (int rc = bw_device(&sms)) return rc;
     const int dtype = Act<T>::kIsBf16 ? LEWIN_DTYPE_BF16 : LEWIN_DTYPE_F32;
     if (!ws || ws_bytes < attn_bwd_ws(a, dtype)) return LEWIN_E_WORKSPACE;
+    const bool det = a->deterministic != 0;
+    if (det && (reinterpret_cast<uintptr_t>(ws) & 15u)) return LEWIN_E_ALIGN;
+    DetSlabs dsl;
+    dsl.base = static_cast<unsigned char*>(ws) + attn_bwd_ws_base(a, dtype);
+    const AttnDet dt = det ? attn_bwd_det(a, dtype, dsl) : AttnDet{};
+    if (det) BCK(dsl.clear(st));
 
     const long long tokens = static_cast<long long>(f.B) * f.H * f.W;
     const int C = f.C, nWin = (f.H / 8) * (f.W / 8), B_ = f.B * nWin;
@@ -1076,7 +1343,7 @@ int attn_bwd(const LewinAttnBwdArgs* a, void* ws, size_t ws_bytes, cudaStream_t 
     {   // dW_out += do^T ctx ; db_out += colsum(do)
         WgradArgs<T> w{};
         w.dY = dy; w.lddy = C; w.X = static_cast<const T*>(f.ctx); w.ldx = C;
-        w.dW = a->d_w_out; w.db = a->d_b_out; w.M = tokens; w.N = C; w.K = C;
+        w.dW = det ? dt.w_out : a->d_w_out; w.db = det ? dt.b_out : a->d_b_out; w.M = tokens; w.N = C; w.K = C;
         w.mapDY = mapped; w.mapX = 0; w.map = map; w.tokens_per_image = tpi;
         w.dy_row_scale = f.windowed ? nullptr : f.drop_scale;
         if constexpr (Act<T>::kIsBf16) {
@@ -1089,25 +1356,25 @@ int attn_bwd(const LewinAttnBwdArgs* a, void* ws, size_t ws_bytes, cudaStream_t 
                 w = v;
             }
         }
-        BCK(launch_wgrad<T>(w, sms, st));
+        BCK(launch_wgrad<T>(w, sms, det, st));
     }
     {   // core backward -> dq | dk | dv
         CoreBwdArgs<T> c{};
         c.qkv = static_cast<const T*>(f.qkv); c.dctx = dctx; c.dqkv = dqkv; c.top = f.top;
         c.rpb_table = f.rpb_table; c.rpb_dense = f.rpb_table ? nullptr : f.rpb_dense;
-        c.d_rpb_table = a->d_rpb_table;
-        c.d_rpb_dense = a->d_rpb_dense;
+        c.d_rpb_table = det ? dt.rpb_table : a->d_rpb_table;
+        c.d_rpb_dense = det ? dt.rpb_dense : a->d_rpb_dense;
         c.mask = f.mask; c.nW_mask = f.mask ? f.nW_mask : 1;
         c.B_ = B_; c.nH = f.nH; c.C = C; c.use_rpb = f.use_rpb;
         c.shift = (f.analytic_shift_mask && !f.windowed) ? f.shift : 0;
         c.H = f.H; c.W = f.W; c.nWw = f.W / 8; c.nWin = nWin;
         c.tmask = f.token_mask; c.Bm = f.token_mask ? f.Bm : 1;
-        BCK(launch_core_bwd<T>(c, sms, st));
+        BCK(launch_core_bwd<T>(c, sms, det, st));
     }
     {   // dW_qkv += dqkv^T LN1(x)[window order] ; db_qkv += colsum(dqkv)
         WgradArgs<T> w{};
         w.dY = dqkv; w.lddy = 3 * C; w.X = x; w.ldx = C;
-        w.dW = a->d_w_qkv; w.db = a->d_b_qkv; w.M = tokens; w.N = 3 * C; w.K = C;
+        w.dW = det ? dt.w_qkv : a->d_w_qkv; w.db = det ? dt.b_qkv : a->d_b_qkv; w.M = tokens; w.N = 3 * C; w.K = C;
         w.mapDY = 0; w.mapX = mapped; w.map = map; w.tokens_per_image = tpi;
         if (!f.windowed) { w.mean = mean; w.rstd = rstd; w.ln_w = f.ln_w; w.ln_b = f.ln_b; }
         if constexpr (Act<T>::kIsBf16) {
@@ -1121,7 +1388,7 @@ int attn_bwd(const LewinAttnBwdArgs* a, void* ws, size_t ws_bytes, cudaStream_t 
             }
         }
         if (w.mean) BCK(launch_ln_stats<T>(x, tokens, C, mean, rstd, st));      // only the register-prologue kernels need them
-        BCK(launch_wgrad<T>(w, sms, st));
+        BCK(launch_wgrad<T>(w, sms, det, st));
     }
     {   // d(LN1 out) = dqkv . W_qkv, scattered back to token order (window_reverse + un-roll)
         GemmArgs<T> g{};
@@ -1131,11 +1398,13 @@ int attn_bwd(const LewinAttnBwdArgs* a, void* ws, size_t ws_bytes, cudaStream_t 
         BCK(launch_dgrad_gemm<T>(g, wqkvT_b, sms, st));
     }
     if (!f.windowed)   // dx = dy + LN1_bwd(dxh)
-        BCK(launch_ln_bwd<T>(dxh, x, dy, static_cast<T*>(a->dx), f.ln_w, a->d_ln_w, a->d_ln_b, tokens, C, sms, st));
+        BCK(launch_ln_bwd<T>(dxh, x, dy, static_cast<T*>(a->dx), f.ln_w, det ? dt.ln_w : a->d_ln_w, det ? dt.ln_b : a->d_ln_b,
+                             tokens, C, sms, det, st));
+    if (det) BCK(dsl.reduce(st));
     return 0;
 }
 
-inline size_t leff_bwd_ws(const LewinLeffBwdArgs* a, int dtype) {
+inline size_t leff_bwd_ws_base(const LewinLeffBwdArgs* a, int dtype) {
     const LewinLeffFwdArgs& f = a->fwd;
     const size_t tokens = static_cast<size_t>(f.B) * f.H * f.W;
     const size_t es = dtype == LEWIN_DTYPE_BF16 ? 2 : 4;
@@ -1143,6 +1412,16 @@ inline size_t leff_bwd_ws(const LewinLeffBwdArgs* a, int dtype) {
     return 2 * bw_align(tokens * 4) + 3 * bw_align(tokens * Ch * es) + bw_align(tokens * C * es) + 2 * bw_align(C * Ch * 4) +
            (dtype == LEWIN_DTYPE_BF16 ? 2 * bw_align(C * Ch * 2) + bw_align(tokens * C * 2) : 0);
            // bf16: images of W2^T, W1^T and the DropPath-scaled dout rows
+}
+// + the partial slabs of deterministic mode after the rest
+inline size_t leff_bwd_ws(const LewinLeffBwdArgs* a, int dtype) {
+    size_t n = leff_bwd_ws_base(a, dtype);
+    if (a->deterministic) {
+        DetSlabs d;
+        leff_bwd_det(a, dtype, d);
+        n += d.bytes;
+    }
+    return n;
 }
 
 template <typename T>
@@ -1157,6 +1436,12 @@ int leff_bwd(const LewinLeffBwdArgs* a, void* ws, size_t ws_bytes, cudaStream_t 
     if (int rc = bw_device(&sms)) return rc;
     const int dtype = Act<T>::kIsBf16 ? LEWIN_DTYPE_BF16 : LEWIN_DTYPE_F32;
     if (!ws || ws_bytes < leff_bwd_ws(a, dtype)) return LEWIN_E_WORKSPACE;
+    const bool det = a->deterministic != 0;
+    if (det && (reinterpret_cast<uintptr_t>(ws) & 15u)) return LEWIN_E_ALIGN;
+    DetSlabs dsl;
+    dsl.base = static_cast<unsigned char*>(ws) + leff_bwd_ws_base(a, dtype);
+    const LeffDet dt = det ? leff_bwd_det(a, dtype, dsl) : LeffDet{};
+    if (det) BCK(dsl.clear(st));
 
     const long long tokens = static_cast<long long>(f.B) * f.H * f.W;
     const int C = f.C, Ch = f.hidden, tpi = f.H * f.W;
@@ -1191,7 +1476,7 @@ int leff_bwd(const LewinLeffBwdArgs* a, void* ws, size_t ws_bytes, cudaStream_t 
     {   // dW2 += (s*dout)^T h2 ; db2 += colsum(s*dout)
         WgradArgs<T> w{};
         w.dY = dout; w.lddy = C; w.X = static_cast<const T*>(f.h2); w.ldx = Ch;
-        w.dW = a->d_w2; w.db = a->d_b2; w.M = tokens; w.N = C; w.K = Ch;
+        w.dW = det ? dt.w2 : a->d_w2; w.db = det ? dt.b2 : a->d_b2; w.M = tokens; w.N = C; w.K = Ch;
         w.tokens_per_image = tpi; w.dy_row_scale = dscale;
         if constexpr (Act<T>::kIsBf16) {
             WgradArgs<T> v = w;                  // DropPath-scaled rows: left by the GEMM above at C >= 128, made here otherwise
@@ -1202,24 +1487,31 @@ int leff_bwd(const LewinLeffBwdArgs* a, void* ws, size_t ws_bytes, cudaStream_t 
                 w = v;
             }
         }
-        BCK(launch_wgrad<T>(w, sms, st));
+        BCK(launch_wgrad<T>(w, sms, det, st));
     }
     // depthwise conv backward: da1 = conv^T(dh2 * gelu'(a2)) * gelu'(a1); dWdw, dbdw
     {
         if (Act<T>::kIsBf16) BCK(launch_gelu_tab_init(st));
         cudaError_t derr = cudaSuccess;
-        if (launch_dwconv_bwd_tiled<T>(dh2, static_cast<const T*>(f.a2), static_cast<const T*>(f.h1), static_cast<const T*>(f.a1),
-                                       da1, da2, f.w_dw, a->d_w_dw, a->d_b_dw, f.B, f.H, f.W, Ch, sms, st, &derr)) {
+        float* dw = det ? dt.w_dw : a->d_w_dw;
+        float* dbias = det ? dt.b_dw : a->d_b_dw;
+        const bool tiled = det ? launch_dwconv_bwd_tiled<T, true>(dh2, static_cast<const T*>(f.a2), static_cast<const T*>(f.h1),
+                                                                  static_cast<const T*>(f.a1), da1, da2, f.w_dw, dw, dbias, f.B, f.H,
+                                                                  f.W, Ch, sms, st, &derr)
+                               : launch_dwconv_bwd_tiled<T>(dh2, static_cast<const T*>(f.a2), static_cast<const T*>(f.h1),
+                                                            static_cast<const T*>(f.a1), da1, da2, f.w_dw, dw, dbias, f.B, f.H, f.W,
+                                                            Ch, sms, st, &derr);
+        if (tiled) {
             BCK(derr);
         } else {
             BCK(launch_dwconv_bwd<T>(dh2, static_cast<const T*>(f.a2), static_cast<const T*>(f.h1), static_cast<const T*>(f.a1),
-                                     da1, f.w_dw, a->d_w_dw, a->d_b_dw, f.B, f.H, f.W, Ch, sms, st));
+                                     da1, f.w_dw, dw, dbias, f.B, f.H, f.W, Ch, sms, det, st));
         }
     }
     {   // dW1 += da1^T LN2(y) ; db1 += colsum(da1)
         WgradArgs<T> w{};
         w.dY = da1; w.lddy = Ch; w.X = y; w.ldx = C;
-        w.dW = a->d_w1; w.db = a->d_b1; w.M = tokens; w.N = Ch; w.K = C;
+        w.dW = det ? dt.w1 : a->d_w1; w.db = det ? dt.b1 : a->d_b1; w.M = tokens; w.N = Ch; w.K = C;
         w.tokens_per_image = tpi;
         if (f.fused) { w.mean = mean; w.rstd = rstd; w.ln_w = f.ln_w; w.ln_b = f.ln_b; }
         if constexpr (Act<T>::kIsBf16) {
@@ -1233,7 +1525,7 @@ int leff_bwd(const LewinLeffBwdArgs* a, void* ws, size_t ws_bytes, cudaStream_t 
             }
         }
         if (w.mean) BCK(launch_ln_stats<T>(y, tokens, C, mean, rstd, st));      // only the register-prologue kernels need them
-        BCK(launch_wgrad<T>(w, sms, st));
+        BCK(launch_wgrad<T>(w, sms, det, st));
     }
     {   // dz = da1 . W1
         GemmArgs<T> g{};
@@ -1243,7 +1535,9 @@ int leff_bwd(const LewinLeffBwdArgs* a, void* ws, size_t ws_bytes, cudaStream_t 
         BCK(launch_dgrad_gemm<T>(g, w1T_b, sms, st));
     }
     if (f.fused)   // dy = dout + LN2_bwd(dz)
-        BCK(launch_ln_bwd<T>(dz, y, dout, static_cast<T*>(a->dy), f.ln_w, a->d_ln_w, a->d_ln_b, tokens, C, sms, st));
+        BCK(launch_ln_bwd<T>(dz, y, dout, static_cast<T*>(a->dy), f.ln_w, det ? dt.ln_w : a->d_ln_w, det ? dt.ln_b : a->d_ln_b,
+                             tokens, C, sms, det, st));
+    if (det) BCK(dsl.reduce(st));
     return 0;
 }
 

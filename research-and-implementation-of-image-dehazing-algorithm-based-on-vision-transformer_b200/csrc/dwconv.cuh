@@ -379,7 +379,8 @@ __device__ __forceinline__ float2 dw_add2(const float2 a, const float2 b) {
 // the TMA unit = the convolution's padding; da2 interior box) completing on one mbarrier per buffer, instead of ~10 per-thread
 // 16-byte cp.async with their index arithmetic (ncu: those loops were 40 % of the kernel's instructions; the box layout
 // [row][column][64 channels] is exactly the layout the accumulation loop reads).
-template <typename T, int TX, bool USE_TMA = false>
+// DET: each CTA stores its sums into slab blockIdx.x of [gridDim.x][Ch, 9] / [gridDim.x][Ch] instead of adding them
+template <typename T, int TX, bool USE_TMA = false, bool DET = false>
 __global__ void __launch_bounds__(256, 2) dwconv_bwd_wgrad_kernel(const T* __restrict__ da2, const T* __restrict__ h1,
                                                                   float* __restrict__ dw, float* __restrict__ dbias,
                                                                   int B, int H, int W, int Ch,
@@ -503,19 +504,36 @@ __global__ void __launch_bounds__(256, 2) dwconv_bwd_wgrad_kernel(const T* __res
 #pragma unroll
         for (int wv = 0; wv < 8; ++wv) sum += red[((wv * 8 + c) * 10 + t) * EPC + j];
         const int cc = c0 + c * EPC + j;
-        if (t < 9) atomicAdd(dw + static_cast<long long>(cc) * 9 + t, sum);
-        else atomicAdd(dbias + cc, sum);
+        if constexpr (DET) {
+            if (t < 9) dw[(static_cast<long long>(blockIdx.x) * Ch + cc) * 9 + t] = sum;
+            else dbias[static_cast<long long>(blockIdx.x) * Ch + cc] = sum;
+        } else {
+            if (t < 9) atomicAdd(dw + static_cast<long long>(cc) * 9 + t, sum);
+            else atomicAdd(dbias + cc, sum);
+        }
     }
 }
 
-// returns false if the shape is not covered (caller falls back to the register-window kernel)
-template <typename T>
+// the tiled kernels serve this shape (otherwise the register-window kernel dwconv_bwd_kernel runs)
+inline bool dwconv_bwd_tiled_ok(int H, int W, int Ch, int elem_bytes) { return !(H % 8 || W % 8 || Ch % (8 * (16 / elem_bytes))); }
+// CTAs along x of the tiled weight-gradient kernel (= its slabs in deterministic mode, with sms = 148)
+inline int dwconv_bwd_wgrad_gx(int B, int H, int W, int Ch, int elem_bytes, int sms) {
+    const int slabs = Ch / (8 * (16 / elem_bytes));
+    const int ntiles = B * (H / 8) * (W / (W % 16 == 0 ? 16 : 8));
+    int gx = (2 * sms + slabs - 1) / slabs;
+    return gx > ntiles ? ntiles : gx;
+}
+
+// returns false if the shape is not covered (caller falls back to the register-window kernel).  DET: dw / dbias are the slabs
+// [gx][Ch, 9] / [gx][Ch] of dwconv_bwd_wgrad_gx(.., 148), every element stored once
+template <typename T, bool DET = false>
 bool launch_dwconv_bwd_tiled(const T* g2, const T* a2, const T* h1, const T* a1, T* da1, T* da2_scratch, const float* w,
                              float* dw, float* dbias, int B, int H, int W, int Ch, int num_sms, cudaStream_t st,
                              cudaError_t* err) {
     constexpr int SLAB = 8 * (16 / sizeof(T));
-    if (H % 8 || W % 8 || Ch % SLAB) return false;
+    if (!dwconv_bwd_tiled_ok(H, W, Ch, sizeof(T))) return false;
     const int slabs = Ch / SLAB;
+    const int gx = dwconv_bwd_wgrad_gx(B, H, W, Ch, sizeof(T), DET ? 148 : num_sms);
     if (W % 16 == 0) {
         if constexpr (Act<T>::kIsBf16) {      // element-wise dGELU + streaming TMA kernel (dwconv_stream.cuh; dws::supported holds here)
             *err = dws::launch_bwd_data(g2, a2, a1, da1, da2_scratch, w, B, H, W, Ch, num_sms, st);
@@ -526,8 +544,6 @@ bool launch_dwconv_bwd_tiled(const T* g2, const T* a2, const T* h1, const T* a1,
             cudaFuncSetAttribute(dwconv_bwd_data_kernel<T, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem16);
             dwconv_bwd_data_kernel<T, 16><<<grid, 256, smem16, st>>>(g2, a2, a1, da1, da2_scratch, w, B, H, W, Ch);
         }
-        const int ntiles = B * (H / 8) * (W / 16);
-        int gx = (2 * num_sms + slabs - 1) / slabs; if (gx > ntiles) gx = ntiles;
         constexpr int wg_smem16 = 2 * (10 * (16 + 2) * 128 + 8 * 16 * 128);
         CUtensorMap hmap{}, dmap{};
         bool tma_done = false;
@@ -535,27 +551,26 @@ bool launch_dwconv_bwd_tiled(const T* g2, const T* a2, const T* h1, const T* a1,
             if (tma::make_nhwc_bf16(&hmap, h1, B, H, W, Ch, 10, 18, SLAB) &&
                 tma::make_nhwc_bf16(&dmap, da2_scratch, B, H, W, Ch, 8, 16, SLAB)) {
                 constexpr int smem_tma = wg_smem16 + 128 /*alignment*/ + 16 /*mbarriers*/;
-                cudaFuncSetAttribute(dwconv_bwd_wgrad_kernel<T, 16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_tma);
-                dwconv_bwd_wgrad_kernel<T, 16, true><<<dim3(gx, slabs), 256, smem_tma, st>>>(da2_scratch, h1, dw, dbias, B, H, W, Ch,
-                                                                                          hmap, dmap);
+                cudaFuncSetAttribute(dwconv_bwd_wgrad_kernel<T, 16, true, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_tma);
+                dwconv_bwd_wgrad_kernel<T, 16, true, DET><<<dim3(gx, slabs), 256, smem_tma, st>>>(da2_scratch, h1, dw, dbias, B, H, W, Ch,
+                                                                                               hmap, dmap);
                 tma_done = true;
             }
         }
         if (!tma_done) {
-            cudaFuncSetAttribute(dwconv_bwd_wgrad_kernel<T, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, wg_smem16);
-            dwconv_bwd_wgrad_kernel<T, 16><<<dim3(gx, slabs), 256, wg_smem16, st>>>(da2_scratch, h1, dw, dbias, B, H, W, Ch, hmap, dmap);
+            cudaFuncSetAttribute(dwconv_bwd_wgrad_kernel<T, 16, false, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, wg_smem16);
+            dwconv_bwd_wgrad_kernel<T, 16, false, DET><<<dim3(gx, slabs), 256, wg_smem16, st>>>(da2_scratch, h1, dw, dbias, B, H, W, Ch,
+                                                                                              hmap, dmap);
         }
     } else {
         const unsigned grid = static_cast<unsigned>(B) * (H / 8) * (W / 8) * slabs;
         constexpr int smem8 = 2 * 10 * 10 * 128 + 9 * SLAB * 4 + kGeluTabSize * 2;
         cudaFuncSetAttribute(dwconv_bwd_data_kernel<T, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem8);
         dwconv_bwd_data_kernel<T, 8><<<grid, 256, smem8, st>>>(g2, a2, a1, da1, da2_scratch, w, B, H, W, Ch);
-        const int ntiles = B * (H / 8) * (W / 8);
-        int gx = (2 * num_sms + slabs - 1) / slabs; if (gx > ntiles) gx = ntiles;
         constexpr int wg_smem8 = 2 * (10 * (8 + 2) * 128 + 8 * 8 * 128);
-        cudaFuncSetAttribute(dwconv_bwd_wgrad_kernel<T, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, wg_smem8);
+        cudaFuncSetAttribute(dwconv_bwd_wgrad_kernel<T, 8, false, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, wg_smem8);
         CUtensorMap unused{};
-        dwconv_bwd_wgrad_kernel<T, 8><<<dim3(gx, slabs), 256, wg_smem8, st>>>(da2_scratch, h1, dw, dbias, B, H, W, Ch, unused, unused);
+        dwconv_bwd_wgrad_kernel<T, 8, false, DET><<<dim3(gx, slabs), 256, wg_smem8, st>>>(da2_scratch, h1, dw, dbias, B, H, W, Ch, unused, unused);
     }
     *err = cudaGetLastError();
     return true;

@@ -263,9 +263,16 @@ int core_only_fwd(const LewinCoreFwdArgs* a, void*, size_t, cudaStream_t stream)
     return 0;
 }
 
+size_t core_only_bwd_ws(const LewinCoreBwdArgs* a, int dtype) {
+    if (!a->deterministic) return 0;
+    DetSlabs d;
+    core_bwd_det(a, dtype, d);
+    return d.bytes;
+}
+
 // autograd of ProbAttention.forward for the saved selection: dq | dk | dv, d(bias)
 template <typename T>
-int core_only_bwd(const LewinCoreBwdArgs* a, void*, size_t, cudaStream_t stream) {
+int core_only_bwd(const LewinCoreBwdArgs* a, void* ws, size_t ws_bytes, cudaStream_t stream) {
     if (!a) return LEWIN_E_NULL;
     const LewinCoreFwdArgs* f = &a->fwd;
     if (int rc = check_core(f)) return rc;
@@ -275,16 +282,33 @@ int core_only_bwd(const LewinCoreBwdArgs* a, void*, size_t, cudaStream_t stream)
     int sms = 0;
     if (int rc = bw_device(&sms)) return rc;
     const int D = core_head_dim(f);
+    const bool det = a->deterministic != 0;
+    const int dtype = Act<T>::kIsBf16 ? LEWIN_DTYPE_BF16 : LEWIN_DTYPE_F32;
+    const size_t need = core_only_bwd_ws(a, dtype);
+    if (need && (!ws || ws_bytes < need)) return LEWIN_E_WORKSPACE;
+    if (need && !aligned16(ws)) return LEWIN_E_ALIGN;
+    DetSlabs dsl;
+    dsl.base = static_cast<unsigned char*>(ws);
+    float* slab = det ? core_bwd_det(a, dtype, dsl) : nullptr;
     CoreBwdArgs<T> c{};
     c.qkv = static_cast<const T*>(f->qkv); c.dctx = static_cast<const T*>(a->dctx); c.dqkv = static_cast<T*>(a->dqkv);
     c.top = f->top;
     c.rpb_table = f->rpb_table; c.rpb_dense = f->rpb_table ? nullptr : f->rpb_dense;
     c.d_rpb_table = a->d_rpb_table; c.d_rpb_dense = f->rpb_table ? nullptr : a->d_rpb_dense;
+    if (det) {      // at most one of the two is written (core_bwd_det)
+        c.d_rpb_table = f->rpb_table ? slab : nullptr;
+        c.d_rpb_dense = f->rpb_table ? nullptr : slab;
+        CK(dsl.clear(stream));
+    }
     c.mask = f->mask; c.nW_mask = f->mask ? f->nW_mask : 1;
     c.B_ = f->B_; c.nH = f->nH; c.C = f->nH * D; c.use_rpb = f->use_rpb;
     c.shift = 0; c.H = 8; c.W = 8; c.nWw = 1; c.nWin = 1;
-    CK(launch_core_bwd<T>(c, sms, stream));
+    CK(launch_core_bwd<T>(c, sms, det, stream));
     g_launches.fetch_add(1, std::memory_order_relaxed);
+    if (det) {
+        CK(dsl.reduce(stream));
+        g_launches.fetch_add(dsl.t.n ? 1 : 0, std::memory_order_relaxed);
+    }
     return 0;
 }
 
@@ -574,7 +598,7 @@ int lewin_probsparse_core_bwd_f32(const LewinCoreBwdArgs* a, void* ws, size_t n,
 int lewin_probsparse_core_bwd_bf16(const LewinCoreBwdArgs* a, void* ws, size_t n, lewin_stream_t s) {
     return core_only_bwd<__nv_bfloat16>(a, ws, n, reinterpret_cast<cudaStream_t>(s));
 }
-size_t lewin_probsparse_core_bwd_workspace_bytes(const LewinCoreBwdArgs*, int) { return 0; }
+size_t lewin_probsparse_core_bwd_workspace_bytes(const LewinCoreBwdArgs* a, int dtype) { return a ? core_only_bwd_ws(a, dtype) : 0; }
 int lewin_attn_fwd_kernel_mask(const LewinAttnFwdArgs* a, int dtype) {
     if (!a) return 0;
     const AttnPlan p = plan_attn(a, dtype == LEWIN_DTYPE_BF16);
@@ -644,7 +668,7 @@ const char* lewin_error_string(int code) {
         case LEWIN_E_NULL: return "required pointer is NULL";
         case LEWIN_E_SHAPE: return "unsupported shape (need H,W % 8 == 0, C % 32 == 0, C <= 1024, head_dim = C / nH in {32, 64, 128}, shift in {0..7})";
         case LEWIN_E_ALIGN: return "pointer not 16-byte aligned";
-        case LEWIN_E_WORKSPACE: return "workspace missing or too small";
+        case LEWIN_E_WORKSPACE: return "workspace missing or too small (the *_workspace_bytes query for the same arguments, deterministic flag included)";
         case LEWIN_E_DTYPE: return "unknown dtype";
         case LEWIN_E_ARCH: return "device is not compute capability 10.x (sm_100a only, no fallback)";
         default: return code > 0 ? "CUDA runtime error (cudaError_t)" : "unknown error";

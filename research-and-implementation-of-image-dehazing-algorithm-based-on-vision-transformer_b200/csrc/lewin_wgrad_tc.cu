@@ -5,5 +5,7 @@
 
 namespace lewin {
 bool wgrad_tc_supported(const WgradArgs<__nv_bfloat16>& g) { return wg3::supported(g); }
-cudaError_t wgrad_tc_launch(const WgradArgs<__nv_bfloat16>& g, int num_sms, cudaStream_t stream) { return wg3::launch(g, num_sms, stream); }
+cudaError_t wgrad_tc_launch(const WgradArgs<__nv_bfloat16>& g, int num_sms, bool det, cudaStream_t stream) {
+    return det ? wg3::launch<true>(g, num_sms, stream) : wg3::launch<false>(g, num_sms, stream);
+}
 }  // namespace lewin

@@ -35,11 +35,19 @@ struct Smem {
     int tm_live[2];                                     // per staging warp: some token has a non-zero input-mask value
 };
 
+// DET (deterministic mode): dynamic shared memory also holds DetDa, the fp32 dA rows of the item's slots; after [B3] each
+// relative-position entry of the table sums them in slot order (no shared atomics), the table partials are stored into slab
+// blockIdx.x of [gridDim.x][225, nH], and d(rpb dense) is added with plain stores into slab blockIdx.x of [gridDim.x][nH, 64, 64]
+// (zeroed by the caller).  Two CTAs per SM.
+constexpr int DA_LD = 68;
+struct DetDa { float da[32 * DA_LD]; };
+
 // TMASK: the call has an input mask per token (a.tmask); a template parameter, as in probsparse_core_v3_kernel
-template <bool TMASK>
+template <bool TMASK, bool DET = false>
 __global__ void __launch_bounds__(THREADS, 3) core_bwd_v2_kernel(const CoreBwdArgs<__nv_bfloat16> a) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     Smem& s = *reinterpret_cast<Smem*>(smem_raw);
+    float* const dab = reinterpret_cast<DetDa*>(smem_raw + sizeof(Smem))->da;      // DET only
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int gq = lane >> 2, tq = lane & 3;
     const int C3 = 3 * a.C;
@@ -229,15 +237,29 @@ __global__ void __launch_bounds__(THREADS, 3) core_bwd_v2_kernel(const CoreBwdAr
                 dot2 = fmaf(gr[j][0], p1[j][0], dot2); dot2 = fmaf(gr[j][1], p1[j][1], dot2);
             }
             dot2 = group_sum<4>(dot2);
-            if (want_tab && my_tok >= 0) {
-                float* tb = s.tacc + h * 225 + (ry + 7) * 15 + (rx - 2 * tq + 7);
+            if constexpr (DET) {
+                if (want_tab && my_tok >= 0) {
 #pragma unroll
-                for (int j = 0; j < 8; ++j) { atomicAdd(tb - j * 15, gr[j][0]); atomicAdd(tb - j * 15 - 1, gr[j][1]); }
-            }
-            if (want_dense && my_tok >= 0) {     // gradient w.r.t. the gathered bias [nH, 64, 64] (AttentionLayer.forward's argument)
-                float* dd = a.d_rpb_dense + (static_cast<long long>(h) * kTok + r) * kTok + 2 * tq;
+                    for (int j = 0; j < 8; ++j)
+                        *reinterpret_cast<float2*>(dab + (warp * 8 + gq) * DA_LD + j * 8 + 2 * tq) = make_float2(gr[j][0], gr[j][1]);
+                }
+                if (want_dense && my_tok >= 0) {
+                    float* dd = a.d_rpb_dense + static_cast<long long>(blockIdx.x) * a.nH * kTok * kTok +
+                                (static_cast<long long>(h) * kTok + r) * kTok + 2 * tq;
 #pragma unroll
-                for (int j = 0; j < 8; ++j) { atomicAdd(dd + j * 8, gr[j][0]); atomicAdd(dd + j * 8 + 1, gr[j][1]); }
+                    for (int j = 0; j < 8; ++j) { dd[j * 8] += gr[j][0]; dd[j * 8 + 1] += gr[j][1]; }
+                }
+            } else {
+                if (want_tab && my_tok >= 0) {
+                    float* tb = s.tacc + h * 225 + (ry + 7) * 15 + (rx - 2 * tq + 7);
+#pragma unroll
+                    for (int j = 0; j < 8; ++j) { atomicAdd(tb - j * 15, gr[j][0]); atomicAdd(tb - j * 15 - 1, gr[j][1]); }
+                }
+                if (want_dense && my_tok >= 0) {     // gradient w.r.t. the gathered bias [nH, 64, 64] (AttentionLayer.forward's argument)
+                    float* dd = a.d_rpb_dense + (static_cast<long long>(h) * kTok + r) * kTok + 2 * tq;
+#pragma unroll
+                    for (int j = 0; j < 8; ++j) { atomicAdd(dd + j * 8, gr[j][0]); atomicAdd(dd + j * 8 + 1, gr[j][1]); }
+                }
             }
 #pragma unroll
             for (int j = 0; j < 8; ++j) {
@@ -311,6 +333,20 @@ __global__ void __launch_bounds__(THREADS, 3) core_bwd_v2_kernel(const CoreBwdAr
             }
         }
         __syncthreads();                                                        // [B3] dS / P2 / dmean exchanged
+        if constexpr (DET) {
+            if (want_tab) {     // table entry e = (dy + 7) * 15 + (dx + 7) takes, per slot in order, the key at (ry - dy, rx - dx)
+                for (int e0 = 0; e0 < 225; e0 += THREADS) {
+                    const int e = e0 + tid, ey = e / 15 - 7, ex = e % 15 - 7;
+                    float sum = 0.f;
+                    for (int sl = 0; sl < kTopU; ++sl) {
+                        const int t = __shfl_sync(0xffffffffu, my_sel, sl);
+                        const int ly = (t >> 3) - ey, lx = (t & 7) - ex;
+                        if (e < 225 && ly >= 0 && ly < 8 && lx >= 0 && lx < 8) sum += dab[sl * DA_LD + ly * 8 + lx];
+                    }
+                    if (e < 225) s.tacc[h * 225 + e] += sum;
+                }
+            }
+        }
 
         // ================= phase B: keys 16*warp..+15:  dk = dS^T Q_sel,  dv = P2^T dctx_sel + dmean   (K = 32 slots)
         {
@@ -366,19 +402,26 @@ __global__ void __launch_bounds__(THREADS, 3) core_bwd_v2_kernel(const CoreBwdAr
         for (int i = tid; i < a.nH * 225; i += THREADS) {
             const int hh = i / 225, rel = i - hh * 225;
             const float v = s.tacc[i];
-            if (v != 0.f) atomicAdd(a.d_rpb_table + rel * a.nH + hh, v);
+            if constexpr (DET) a.d_rpb_table[static_cast<long long>(blockIdx.x) * a.nH * 225 + rel * a.nH + hh] = v;
+            else if (v != 0.f) atomicAdd(a.d_rpb_table + rel * a.nH + hh, v);
         }
     }
 }
 
-inline cudaError_t launch(const CoreBwdArgs<__nv_bfloat16>& a, int num_sms, cudaStream_t stream) {
-    auto k = a.tmask ? core_bwd_v2_kernel<true> : core_bwd_v2_kernel<false>;
-    const size_t smem = sizeof(Smem);
+// CTAs of a launch (in deterministic mode with sms = 148: the slabs of the bias gradients)
+inline long long grid(long long items, int sms, bool det) {
+    const long long cap = static_cast<long long>(sms) * (det ? 2 : 3);
+    return items < cap ? items : cap;
+}
+
+inline cudaError_t launch(const CoreBwdArgs<__nv_bfloat16>& a, int num_sms, bool det, cudaStream_t stream) {
+    auto k = det ? (a.tmask ? core_bwd_v2_kernel<true, true> : core_bwd_v2_kernel<false, true>)
+                 : (a.tmask ? core_bwd_v2_kernel<true> : core_bwd_v2_kernel<false>);
+    const size_t smem = sizeof(Smem) + (det ? sizeof(DetDa) : 0);
     cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
     if (e != cudaSuccess) return e;
     const long long items = static_cast<long long>(a.B_) * a.nH;
-    const long long cap = static_cast<long long>(num_sms) * 3;
-    k<<<static_cast<unsigned>(items < cap ? items : cap), THREADS, smem, stream>>>(a);
+    k<<<static_cast<unsigned>(grid(items, det ? 148 : num_sms, det)), THREADS, smem, stream>>>(a);
     return cudaGetLastError();
 }
 

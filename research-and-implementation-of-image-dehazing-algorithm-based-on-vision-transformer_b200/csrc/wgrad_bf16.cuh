@@ -37,7 +37,8 @@ __device__ __forceinline__ void ldsm_x2_t(uint32_t (&r)[2], const void* p) {
 }
 
 // WARPS_N warps along n (dW rows), 8 / WARPS_N along k: 4 x 2 for the 128- and 64-row tiles, 2 x 4 for the 32-row tiles of C = 32
-template <int NT, int KT, int WARPS_N>
+// DET: the per-element partials are stored into split blockIdx.z's slab of [splits][N, K] / [splits][N] instead of added
+template <int NT, int KT, int WARPS_N, bool DET = false>
 __global__ void __launch_bounds__(THREADS) wgrad_bf16_kernel(const WgradArgs<__nv_bfloat16> g) {
     using S = Smem<NT, KT>;
     constexpr int LDN = S::LDN, LDK = S::LDK;
@@ -185,6 +186,23 @@ __global__ void __launch_bounds__(THREADS) wgrad_bf16_kernel(const WgradArgs<__n
             }
         }
     }
+    if constexpr (DET) {
+        float* dW = g.dW + static_cast<long long>(blockIdx.z) * g.N * g.K;
+        float* db = g.db + static_cast<long long>(blockIdx.z) * g.N;      // (read only when want_db)
+#pragma unroll
+        for (int i = 0; i < MT; ++i)
+#pragma unroll
+            for (int half = 0; half < 2; ++half) {
+                const int n = n0 + wn * WN + i * 16 + gq + half * 8;
+#pragma unroll
+                for (int j = 0; j < NTL; ++j) {
+                    const int k = k0 + wk * WK + j * 8 + 2 * tq;
+                    *reinterpret_cast<float2*>(dW + static_cast<long long>(n) * g.K + k) = make_float2(acc[i][j][half * 2], acc[i][j][half * 2 + 1]);
+                }
+                if (want_db && tq == 0) db[n] = accb[i][half * 2];
+            }
+        return;
+    }
 #pragma unroll
     for (int i = 0; i < MT; ++i)
 #pragma unroll
@@ -204,7 +222,7 @@ inline bool supported(const WgradArgs<__nv_bfloat16>& g) {
     return !g.dy_aux && g.N % 32 == 0 && g.K % 32 == 0 && g.M < (1ll << 31);
 }
 
-template <int NT, int KT, int WARPS_N>
+template <int NT, int KT, int WARPS_N, bool DET>
 cudaError_t launch_t(WgradArgs<__nv_bfloat16> g, int num_sms, cudaStream_t st) {
     const long long tiles = static_cast<long long>(g.N / NT) * (g.K / KT);
     long long want = (static_cast<long long>(num_sms) * 3 + tiles - 1) / tiles;
@@ -213,9 +231,10 @@ cudaError_t launch_t(WgradArgs<__nv_bfloat16> g, int num_sms, cudaStream_t st) {
     if (want < 1) want = 1;
     long long rps = (g.M + want - 1) / want;
     rps = (rps + TOK - 1) / TOK * TOK;
+    if (DET) rps = det_wgrad_rows_per_split(g.M, g.N, g.K);
     const unsigned splits = static_cast<unsigned>((g.M + rps - 1) / rps);
     g.rows_per_split = rps;
-    auto k = wgrad_bf16_kernel<NT, KT, WARPS_N>;
+    auto k = wgrad_bf16_kernel<NT, KT, WARPS_N, DET>;
     const size_t smem = sizeof(Smem<NT, KT>);
     cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
     if (e != cudaSuccess) return e;
@@ -223,14 +242,15 @@ cudaError_t launch_t(WgradArgs<__nv_bfloat16> g, int num_sms, cudaStream_t st) {
     return cudaGetLastError();
 }
 
-inline cudaError_t launch(const WgradArgs<__nv_bfloat16>& g, int num_sms, cudaStream_t st) {
+template <bool DET>
+cudaError_t launch(const WgradArgs<__nv_bfloat16>& g, int num_sms, cudaStream_t st) {
     if (g.K % 64 == 0) {
-        if (g.N % 128 == 0) return launch_t<128, 64, 4>(g, num_sms, st);
-        if (g.N % 64 == 0) return launch_t<64, 64, 4>(g, num_sms, st);
-        return launch_t<32, 64, 2>(g, num_sms, st);
+        if (g.N % 128 == 0) return launch_t<128, 64, 4, DET>(g, num_sms, st);
+        if (g.N % 64 == 0) return launch_t<64, 64, 4, DET>(g, num_sms, st);
+        return launch_t<32, 64, 2, DET>(g, num_sms, st);
     }
-    if (g.N % 128 == 0) return launch_t<128, 32, 4>(g, num_sms, st);
-    return launch_t<32, 32, 2>(g, num_sms, st);
+    if (g.N % 128 == 0) return launch_t<128, 32, 4, DET>(g, num_sms, st);
+    return launch_t<32, 32, 2, DET>(g, num_sms, st);
 }
 
 }  // namespace wg2

@@ -13,7 +13,9 @@
 //   * one MMA thread issues 4 x tcgen05.mma kind::f16 (a_major = b_major = MN, K = 16 tokens each) per stage into the TMEM
 //     accumulator, plus 4 N = 16 MMAs against a constant all-ones tile whose result column is colsum(dY) (the bias gradient);
 //   * after the last stage 4 warps read the accumulator (thread == dW row), transpose 32 x 32 pieces through shared memory and
-//     add them to dW with coalesced red.global.add.f32 (splits over the token axis accumulate in place).
+//     add them to dW with coalesced red.global.add.f32 (splits over the token axis accumulate in place).  DET: the same
+//     coalesced rows are stored into split blockIdx.z's slab of [splits][N, K] (det_wgrad_rows_per_split), summed later in
+//     split order.
 // Operands with a prologue (LayerNorm, roll + window gather, DropPath scale) are materialised by their callers first
 // (ln_apply_kernel / scale_gather_rows_kernel, one C-sized pass each - small next to the hidden-sized operands).
 #pragma once
@@ -40,7 +42,7 @@ __device__ __forceinline__ uint64_t make_desc_mn(uint32_t smem_addr) {
 
 constexpr size_t fixed_smem() { return 1024 + BLK /*ones*/ + 4 * 32 * STG_LD * 4 + (2 * 8 + 1) * 8 + 16; }
 
-template <int BK>
+template <int BK, bool DET = false>
 __global__ void __launch_bounds__(THREADS, 1) wgrad_tc_kernel(const WgradArgs<__nv_bfloat16> g, const __grid_constant__ CUtensorMap dymap,
                                                              const __grid_constant__ CUtensorMap xmap, int S) {
     constexpr int NB = (BK + 63) / 64;            // 64-feature blocks of X per stage
@@ -129,7 +131,8 @@ __global__ void __launch_bounds__(THREADS, 1) wgrad_tc_kernel(const WgradArgs<__
         if (stages > 0) {
             const uint32_t t_addr = tmem_d + (static_cast<uint32_t>(warp * 32) << 16);
             const int row0 = n0 + warp * 32;          // this warp's first dW row; rows >= N exist only as zero-filled operand rows
-            float* dst = g.dW + static_cast<long long>(row0) * g.K + k0;
+            float* dW = DET ? g.dW + static_cast<long long>(blockIdx.z) * g.N * g.K : g.dW;
+            float* dst = dW + static_cast<long long>(row0) * g.K + k0;
             const int nrows = g.N - row0 < 32 ? g.N - row0 : 32;
 #pragma unroll 1
             for (int c = 0; c < BK / 32; ++c) {
@@ -138,13 +141,21 @@ __global__ void __launch_bounds__(THREADS, 1) wgrad_tc_kernel(const WgradArgs<__
 #pragma unroll
                 for (int j = 0; j < 32; ++j) my[lane * STG_LD + j] = v[j];
                 __syncwarp();
-                for (int r = 0; r < nrows; ++r) atomicAdd(dst + static_cast<long long>(r) * g.K + c * 32 + lane, my[r * STG_LD + lane]);
+                if constexpr (DET) {
+                    for (int r = 0; r < nrows; ++r) dst[static_cast<long long>(r) * g.K + c * 32 + lane] = my[r * STG_LD + lane];
+                } else {
+                    for (int r = 0; r < nrows; ++r) atomicAdd(dst + static_cast<long long>(r) * g.K + c * 32 + lane, my[r * STG_LD + lane]);
+                }
                 __syncwarp();
             }
             if (want_db) {
                 float v[32];
                 tc::tmem_ld32(t_addr + BK, v);       // 16 identical columns (+ 16 unused): colsum(dY) of this row's feature
-                if (lane < nrows) atomicAdd(g.db + row0 + lane, v[0]);
+                if constexpr (DET) {
+                    if (lane < nrows) g.db[static_cast<long long>(blockIdx.z) * g.N + row0 + lane] = v[0];
+                } else {
+                    if (lane < nrows) atomicAdd(g.db + row0 + lane, v[0]);
+                }
             }
         }
     }
@@ -162,7 +173,7 @@ inline bool supported(const WgradArgs<__nv_bfloat16>& g) {
     return tma::encode_fn() != nullptr;
 }
 
-template <int BK>
+template <int BK, bool DET>
 cudaError_t launch_bk(WgradArgs<__nv_bfloat16> g, int num_sms, cudaStream_t stream) {
     constexpr int STAGE = 2 * BLK + ((BK + 63) / 64) * BLK;
     constexpr size_t fixed = fixed_smem();
@@ -172,7 +183,7 @@ cudaError_t launch_bk(WgradArgs<__nv_bfloat16> g, int num_sms, cudaStream_t stre
     CUtensorMap dymap{}, xmap{};
     if (!tma::make_2d_bf16_sw128(&dymap, g.dY, g.M, g.N, g.lddy, TOK) || !tma::make_2d_bf16_sw128(&xmap, g.X, g.M, g.K, g.ldx, TOK))
         return cudaErrorNotSupported;
-    auto k = wgrad_tc_kernel<BK>;
+    auto k = wgrad_tc_kernel<BK, DET>;
     cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
     if (e != cudaSuccess) return e;
     const int n_tiles = (g.N + NT - 1) / NT;
@@ -183,19 +194,21 @@ cudaError_t launch_bk(WgradArgs<__nv_bfloat16> g, int num_sms, cudaStream_t stre
     if (want < 1) want = 1;
     long long rps = (g.M + want - 1) / want;
     rps = (rps + TOK - 1) / TOK * TOK;
+    if (DET) rps = det_wgrad_rows_per_split(g.M, g.N, g.K);
     const unsigned splits = static_cast<unsigned>((g.M + rps - 1) / rps);
     g.rows_per_split = rps;
     k<<<dim3(n_tiles, g.K / BK, splits), THREADS, smem, stream>>>(g, dymap, xmap, S);
     return cudaGetLastError();
 }
 
-inline cudaError_t launch(const WgradArgs<__nv_bfloat16>& g, int num_sms, cudaStream_t stream) {
-    if (g.K % 256 == 0) return launch_bk<256>(g, num_sms, stream);
-    if (g.K == 128) return launch_bk<128>(g, num_sms, stream);
-    if (g.K == 64) return launch_bk<64>(g, num_sms, stream);
-    if (g.K == 32) return launch_bk<32>(g, num_sms, stream);
-    if (g.K == 96) return launch_bk<96>(g, num_sms, stream);
-    if (g.K == 192) return launch_bk<192>(g, num_sms, stream);
+template <bool DET>
+cudaError_t launch(const WgradArgs<__nv_bfloat16>& g, int num_sms, cudaStream_t stream) {
+    if (g.K % 256 == 0) return launch_bk<256, DET>(g, num_sms, stream);
+    if (g.K == 128) return launch_bk<128, DET>(g, num_sms, stream);
+    if (g.K == 64) return launch_bk<64, DET>(g, num_sms, stream);
+    if (g.K == 32) return launch_bk<32, DET>(g, num_sms, stream);
+    if (g.K == 96) return launch_bk<96, DET>(g, num_sms, stream);
+    if (g.K == 192) return launch_bk<192, DET>(g, num_sms, stream);
     return cudaErrorInvalidValue;
 }
 

@@ -7,5 +7,6 @@ namespace lewin {
 // true if dW[N,K] += dY^T X with these arguments can run on the tensor-memory kernel: plain bf16 operands (no gather / LN /
 // DropPath / gelu' prologue), N % 128 == 0, K % 128 == 0
 bool wgrad_tc_supported(const WgradArgs<__nv_bfloat16>& g);
-cudaError_t wgrad_tc_launch(const WgradArgs<__nv_bfloat16>& g, int num_sms, cudaStream_t stream);
+// det: stores per-split partials into the slabs g.dW / g.db (det_wgrad_rows_per_split) instead of accumulating
+cudaError_t wgrad_tc_launch(const WgradArgs<__nv_bfloat16>& g, int num_sms, bool det, cudaStream_t stream);
 }  // namespace lewin

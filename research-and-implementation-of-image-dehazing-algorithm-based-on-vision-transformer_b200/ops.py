@@ -52,13 +52,20 @@ def _dtype_tag(x):
         raise RuntimeError(f"lewin_b200: unsupported activation dtype {x.dtype} (float32 or bfloat16)") from None
 
 
+def _deterministic():
+    """The `deterministic` field of the backward calls: torch.use_deterministic_algorithms(True) (warn_only included, since
+    the library has a deterministic implementation) asks for fixed-order parameter-gradient sums.  Read at backward time."""
+    return int(torch.are_deterministic_algorithms_enabled())
+
+
 def _workspace(nbytes, device):
     return torch.empty(max(int(nbytes), 16), dtype=torch.uint8, device=device)
 
 
 def _zero_grads(like, device, separate=False):
     """fp32 zero gradient buffers for the given parameter tensors (None entries stay None): ONE flat allocation and one
-    fill kernel, handed out as views (the backward kernels accumulate into them with atomics).  separate=True gives every
+    fill kernel, handed out as views (each backward call accumulates into them: with fp32 atomics, or with one add per element
+    under torch.use_deterministic_algorithms).  separate=True gives every
     gradient its own storage (returns of a torch.library op may not alias each other)."""
     if separate:
         return [None if t is None else torch.zeros(t.shape, dtype=torch.float32, device=device) for t in like]
@@ -288,7 +295,7 @@ def _attn_backward(saved, geom, dy, separate_grads=False):
     a = _lib.LewinAttnBwdArgs(
         fwd=fwd, dy=_ptr(dy), dx=_ptr(dx), d_ln_w=_ptr(d_ln_w), d_ln_b=_ptr(d_ln_b),
         d_w_qkv=_ptr(d_w_qkv), d_b_qkv=_ptr(d_b_qkv), d_w_out=_ptr(d_w_out), d_b_out=_ptr(d_b_out),
-        d_rpb_table=_ptr(d_tab), d_rpb_dense=_ptr(d_dense))
+        d_rpb_table=_ptr(d_tab), d_rpb_dense=_ptr(d_dense), deterministic=_deterministic())
     ws = _workspace(lib.lewin_attn_bwd_workspace_bytes(a, _lib.DTYPE_TAG[dt]), dev)
     fn = getattr(lib, f"lewin_attn_bwd_{dt}")
     with torch.cuda.device(dev):
@@ -379,7 +386,8 @@ def _leff_backward(saved, geom, dout, separate_grads=False):
         h1=_ptr(h1), h2=_ptr(h2), a1=_ptr(a1), a2=_ptr(a2))
     a = _lib.LewinLeffBwdArgs(
         fwd=fwd, dout=_ptr(dout), dy=_ptr(dy), d_ln_w=_ptr(d_ln_w), d_ln_b=_ptr(d_ln_b),
-        d_w1=_ptr(d_w1), d_b1=_ptr(d_b1), d_w_dw=_ptr(d_wdw), d_b_dw=_ptr(d_bdw), d_w2=_ptr(d_w2), d_b2=_ptr(d_b2))
+        d_w1=_ptr(d_w1), d_b1=_ptr(d_b1), d_w_dw=_ptr(d_wdw), d_b_dw=_ptr(d_bdw), d_w2=_ptr(d_w2), d_b2=_ptr(d_b2),
+        deterministic=_deterministic())
     ws = _workspace(lib.lewin_leff_bwd_workspace_bytes(a, _lib.DTYPE_TAG[dt]), dev)
     fn = getattr(lib, f"lewin_leff_bwd_{dt}")
     with torch.cuda.device(dev):
@@ -492,7 +500,8 @@ class _CoreFn(torch.autograd.Function):
                                     head_dim=C3 // 3 // nH, reserved=0,
                                     qkv=_ptr(qkv), ctx=_ptr(dctx), rpb_table=_ptr(tab), rpb_dense=_ptr(dense),
                                     index_sample=None, mask=_ptr(mask), top=_ptr(top))
-        a = _lib.LewinCoreBwdArgs(fwd=fwd, dctx=_ptr(dctx), dqkv=_ptr(dqkv), d_rpb_table=_ptr(d_tab), d_rpb_dense=_ptr(d_dense))
+        a = _lib.LewinCoreBwdArgs(fwd=fwd, dctx=_ptr(dctx), dqkv=_ptr(dqkv), d_rpb_table=_ptr(d_tab), d_rpb_dense=_ptr(d_dense),
+                                  deterministic=_deterministic())
         ws = _workspace(lib.lewin_probsparse_core_bwd_workspace_bytes(a, _lib.DTYPE_TAG[dt]), dev)
         fn = getattr(lib, f"lewin_probsparse_core_bwd_{dt}")
         with torch.cuda.device(dev):

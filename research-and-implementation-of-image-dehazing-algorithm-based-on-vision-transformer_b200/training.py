@@ -141,6 +141,7 @@ class TrainStep:
         self.idx = model.draw_index_samples().to(self.dev, dtype=torch.int32)
         self._loss = torch.zeros((), device=self.dev)
         self._graph = None
+        self._graph_deterministic = None
         self.steps = 0
 
     # ---------------------------------------------------------------- pieces
@@ -175,10 +176,19 @@ class TrainStep:
             self.opt.step()
             self._loss.copy_(loss.detach())
         self._graph = g
+        self._graph_deterministic = torch.are_deterministic_algorithms_enabled()
 
     # ---------------------------------------------------------------- public
     def step(self, input_, target, epoch=0):
-        """One iteration on device (or pinned-host) tensors ``input_`` (hazy) and ``target`` (clean), [B, 3, H, W] in [0, 1]."""
+        """One iteration on device (or pinned-host) tensors ``input_`` (hazy) and ``target`` (clean), [B, 3, H, W] in [0, 1].
+
+        A captured graph keeps the backward kernels of the torch.use_deterministic_algorithms setting it was captured under;
+        if the setting has changed since, this raises instead of replaying them."""
+        if self._graph is not None and torch.are_deterministic_algorithms_enabled() != self._graph_deterministic:
+            raise RuntimeError(
+                "TrainStep: torch.use_deterministic_algorithms changed since this step's CUDA graph was captured "
+                f"(captured with {self._graph_deterministic}); a captured graph cannot switch its backward kernels. "
+                "Build a new TrainStep after changing the setting.")
         input_ = input_.to(self.dev, non_blocking=True)
         target = target.to(self.dev, non_blocking=True)
         if self.mixup_after_epoch is not None and epoch > self.mixup_after_epoch:       # My_train.py:220-221
