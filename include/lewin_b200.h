@@ -151,8 +151,9 @@ int lewin_attn_fwd_bf16(const LewinAttnFwdArgs* a, void* workspace, size_t works
 
 /* Backward of the attention half (autograd of the same reference lines; gradient paths in
  * SURVEY.md section 3.4).  Gradients of parameters are ACCUMULATED (+=) into fp32 buffers the
- * caller zero-initialises, dx is written.  Shapes as the forward's (C % 32 == 0, C <= 1024,
- * head_dim = C / nH in {32, 64, 128}) with nH <= 16; anything else returns LEWIN_E_SHAPE.
+ * caller zero-initialises, dx is written.  `fwd` is checked with the forward's rules (shape, mask, band, token mask,
+ * 16-byte alignment of every pointer given; y and index_sample are not read and may be NULL) and the same codes, plus
+ * nH <= 16 (LEWIN_E_SHAPE); dy, dx and every gradient pointer given must be 16-byte aligned (LEWIN_E_ALIGN).
  *
  * `deterministic` (all three backward structs): 0 = parameter gradients are summed with fp32 atomics, whose order varies from
  * run to run.  1 = every parameter gradient of the call is a fixed-order sum: each reduction unit stores its partial into its
@@ -272,8 +273,8 @@ int lewin_leff_fwd_f32 (const LewinLeffFwdArgs* a, void* workspace, size_t works
 int lewin_leff_fwd_bf16(const LewinLeffFwdArgs* a, void* workspace, size_t workspace_bytes, lewin_stream_t stream);
 
 /* Backward of the LeFF half: parameter gradients ACCUMULATED into zero-initialised fp32 buffers (with `deterministic` = 1 as
- * fixed-order sums, see LewinAttnBwdArgs), dy written.
- * C % 32 == 0, hidden % 32 == 0, C <= 1024 (as the forward); anything else returns LEWIN_E_SHAPE. */
+ * fixed-order sums, see LewinAttnBwdArgs), dy written.  `fwd` is checked with the forward's rules and codes (out is not
+ * read and may be NULL); dout, dy and every gradient pointer given must be 16-byte aligned (LEWIN_E_ALIGN). */
 typedef struct {
     LewinLeffFwdArgs fwd;
     const void* dout;              /* gradient of `out` */

@@ -38,8 +38,7 @@ def attn_fwd(x: Tensor, ln_w: Optional[Tensor], ln_b: Optional[Tensor], w_qkv: T
                                       drop_scale, geom, token_mask)
     if not save:
         return y, top, x.new_empty((0,)), x.new_empty((0,))
-    qkv, cbuf = saved[12], saved[13]
-    return y, top, qkv, (cbuf if cbuf is not qkv else cbuf.clone())       # op outputs must not alias
+    return y, top, saved.qkv, (saved.ctx if saved.ctx is not saved.qkv else saved.ctx.clone())      # op outputs must not alias
 
 
 @attn_fwd.register_fake
@@ -63,9 +62,9 @@ def attn_bwd(dy: Tensor, x: Tensor, ln_w: Optional[Tensor], ln_b: Optional[Tenso
     """-> (dx, d_ln_w, d_ln_b, d_w_qkv, d_b_qkv, d_w_out, d_b_out, d_rpb); d_rpb has the shape of whichever bias was given."""
     geom = (B, H, W, num_heads, shift, windowed, use_rpb, analytic_shift_mask, True)
     f = ops._f32c
-    saved = (x.contiguous(), f(ln_w), f(ln_b), f(w_qkv), f(b_qkv), f(w_out), f(b_out), f(rpb_table), f(rpb_dense),
-             ops.prepare_index_sample(index_sample, x.device), f(mask), f(drop_scale), qkv, ctx, top,
-             ops._token_mask(token_mask, B, H, W, x.device))
+    saved = ops.AttnSaved(x.contiguous(), f(ln_w), f(ln_b), f(w_qkv), f(b_qkv), f(w_out), f(b_out), f(rpb_table), f(rpb_dense),
+                          ops.prepare_index_sample(index_sample, x.device), f(mask), f(drop_scale), qkv, ctx, top,
+                          ops._token_mask(token_mask, B, H, W, x.device))
     dx, d_ln_w, d_ln_b, d_wq, d_bq, d_wo, d_bo, d_tab, d_dense = ops._attn_backward(saved, geom, dy, separate_grads=True)
     d_rpb = d_tab if d_tab is not None else d_dense
     z = dx.new_empty((0,), dtype=torch.float32)
@@ -121,8 +120,7 @@ def leff_fwd(y: Tensor, ln_w: Optional[Tensor], ln_b: Optional[Tensor], w1: Tens
     out, saved = ops._leff_forward(y, ln_w, ln_b, w1, b1, w_dw, b_dw, w2, b2, drop_scale, (B, H, W, fused, save))
     if saved is None:
         return (out,) + tuple(y.new_empty((0,)) for _ in range(4))
-    h1, h2, a1, a2 = saved[10:14]
-    return out, h1, (h2 if h2 is not h1 else h2.clone()), a1, a2          # op outputs must not alias
+    return out, saved.h1, (saved.h2 if saved.h2 is not saved.h1 else saved.h2.clone()), saved.a1, saved.a2      # no aliasing
 
 
 @leff_fwd.register_fake
@@ -139,7 +137,8 @@ def leff_bwd(dout: Tensor, y: Tensor, ln_w: Optional[Tensor], ln_b: Optional[Ten
              ) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor, Tensor, Tensor, Tensor, Tensor]:
     """-> (dy, d_ln_w, d_ln_b, d_w1, d_b1, d_w_dw, d_b_dw, d_w2, d_b2)."""
     f = ops._f32c
-    saved = (y.contiguous(), f(ln_w), f(ln_b), f(w1), f(b1), f(w_dw), f(b_dw), f(w2), f(b2), f(drop_scale), h1, h2, a1, a2)
+    saved = ops.LeffSaved(y.contiguous(), f(ln_w), f(ln_b), f(w1), f(b1), f(w_dw), f(b_dw), f(w2), f(b2), f(drop_scale), h1, h2,
+                          a1, a2)
     dy, d_ln_w, d_ln_b, *rest = ops._leff_backward(saved, (B, H, W, fused, True), dout, separate_grads=True)
     z = dy.new_empty((0,), dtype=torch.float32)
     return (dy, _req(d_ln_w, z), _req(d_ln_b, z)) + tuple(rest)

@@ -27,10 +27,10 @@
 #include "wgrad_tc_api.h"
 #include "core_bwd_args.cuh"
 #include "probsparse_core_bwd_v2.cuh"
+#include "ws_layout.h"
 
 namespace lewin {
 
-inline size_t bw_align(size_t v) { return (v + 255) / 256 * 256; }
 
 // ------------------------------------------------------------------------------ transpose
 __global__ void transpose_kernel(const float* __restrict__ src, float* __restrict__ dst, int R, int Cc) {
@@ -1077,21 +1077,19 @@ __global__ void __launch_bounds__(256) det_reduce_kernel(const DetTable t) {
     }
 }
 
-// The slabs of one backward call, in the order the call registers them: the workspace query (base == nullptr) and the launch
-// run the same registration code, so slot counts and offsets have a single source.
+// The slabs of one backward call, in the order the call registers them, taken from the call's workspace layout: the workspace
+// query (a counting layout) and the launch run the same registration code, so slot counts and offsets have a single source.
 struct DetSlabs {
-    unsigned char* base = nullptr;
-    size_t bytes = 0;
+    WsLayout* layout = nullptr;           // set by the entry's layout function before it registers a slab
     DetTable t{};
     bool zero[kDetMaxSums] = {};          // the slab has elements no unit stores: cleared before the kernels run
     bool overflow = false;                // more slabs than the reduction table holds: clear() refuses, nothing is launched
     float* add(float* dst, long long slots, long long len, bool holes = false) {
         if (t.n == kDetMaxSums) { overflow = true; return nullptr; }
-        float* p = base ? reinterpret_cast<float*>(base + bytes) : nullptr;
+        float* p = layout->take<float>(static_cast<size_t>(slots) * static_cast<size_t>(len) * sizeof(float));
         t.e[t.n] = DetSum{p, dst, slots, len};
         zero[t.n] = holes;
         ++t.n;
-        bytes += bw_align(static_cast<size_t>(slots) * static_cast<size_t>(len) * sizeof(float));
         return p;
     }
     cudaError_t clear(cudaStream_t st) const {      // called before the first kernel of the call
@@ -1176,41 +1174,6 @@ inline float* core_bwd_det(const LewinCoreBwdArgs* a, int dtype, DetSlabs& d) {
     return nullptr;
 }
 
-// ------------------------------------------------------------------------------ host orchestration
-#define BCK(expr)                                           \
-    do {                                                    \
-        cudaError_t _e = (expr);                            \
-        if (_e != cudaSuccess) return static_cast<int>(_e); \
-    } while (0)
-
-inline int bw_device(int* sms) {
-    int dev = 0, cc = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess) return LEWIN_E_ARCH;
-    cudaDeviceGetAttribute(sms, cudaDevAttrMultiProcessorCount, dev);
-    cudaDeviceGetAttribute(&cc, cudaDevAttrComputeCapabilityMajor, dev);
-    return cc == 10 ? 0 : LEWIN_E_ARCH;
-}
-
-inline size_t attn_bwd_ws_base(const LewinAttnBwdArgs* a, int dtype) {
-    const LewinAttnFwdArgs& f = a->fwd;
-    const size_t tokens = static_cast<size_t>(f.B) * f.H * f.W;
-    const size_t es = dtype == LEWIN_DTYPE_BF16 ? 2 : 4;
-    const size_t C = f.C;
-    return 2 * bw_align(tokens * 4) + bw_align(tokens * C * es) + bw_align(tokens * 3 * C * es) +
-           bw_align(tokens * C * es) + bw_align(C * C * 4) + bw_align(3 * C * C * 4) +
-           (dtype == LEWIN_DTYPE_BF16 ? bw_align(3 * C * C * 2) + bw_align(C * C * 2) + bw_align(tokens * C * 2) : 0);
-           // bf16: images of W_qkv^T / W_out^T and the scaled, window-ordered dy rows for the streamed-W GEMMs
-}
-// + the partial slabs of deterministic mode after the rest
-inline size_t attn_bwd_ws(const LewinAttnBwdArgs* a, int dtype) {
-    size_t n = attn_bwd_ws_base(a, dtype);
-    if (a->deterministic) {
-        DetSlabs d;
-        attn_bwd_det(a, dtype, d);
-        n += d.bytes;
-    }
-    return n;
-}
 
 // Data-gradient GEMM dX = dY . W (W^T staged as the [N, K] operand).  bf16 at the C >= 256 levels: the forward's
 // warp-specialised streamed-W tcgen05 kernel (TMA operands, 3x the first-generation kernel's rate) whenever the operand
@@ -1274,271 +1237,7 @@ inline cudaError_t launch_dgrad_gemm(const GemmArgs<T>& g, __nv_bfloat16* wT_bf1
             return ws::wss_launch<EPI_BIAS>(h, wT_bf16, sms, st);
         }
     }
-    return launch_gemm_any<T, EPI_BIAS>(g, st);
-}
-
-// LewinAttnFwdArgs::token_mask: the fused block half of a whole image only, never with the dense mask, Bm divides B
-inline int check_token_mask(const LewinAttnFwdArgs* a) {
-    if (!a->token_mask) return 0;
-    if (a->windowed || a->band_mode || a->mask || a->Bm <= 0 || a->B % a->Bm) return LEWIN_E_SHAPE;
-    if (reinterpret_cast<uintptr_t>(a->token_mask) & 15u) return LEWIN_E_ALIGN;
-    return 0;
-}
-
-template <typename T>
-int attn_bwd(const LewinAttnBwdArgs* a, void* ws, size_t ws_bytes, cudaStream_t st) {
-    if (!a || !a->dy || !a->dx) return LEWIN_E_NULL;
-    const LewinAttnFwdArgs& f = a->fwd;
-    if (!f.x || !f.w_qkv || !f.w_out || !f.qkv || !f.ctx || !f.top) return LEWIN_E_NULL;
-    if (!a->d_w_qkv || !a->d_b_qkv || !a->d_w_out || !a->d_b_out) return LEWIN_E_NULL;
-    if (!f.windowed && (!f.ln_w || !f.ln_b || !a->d_ln_w || !a->d_ln_b)) return LEWIN_E_NULL;
-    if (f.H % 8 || f.W % 8 || f.C % 32 || !head_dim_ok(f.C, f.nH) || f.C > 1024 || f.nH > 16) return LEWIN_E_SHAPE;
-    if (int rc = check_token_mask(&f)) return rc;
-    int sms = 0;
-    if (int rc = bw_device(&sms)) return rc;
-    const int dtype = Act<T>::kIsBf16 ? LEWIN_DTYPE_BF16 : LEWIN_DTYPE_F32;
-    if (!ws || ws_bytes < attn_bwd_ws(a, dtype)) return LEWIN_E_WORKSPACE;
-    const bool det = a->deterministic != 0;
-    if (det && (reinterpret_cast<uintptr_t>(ws) & 15u)) return LEWIN_E_ALIGN;
-    DetSlabs dsl;
-    dsl.base = static_cast<unsigned char*>(ws) + attn_bwd_ws_base(a, dtype);
-    const AttnDet dt = det ? attn_bwd_det(a, dtype, dsl) : AttnDet{};
-    if (det) BCK(dsl.clear(st));
-
-    const long long tokens = static_cast<long long>(f.B) * f.H * f.W;
-    const int C = f.C, nWin = (f.H / 8) * (f.W / 8), B_ = f.B * nWin;
-    const int tpi = f.H * f.W;
-    unsigned char* p = static_cast<unsigned char*>(ws);
-    float* mean = reinterpret_cast<float*>(p); p += bw_align(tokens * 4);
-    float* rstd = reinterpret_cast<float*>(p); p += bw_align(tokens * 4);
-    T* dctx = reinterpret_cast<T*>(p); p += bw_align(tokens * C * sizeof(T));
-    T* dqkv = reinterpret_cast<T*>(p); p += bw_align(tokens * 3 * C * sizeof(T));
-    T* dxh = reinterpret_cast<T*>(p); p += bw_align(tokens * C * sizeof(T));
-    float* woT = reinterpret_cast<float*>(p); p += bw_align(static_cast<size_t>(C) * C * 4);
-    float* wqkvT = reinterpret_cast<float*>(p); p += bw_align(static_cast<size_t>(3) * C * C * 4);
-    __nv_bfloat16* wqkvT_b = Act<T>::kIsBf16 ? reinterpret_cast<__nv_bfloat16*>(p) : nullptr;
-    p += bw_align(static_cast<size_t>(3) * C * C * 2);
-    __nv_bfloat16* woT_b = Act<T>::kIsBf16 ? reinterpret_cast<__nv_bfloat16*>(p) : nullptr;
-    p += bw_align(static_cast<size_t>(C) * C * 2);
-    __nv_bfloat16* dy_s = Act<T>::kIsBf16 ? reinterpret_cast<__nv_bfloat16*>(p) : nullptr;
-
-    const T* x = static_cast<const T*>(f.x);
-    const T* dy = static_cast<const T*>(a->dy);
-    WinMap map{f.H, f.W, f.W / 8, nWin, f.shift, f.shift};
-    const int mapped = f.windowed ? 0 : 1;
-
-    // W_out [C(out), C(in)] -> as the [N = in, K = out] operand of dctx = do . W_out
-    BCK(launch_transpose(f.w_out, woT, C, C, st));
-    BCK(launch_transpose(f.w_qkv, wqkvT, 3 * C, C, st));
-
-    bool dy_s_filled = false;
-    {   // dctx = (s_b * gather(dy)) . W_out
-        GemmArgs<T> g{};
-        g.A = dy; g.lda = C; g.Wt = woT; g.bias = nullptr;
-        g.Y = dctx; g.ldy = C; g.M = tokens; g.N = C; g.K = C;
-        g.mapA = mapped; g.mapY = 0; g.map = map; g.tokens_per_image = tpi;
-        g.a_row_scale = f.windowed ? nullptr : f.drop_scale;
-        BCK(launch_dgrad_gemm<T>(g, woT_b, sms, st, dy_s, &dy_s_filled));
-    }
-    {   // dW_out += do^T ctx ; db_out += colsum(do)
-        WgradArgs<T> w{};
-        w.dY = dy; w.lddy = C; w.X = static_cast<const T*>(f.ctx); w.ldx = C;
-        w.dW = det ? dt.w_out : a->d_w_out; w.db = det ? dt.b_out : a->d_b_out; w.M = tokens; w.N = C; w.K = C;
-        w.mapDY = mapped; w.mapX = 0; w.map = map; w.tokens_per_image = tpi;
-        w.dy_row_scale = f.windowed ? nullptr : f.drop_scale;
-        if constexpr (Act<T>::kIsBf16) {
-            // plain operand for the tcgen05 kernel: the window-ordered, DropPath-scaled rows (left behind by the data-gradient
-            // GEMM at C >= 128, made here otherwise)
-            WgradArgs<T> v = w;
-            v.dY = dy_s; v.mapDY = 0; v.dy_row_scale = nullptr;
-            if ((w.mapDY || w.dy_row_scale) && wgrad_tc_supported(v)) {
-                if (!dy_s_filled) BCK(launch_scale_gather_rows(dy, dy_s, w.dy_row_scale, tokens, C, C, mapped, map, tpi, sms, st));
-                w = v;
-            }
-        }
-        BCK(launch_wgrad<T>(w, sms, det, st));
-    }
-    {   // core backward -> dq | dk | dv
-        CoreBwdArgs<T> c{};
-        c.qkv = static_cast<const T*>(f.qkv); c.dctx = dctx; c.dqkv = dqkv; c.top = f.top;
-        c.rpb_table = f.rpb_table; c.rpb_dense = f.rpb_table ? nullptr : f.rpb_dense;
-        c.d_rpb_table = det ? dt.rpb_table : a->d_rpb_table;
-        c.d_rpb_dense = det ? dt.rpb_dense : a->d_rpb_dense;
-        c.mask = f.mask; c.nW_mask = f.mask ? f.nW_mask : 1;
-        c.B_ = B_; c.nH = f.nH; c.C = C; c.use_rpb = f.use_rpb;
-        c.shift = (f.analytic_shift_mask && !f.windowed) ? f.shift : 0;
-        c.H = f.H; c.W = f.W; c.nWw = f.W / 8; c.nWin = nWin;
-        c.tmask = f.token_mask; c.Bm = f.token_mask ? f.Bm : 1;
-        BCK(launch_core_bwd<T>(c, sms, det, st));
-    }
-    {   // dW_qkv += dqkv^T LN1(x)[window order] ; db_qkv += colsum(dqkv)
-        WgradArgs<T> w{};
-        w.dY = dqkv; w.lddy = 3 * C; w.X = x; w.ldx = C;
-        w.dW = det ? dt.w_qkv : a->d_w_qkv; w.db = det ? dt.b_qkv : a->d_b_qkv; w.M = tokens; w.N = 3 * C; w.K = C;
-        w.mapDY = 0; w.mapX = mapped; w.map = map; w.tokens_per_image = tpi;
-        if (!f.windowed) { w.mean = mean; w.rstd = rstd; w.ln_w = f.ln_w; w.ln_b = f.ln_b; }
-        if constexpr (Act<T>::kIsBf16) {
-            // LN1 + roll + window_partition in one C-sized pass (into dxh, which is free until the next GEMM writes
-            // it), so the weight gradient streams plain rows into the tcgen05 kernel
-            WgradArgs<T> v = w;
-            v.X = dxh; v.mapX = 0; v.mean = nullptr; v.rstd = nullptr; v.ln_w = nullptr; v.ln_b = nullptr;
-            if (!f.windowed && wgrad_tc_supported(v)) {
-                BCK(launch_ln_apply(x, dxh, f.ln_w, f.ln_b, tokens, C, 1, map, st));
-                w = v;
-            }
-        }
-        if (w.mean) BCK(launch_ln_stats<T>(x, tokens, C, mean, rstd, st));      // only the register-prologue kernels need them
-        BCK(launch_wgrad<T>(w, sms, det, st));
-    }
-    {   // d(LN1 out) = dqkv . W_qkv, scattered back to token order (window_reverse + un-roll)
-        GemmArgs<T> g{};
-        g.A = dqkv; g.lda = 3 * C; g.Wt = wqkvT; g.bias = nullptr;
-        g.Y = f.windowed ? static_cast<T*>(a->dx) : dxh; g.ldy = C; g.M = tokens; g.N = C; g.K = 3 * C;
-        g.mapA = 0; g.mapY = mapped; g.map = map; g.tokens_per_image = tpi;
-        BCK(launch_dgrad_gemm<T>(g, wqkvT_b, sms, st));
-    }
-    if (!f.windowed)   // dx = dy + LN1_bwd(dxh)
-        BCK(launch_ln_bwd<T>(dxh, x, dy, static_cast<T*>(a->dx), f.ln_w, det ? dt.ln_w : a->d_ln_w, det ? dt.ln_b : a->d_ln_b,
-                             tokens, C, sms, det, st));
-    if (det) BCK(dsl.reduce(st));
-    return 0;
-}
-
-inline size_t leff_bwd_ws_base(const LewinLeffBwdArgs* a, int dtype) {
-    const LewinLeffFwdArgs& f = a->fwd;
-    const size_t tokens = static_cast<size_t>(f.B) * f.H * f.W;
-    const size_t es = dtype == LEWIN_DTYPE_BF16 ? 2 : 4;
-    const size_t C = f.C, Ch = f.hidden;
-    return 2 * bw_align(tokens * 4) + 3 * bw_align(tokens * Ch * es) + bw_align(tokens * C * es) + 2 * bw_align(C * Ch * 4) +
-           (dtype == LEWIN_DTYPE_BF16 ? 2 * bw_align(C * Ch * 2) + bw_align(tokens * C * 2) : 0);
-           // bf16: images of W2^T, W1^T and the DropPath-scaled dout rows
-}
-// + the partial slabs of deterministic mode after the rest
-inline size_t leff_bwd_ws(const LewinLeffBwdArgs* a, int dtype) {
-    size_t n = leff_bwd_ws_base(a, dtype);
-    if (a->deterministic) {
-        DetSlabs d;
-        leff_bwd_det(a, dtype, d);
-        n += d.bytes;
-    }
-    return n;
-}
-
-template <typename T>
-int leff_bwd(const LewinLeffBwdArgs* a, void* ws, size_t ws_bytes, cudaStream_t st) {
-    if (!a || !a->dout || !a->dy) return LEWIN_E_NULL;
-    const LewinLeffFwdArgs& f = a->fwd;
-    if (!f.y || !f.w1 || !f.w_dw || !f.w2 || !f.h1 || !f.h2 || !f.a1 || !f.a2) return LEWIN_E_NULL;
-    if (!a->d_w1 || !a->d_b1 || !a->d_w_dw || !a->d_b_dw || !a->d_w2 || !a->d_b2) return LEWIN_E_NULL;
-    if (f.fused && (!f.ln_w || !f.ln_b || !a->d_ln_w || !a->d_ln_b)) return LEWIN_E_NULL;
-    if (f.C % 32 || f.hidden % 32 || f.C > 1024) return LEWIN_E_SHAPE;
-    int sms = 0;
-    if (int rc = bw_device(&sms)) return rc;
-    const int dtype = Act<T>::kIsBf16 ? LEWIN_DTYPE_BF16 : LEWIN_DTYPE_F32;
-    if (!ws || ws_bytes < leff_bwd_ws(a, dtype)) return LEWIN_E_WORKSPACE;
-    const bool det = a->deterministic != 0;
-    if (det && (reinterpret_cast<uintptr_t>(ws) & 15u)) return LEWIN_E_ALIGN;
-    DetSlabs dsl;
-    dsl.base = static_cast<unsigned char*>(ws) + leff_bwd_ws_base(a, dtype);
-    const LeffDet dt = det ? leff_bwd_det(a, dtype, dsl) : LeffDet{};
-    if (det) BCK(dsl.clear(st));
-
-    const long long tokens = static_cast<long long>(f.B) * f.H * f.W;
-    const int C = f.C, Ch = f.hidden, tpi = f.H * f.W;
-    unsigned char* p = static_cast<unsigned char*>(ws);
-    float* mean = reinterpret_cast<float*>(p); p += bw_align(tokens * 4);
-    float* rstd = reinterpret_cast<float*>(p); p += bw_align(tokens * 4);
-    T* dh2 = reinterpret_cast<T*>(p); p += bw_align(tokens * Ch * sizeof(T));
-    T* da1 = reinterpret_cast<T*>(p); p += bw_align(tokens * Ch * sizeof(T));
-    T* da2 = reinterpret_cast<T*>(p); p += bw_align(tokens * Ch * sizeof(T));
-    T* dz = reinterpret_cast<T*>(p); p += bw_align(tokens * C * sizeof(T));
-    float* w2T = reinterpret_cast<float*>(p); p += bw_align(static_cast<size_t>(C) * Ch * 4);
-    float* w1T = reinterpret_cast<float*>(p); p += bw_align(static_cast<size_t>(C) * Ch * 4);
-    __nv_bfloat16* w2T_b = Act<T>::kIsBf16 ? reinterpret_cast<__nv_bfloat16*>(p) : nullptr;
-    __nv_bfloat16* w1T_b = Act<T>::kIsBf16 ? reinterpret_cast<__nv_bfloat16*>(p + bw_align(static_cast<size_t>(C) * Ch * 2)) : nullptr;
-    __nv_bfloat16* dout_s = Act<T>::kIsBf16 ? reinterpret_cast<__nv_bfloat16*>(p + 2 * bw_align(static_cast<size_t>(C) * Ch * 2)) : nullptr;
-
-    const T* y = static_cast<const T*>(f.y);
-    const T* dout = static_cast<const T*>(a->dout);
-    const float* dscale = f.fused ? f.drop_scale : nullptr;
-
-    BCK(launch_transpose(f.w2, w2T, C, Ch, st));      // [C, Ch] -> [Ch, C]  (N = Ch, K = C)
-    BCK(launch_transpose(f.w1, w1T, Ch, C, st));      // [Ch, C] -> [C, Ch]  (N = C, K = Ch)
-
-    bool dout_s_filled = false;
-    {   // dh2 = (s*dout) . W2
-        GemmArgs<T> g{};
-        g.A = dout; g.lda = C; g.Wt = w2T; g.bias = nullptr;
-        g.Y = dh2; g.ldy = Ch; g.M = tokens; g.N = Ch; g.K = C;
-        g.tokens_per_image = tpi; g.a_row_scale = dscale;
-        BCK(launch_dgrad_gemm<T>(g, w2T_b, sms, st, dout_s, &dout_s_filled));
-    }
-    {   // dW2 += (s*dout)^T h2 ; db2 += colsum(s*dout)
-        WgradArgs<T> w{};
-        w.dY = dout; w.lddy = C; w.X = static_cast<const T*>(f.h2); w.ldx = Ch;
-        w.dW = det ? dt.w2 : a->d_w2; w.db = det ? dt.b2 : a->d_b2; w.M = tokens; w.N = C; w.K = Ch;
-        w.tokens_per_image = tpi; w.dy_row_scale = dscale;
-        if constexpr (Act<T>::kIsBf16) {
-            WgradArgs<T> v = w;                  // DropPath-scaled rows: left by the GEMM above at C >= 128, made here otherwise
-            v.dY = dout_s; v.dy_row_scale = nullptr;
-            if (w.dy_row_scale && wgrad_tc_supported(v)) {
-                WinMap nomap{};
-                if (!dout_s_filled) BCK(launch_scale_gather_rows(dout, dout_s, dscale, tokens, C, C, 0, nomap, tpi, sms, st));
-                w = v;
-            }
-        }
-        BCK(launch_wgrad<T>(w, sms, det, st));
-    }
-    // depthwise conv backward: da1 = conv^T(dh2 * gelu'(a2)) * gelu'(a1); dWdw, dbdw
-    {
-        if (Act<T>::kIsBf16) BCK(launch_gelu_tab_init(st));
-        cudaError_t derr = cudaSuccess;
-        float* dw = det ? dt.w_dw : a->d_w_dw;
-        float* dbias = det ? dt.b_dw : a->d_b_dw;
-        const bool tiled = det ? launch_dwconv_bwd_tiled<T, true>(dh2, static_cast<const T*>(f.a2), static_cast<const T*>(f.h1),
-                                                                  static_cast<const T*>(f.a1), da1, da2, f.w_dw, dw, dbias, f.B, f.H,
-                                                                  f.W, Ch, sms, st, &derr)
-                               : launch_dwconv_bwd_tiled<T>(dh2, static_cast<const T*>(f.a2), static_cast<const T*>(f.h1),
-                                                            static_cast<const T*>(f.a1), da1, da2, f.w_dw, dw, dbias, f.B, f.H, f.W,
-                                                            Ch, sms, st, &derr);
-        if (tiled) {
-            BCK(derr);
-        } else {
-            BCK(launch_dwconv_bwd<T>(dh2, static_cast<const T*>(f.a2), static_cast<const T*>(f.h1), static_cast<const T*>(f.a1),
-                                     da1, f.w_dw, dw, dbias, f.B, f.H, f.W, Ch, sms, det, st));
-        }
-    }
-    {   // dW1 += da1^T LN2(y) ; db1 += colsum(da1)
-        WgradArgs<T> w{};
-        w.dY = da1; w.lddy = Ch; w.X = y; w.ldx = C;
-        w.dW = det ? dt.w1 : a->d_w1; w.db = det ? dt.b1 : a->d_b1; w.M = tokens; w.N = Ch; w.K = C;
-        w.tokens_per_image = tpi;
-        if (f.fused) { w.mean = mean; w.rstd = rstd; w.ln_w = f.ln_w; w.ln_b = f.ln_b; }
-        if constexpr (Act<T>::kIsBf16) {
-            // LN2(y) in one C-sized pass (into dz, free until the next GEMM writes it) -> plain operand for the tcgen05 kernel
-            WgradArgs<T> v = w;
-            v.X = dz; v.mean = nullptr; v.rstd = nullptr; v.ln_w = nullptr; v.ln_b = nullptr;
-            if (f.fused && wgrad_tc_supported(v)) {
-                WinMap nomap{};
-                BCK(launch_ln_apply(y, dz, f.ln_w, f.ln_b, tokens, C, 0, nomap, st));
-                w = v;
-            }
-        }
-        if (w.mean) BCK(launch_ln_stats<T>(y, tokens, C, mean, rstd, st));      // only the register-prologue kernels need them
-        BCK(launch_wgrad<T>(w, sms, det, st));
-    }
-    {   // dz = da1 . W1
-        GemmArgs<T> g{};
-        g.A = da1; g.lda = Ch; g.Wt = w1T; g.bias = nullptr;
-        g.Y = f.fused ? dz : static_cast<T*>(a->dy); g.ldy = C; g.M = tokens; g.N = C; g.K = Ch;
-        g.tokens_per_image = tpi;
-        BCK(launch_dgrad_gemm<T>(g, w1T_b, sms, st));
-    }
-    if (f.fused)   // dy = dout + LN2_bwd(dz)
-        BCK(launch_ln_bwd<T>(dz, y, dout, static_cast<T*>(a->dy), f.ln_w, det ? dt.ln_w : a->d_ln_w, det ? dt.ln_b : a->d_ln_b,
-                             tokens, C, sms, det, st));
-    if (det) BCK(dsl.reduce(st));
-    return 0;
+    return launch_gemm_any<T, EPI_BIAS>(g, sms, st);
 }
 
 }  // namespace lewin

@@ -777,49 +777,43 @@ cudaError_t launch_gemm_tc_stages(const GemmArgs<__nv_bfloat16>& g, cudaStream_t
     return cudaGetLastError();
 }
 
-inline int tc_num_sms() {
-    int dev = 0, n = 148;
-    if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev);
-    return n;
-}
-
 template <int BN, int KC, int EPI>
-cudaError_t launch_gemm_tc_inst(const GemmArgs<__nv_bfloat16>& g, cudaStream_t stream) {
+cudaError_t launch_gemm_tc_inst(const GemmArgs<__nv_bfloat16>& g, int num_sms, cudaStream_t stream) {
     if (g.M >= 4 * TC_BM) {
-        if (g.K == KC) return launch_gemm_tcp<BN, KC, 1, EPI>(g, tc_num_sms(), stream);
-        if (g.K == 2 * KC) return launch_gemm_tcp<BN, KC, 2, EPI>(g, tc_num_sms(), stream);
+        if (g.K == KC) return launch_gemm_tcp<BN, KC, 1, EPI>(g, num_sms, stream);
+        if (g.K == 2 * KC) return launch_gemm_tcp<BN, KC, 2, EPI>(g, num_sms, stream);
     }
     if (g.K == KC) return launch_gemm_tc_stages<BN, KC, EPI, 1>(g, stream);
     return launch_gemm_tc_stages<BN, KC, EPI, 2>(g, stream);
 }
 
 template <int KC, int EPI>
-cudaError_t launch_gemm_tc_kc(const GemmArgs<__nv_bfloat16>& g, cudaStream_t stream) {
+cudaError_t launch_gemm_tc_kc(const GemmArgs<__nv_bfloat16>& g, int num_sms, cudaStream_t stream) {
     const int N = g.N;
     // wide (192/256-column, 256-thread) tiles measured faster than 128-column / 128-thread tiles on every shape
-    if (N % 256 == 0) return launch_gemm_tc_inst<256, KC, EPI>(g, stream);
-    if (N % 192 == 0) return launch_gemm_tc_inst<192, KC, EPI>(g, stream);
-    if (N % 128 == 0) return launch_gemm_tc_inst<128, KC, EPI>(g, stream);
-    if (N % 96 == 0) return launch_gemm_tc_inst<96, KC, EPI>(g, stream);
-    if (N % 64 == 0) return launch_gemm_tc_inst<64, KC, EPI>(g, stream);
-    return launch_gemm_tc_inst<32, KC, EPI>(g, stream);
+    if (N % 256 == 0) return launch_gemm_tc_inst<256, KC, EPI>(g, num_sms, stream);
+    if (N % 192 == 0) return launch_gemm_tc_inst<192, KC, EPI>(g, num_sms, stream);
+    if (N % 128 == 0) return launch_gemm_tc_inst<128, KC, EPI>(g, num_sms, stream);
+    if (N % 96 == 0) return launch_gemm_tc_inst<96, KC, EPI>(g, num_sms, stream);
+    if (N % 64 == 0) return launch_gemm_tc_inst<64, KC, EPI>(g, num_sms, stream);
+    return launch_gemm_tc_inst<32, KC, EPI>(g, num_sms, stream);
 }
 
 // bf16 GEMM dispatch: tcgen05 path (N % 32 == 0, K % 32 == 0 always hold for LeWin shapes)
 template <int EPI>
-cudaError_t launch_gemm_tc(const GemmArgs<__nv_bfloat16>& g, cudaStream_t stream) {
-    if (g.K % 64 == 0) return launch_gemm_tc_kc<64, EPI>(g, stream);
-    return launch_gemm_tc_kc<32, EPI>(g, stream);
+cudaError_t launch_gemm_tc(const GemmArgs<__nv_bfloat16>& g, int num_sms, cudaStream_t stream) {
+    if (g.K % 64 == 0) return launch_gemm_tc_kc<64, EPI>(g, num_sms, stream);
+    return launch_gemm_tc_kc<32, EPI>(g, num_sms, stream);
 }
 
 // Dispatch used by the ABI: bf16 activations -> tcgen05 kernel; fp32 activations -> 3xTF32 on tcgen05 (gemm_t32.cuh) for
 // the forward shapes, the 3xTF32 mma.sync kernel otherwise
 template <typename T, int EPI>
-cudaError_t launch_gemm_any(const GemmArgs<T>& g, cudaStream_t stream) {
+cudaError_t launch_gemm_any(const GemmArgs<T>& g, int num_sms, cudaStream_t stream) {
     if constexpr (Act<T>::kIsBf16) {
-        return launch_gemm_tc<EPI>(g, stream);
+        return launch_gemm_tc<EPI>(g, num_sms, stream);
     } else {
-        if (gemm_t32_supported(g, EPI)) return gemm_t32_launch(g, EPI, stream);
+        if (gemm_t32_supported(g, EPI)) return gemm_t32_launch(g, EPI, num_sms, stream);
         return launch_gemm<EPI>(g, stream);
     }
 }

@@ -1,31 +1,11 @@
 // Translation unit of the implicit-GEMM projection convolutions (see conv_igemm.cuh): Downsample and OutputProj, bf16 inference.
 #define LEWIN_TU_LITE 1
-#include "../../include/lewin_b200.h"
+#include "abi_host.h"
 #include "conv_igemm.cuh"
 
 using namespace lewin;
 
 namespace {
-
-inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
-inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
-
-inline int device_sms(int* sms) {
-    int dev = 0, cc = 0;
-    cudaError_t e = cudaGetDevice(&dev);
-    if (e != cudaSuccess) return static_cast<int>(e);
-    e = cudaDeviceGetAttribute(sms, cudaDevAttrMultiProcessorCount, dev);
-    if (e != cudaSuccess) return static_cast<int>(e);
-    e = cudaDeviceGetAttribute(&cc, cudaDevAttrComputeCapabilityMajor, dev);
-    if (e != cudaSuccess) return static_cast<int>(e);
-    return cc == 10 ? 0 : LEWIN_E_ARCH;
-}
-
-#define CK(expr)                                         \
-    do {                                                 \
-        cudaError_t _e = (expr);                         \
-        if (_e != cudaSuccess) return static_cast<int>(_e); \
-    } while (0)
 
 inline cudaError_t prep(const float* w, __nv_bfloat16* wb, int n_real, int N, int C, int taps, cudaStream_t st) {
     const long long total = static_cast<long long>(taps) * N * C;
@@ -35,13 +15,19 @@ inline cudaError_t prep(const float* w, __nv_bfloat16* wb, int n_real, int N, in
     return cudaGetLastError();
 }
 
+// bf16 images of the weights: [16 taps][2 Cin][Cin] (downsample), [9 taps][Cout][Cin] (conv3x3 unless the caller gives w_bf16)
+__nv_bfloat16* downsample_layout(const LewinDownsampleArgs* a, WsLayout& L) {
+    return L.take<__nv_bfloat16>(static_cast<size_t>(16) * 2 * a->Cin * a->Cin * 2);
+}
+__nv_bfloat16* conv3x3_layout(const LewinConv3x3Args* a, WsLayout& L) {
+    return a->w_bf16 ? nullptr : L.take<__nv_bfloat16>(static_cast<size_t>(9) * a->Cout * a->Cin * 2);
+}
+
 }  // namespace
 
 extern "C" {
 
-size_t lewin_downsample_fwd_workspace_bytes(const LewinDownsampleArgs* a, int) {
-    return a ? align_up(static_cast<size_t>(16) * 2 * a->Cin * a->Cin * 2, 256) : 0;
-}
+size_t lewin_downsample_fwd_workspace_bytes(const LewinDownsampleArgs* a, int) { return a ? layout_bytes(downsample_layout, a) : 0; }
 
 int lewin_downsample_fwd_bf16(const LewinDownsampleArgs* a, void* ws, size_t ws_bytes, lewin_stream_t s) {
     cudaStream_t stream = reinterpret_cast<cudaStream_t>(s);
@@ -52,12 +38,10 @@ int lewin_downsample_fwd_bf16(const LewinDownsampleArgs* a, void* ws, size_t ws_
         ldx < Cin || ldx % 8 || ldo < N || ldo % 8)
         return LEWIN_E_SHAPE;
     if (!aligned16(a->x) || !aligned16(a->out)) return LEWIN_E_ALIGN;
+    WsLayout L;
+    __nv_bfloat16* wb = nullptr;
     int sms = 0;
-    if (int rc = device_sms(&sms)) return rc;
-    if (!ws || ws_bytes < lewin_downsample_fwd_workspace_bytes(a, LEWIN_DTYPE_BF16)) return LEWIN_E_WORKSPACE;
-    if (!aligned16(ws)) return LEWIN_E_ALIGN;
-    __nv_bfloat16* wb = static_cast<__nv_bfloat16*>(ws);
-    CK(prep(a->weight, wb, N, N, Cin, 16, stream));
+    if (int rc = enter(ws, ws_bytes, downsample_layout, a, L, wb, sms)) return rc;
 
     const int pad = a->pad_h ? 1 : 0;
     cv::Args k{};
@@ -85,15 +69,14 @@ int lewin_downsample_fwd_bf16(const LewinDownsampleArgs* a, void* ws, size_t ws_
                                       static_cast<unsigned long long>(a->H) * a->W * ld2};
     CUtensorMap amap{}, wmap{};
     if (!cv::make_5d(&amap, a->x, dims, st, KCH, 8, 16, KCH == 64) || !cv::make_w2d(&wmap, wb, 16ll * N, Cin, BN, KCH)) return LEWIN_E_SHAPE;
+    CK(prep(a->weight, wb, N, N, Cin, 16, stream));
     if (KCH == 32) { CK((cv::launch_inst<32, 64>(k, amap, wmap, sms, stream))); }
     else if (BN == 128) { CK((cv::launch_inst<64, 128>(k, amap, wmap, sms, stream))); }
     else { CK((cv::launch_inst<64, 256>(k, amap, wmap, sms, stream))); }
     return 0;
 }
 
-size_t lewin_conv3x3_fwd_workspace_bytes(const LewinConv3x3Args* a, int) {
-    return (a && !a->w_bf16) ? align_up(static_cast<size_t>(9) * a->Cout * a->Cin * 2, 256) : 0;
-}
+size_t lewin_conv3x3_fwd_workspace_bytes(const LewinConv3x3Args* a, int) { return a ? layout_bytes(conv3x3_layout, a) : 0; }
 
 int lewin_conv3x3_fwd_bf16(const LewinConv3x3Args* a, void* ws, size_t ws_bytes, lewin_stream_t s) {
     cudaStream_t stream = reinterpret_cast<cudaStream_t>(s);
@@ -103,15 +86,11 @@ int lewin_conv3x3_fwd_bf16(const LewinConv3x3Args* a, void* ws, size_t ws_bytes,
     if (a->B <= 0 || a->H < 1 || a->W < 8 || a->W % 8 || Cin % 64 || Cin > 512 || N % 64 || N > 512 || ldx < Cin || ldx % 8 || ldo < N || ldo % 8)
         return LEWIN_E_SHAPE;
     if (!aligned16(a->x) || !aligned16(a->out) || (a->w_bf16 && !aligned16(a->w_bf16))) return LEWIN_E_ALIGN;
+    WsLayout L;
+    __nv_bfloat16* w_img = nullptr;                   // the per-call image of `weight`, or null
     int sms = 0;
-    if (int rc = device_sms(&sms)) return rc;
-    const __nv_bfloat16* wb = static_cast<const __nv_bfloat16*>(a->w_bf16);
-    if (!wb) {
-        if (!ws || ws_bytes < lewin_conv3x3_fwd_workspace_bytes(a, LEWIN_DTYPE_BF16)) return LEWIN_E_WORKSPACE;
-        if (!aligned16(ws)) return LEWIN_E_ALIGN;
-        CK(prep(a->weight, static_cast<__nv_bfloat16*>(ws), N, N, Cin, 9, stream));
-        wb = static_cast<const __nv_bfloat16*>(ws);
-    }
+    if (int rc = enter(ws, ws_bytes, conv3x3_layout, a, L, w_img, sms)) return rc;
+    const __nv_bfloat16* wb = w_img ? w_img : static_cast<const __nv_bfloat16*>(a->w_bf16);
     cv::Args k{};
     k.B = a->B; k.Hout = a->H; k.Wout = a->W;
     k.N = N; k.n_real = N;
@@ -135,6 +114,7 @@ int lewin_conv3x3_fwd_bf16(const LewinConv3x3Args* a, void* ws, size_t ws_bytes,
                                       static_cast<unsigned long long>(a->H) * a->W * ld2};
     CUtensorMap amap{}, wmap{};
     if (!cv::make_5d(&amap, a->x, dims, st, 64, PX, PY, true) || !cv::make_w2d(&wmap, wb, 9ll * N, Cin, BN, 64)) return LEWIN_E_SHAPE;
+    if (w_img) CK(prep(a->weight, w_img, N, N, Cin, 9, stream));
     if (BN == 64) { CK((cv::launch_inst<64, 64>(k, amap, wmap, sms, stream))); }
     else if (BN == 128) { CK((cv::launch_inst<64, 128>(k, amap, wmap, sms, stream))); }
     else { CK((cv::launch_inst<64, 256>(k, amap, wmap, sms, stream))); }

@@ -5,21 +5,6 @@
 
 namespace lewin {
 
-namespace {
-int sm_count() {
-    static int cached[64] = {0};
-    int dev = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess) return 148;
-    int& c = cached[dev & 63];
-    if (c == 0) {
-        int n = 0;
-        if (cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || n <= 0) n = 148;
-        c = n;
-    }
-    return c;
-}
-}  // namespace
-
 bool gemm_t32_supported(const GemmArgs<float>& g, int epi) {
     if (epi == EPI_BIAS) return t32::supported<EPI_BIAS>(g);
     if (epi == EPI_BIAS_GELU) return t32::supported<EPI_BIAS_GELU>(g);
@@ -27,8 +12,7 @@ bool gemm_t32_supported(const GemmArgs<float>& g, int epi) {
     return false;
 }
 
-cudaError_t gemm_t32_launch(const GemmArgs<float>& g, int epi, cudaStream_t stream) {
-    const int sms = sm_count();
+cudaError_t gemm_t32_launch(const GemmArgs<float>& g, int epi, int sms, cudaStream_t stream) {
     if (epi == EPI_BIAS) return t32::launch<EPI_BIAS>(g, sms, stream);
     if (epi == EPI_BIAS_GELU) return t32::launch<EPI_BIAS_GELU>(g, sms, stream);
     if (epi == EPI_BIAS_RESID) return t32::launch<EPI_BIAS_RESID>(g, sms, stream);

@@ -13,6 +13,7 @@ from __future__ import annotations
 
 import threading
 import weakref
+from collections import namedtuple
 
 import torch
 
@@ -215,11 +216,30 @@ def _token_mask(token_mask, B, H, W, device):
     return tm
 
 
+# The tensors of an attention-half call as they cross the ABI, which its backward reads again: the fp32 parameters, the int32
+# sample indices, q|k|v, ctx, the selection and the token mask.
+AttnSaved = namedtuple("AttnSaved", "x ln_w ln_b w_qkv b_qkv w_out b_out rpb_table rpb_dense index_sample mask drop_scale qkv "
+                                    "ctx top token_mask")
+
+
+def _attn_args(geom, s, *, y, save):
+    """LewinAttnFwdArgs of a forward (y given) or backward (y = None) call on the tensors ``s`` (an AttnSaved)."""
+    B, H, W, nH, shift, windowed, use_rpb, analytic = geom[:8]
+    return _lib.LewinAttnFwdArgs(
+        B=B, H=H, W=W, C=s.x.shape[-1], nH=nH, shift=shift, windowed=int(windowed), use_rpb=int(use_rpb),
+        analytic_shift_mask=int(analytic), nW_mask=0 if s.mask is None else s.mask.shape[0],
+        save_for_backward=int(save), reserved=0,
+        x=_ptr(s.x), y=_ptr(y), ln_w=_ptr(s.ln_w), ln_b=_ptr(s.ln_b), w_qkv=_ptr(s.w_qkv), b_qkv=_ptr(s.b_qkv),
+        w_out=_ptr(s.w_out), b_out=_ptr(s.b_out), rpb_table=_ptr(s.rpb_table), rpb_dense=_ptr(s.rpb_dense),
+        index_sample=_ptr(s.index_sample), mask=_ptr(s.mask), drop_scale=_ptr(s.drop_scale),
+        qkv=_ptr(s.qkv), ctx=_ptr(s.ctx), top=_ptr(s.top), token_mask=_ptr(s.token_mask),
+        Bm=0 if s.token_mask is None else s.token_mask.shape[0])
+
+
 def _attn_forward(x, ln_w, ln_b, w_qkv, b_qkv, w_out, b_out, rpb_table, rpb_dense, index_sample, mask, drop_scale, geom,
                   token_mask=None):
-    """One lewin_attn_fwd_* call.  Returns (y, top, saved): ``saved`` is what the backward call needs (the fp32 parameter
-    tensors as they crossed the ABI, the int32 sample indices, q|k|v, ctx, top, the token mask).  Shared by the
-    autograd.Function below and the torch.library ops of compile_ops.py."""
+    """One lewin_attn_fwd_* call.  Returns (y, top, saved): ``saved`` is the AttnSaved the backward call needs.  Shared by
+    the autograd.Function below and the torch.library ops of compile_ops.py."""
     B, H, W, nH, shift, windowed, use_rpb, analytic, need_grad = geom[:9]
     band = geom[9] if len(geom) > 9 else None          # (y0, Hg): row band of a taller image (forward only)
     lib = _lib.load()
@@ -231,18 +251,11 @@ def _attn_forward(x, ln_w, ln_b, w_qkv, b_qkv, w_out, b_out, rpb_table, rpb_dens
     dev = x.device
     y = torch.empty_like(x)
     top = torch.empty((tokens // 64, nH, 25), dtype=torch.uint8, device=dev)
-    params = [_f32c(t) for t in (ln_w, ln_b, w_qkv, b_qkv, w_out, b_out, rpb_table, rpb_dense, mask, drop_scale)]
-    ln_w_, ln_b_, w_qkv_, b_qkv_, w_out_, b_out_, tab_, dense_, mask_, ds_ = params
-    idx = prepare_index_sample(index_sample, dev)
-    tm = _token_mask(token_mask, B, H, W, dev)
-    a = _lib.LewinAttnFwdArgs(
-        B=B, H=H, W=W, C=C, nH=nH, shift=shift, windowed=int(windowed), use_rpb=int(use_rpb),
-        analytic_shift_mask=int(analytic), nW_mask=0 if mask_ is None else mask_.shape[0],
-        save_for_backward=int(need_grad), reserved=0,
-        x=_ptr(x), y=_ptr(y), ln_w=_ptr(ln_w_), ln_b=_ptr(ln_b_), w_qkv=_ptr(w_qkv_), b_qkv=_ptr(b_qkv_),
-        w_out=_ptr(w_out_), b_out=_ptr(b_out_), rpb_table=_ptr(tab_), rpb_dense=_ptr(dense_),
-        index_sample=_ptr(idx), mask=_ptr(mask_), drop_scale=_ptr(ds_),
-        qkv=None, ctx=None, top=_ptr(top), token_mask=_ptr(tm), Bm=0 if tm is None else tm.shape[0])
+    ln_w_, ln_b_, w_qkv_, b_qkv_, w_out_, b_out_, tab_, dense_, mask_, ds_ = [
+        _f32c(t) for t in (ln_w, ln_b, w_qkv, b_qkv, w_out, b_out, rpb_table, rpb_dense, mask, drop_scale)]
+    s = AttnSaved(x, ln_w_, ln_b_, w_qkv_, b_qkv_, w_out_, b_out_, tab_, dense_, prepare_index_sample(index_sample, dev), mask_,
+                  ds_, None, None, top, _token_mask(token_mask, B, H, W, dev))
+    a = _attn_args(geom, s, y=y, save=need_grad)
     if band is not None:
         if need_grad:
             raise RuntimeError("lewin_b200.lewin_attn: row-band mode is forward only")
@@ -268,32 +281,23 @@ def _attn_forward(x, ln_w, ln_b, w_qkv, b_qkv, w_out, b_out, rpb_table, rpb_dens
         _lib.check(fn(a, ws.data_ptr(), ws.numel(), _stream()), f"lewin_attn_fwd_{dt}")
     if TopRecorder.active is not None:
         TopRecorder.active.tops.append(top)
-    return y, top, (x, ln_w_, ln_b_, w_qkv_, b_qkv_, w_out_, b_out_, tab_, dense_, idx, mask_, ds_, qkv, cbuf, top, tm)
+    return y, top, s._replace(qkv=qkv, ctx=cbuf)
 
 
 def _attn_backward(saved, geom, dy, separate_grads=False):
-    """One lewin_attn_bwd_* call on the tensors _attn_forward saved -> (dx, d_ln_w, d_ln_b, d_w_qkv, d_b_qkv, d_w_out, d_b_out,
+    """One lewin_attn_bwd_* call on the AttnSaved of the forward -> (dx, d_ln_w, d_ln_b, d_w_qkv, d_b_qkv, d_w_out, d_b_out,
     d_rpb_table, d_rpb_dense); entries of absent parameters are None."""
-    (x, ln_w, ln_b, w_qkv, b_qkv, w_out, b_out, tab, dense, idx, mask, ds, qkv, cbuf, top, tm) = saved
-    B, H, W, nH, shift, windowed, use_rpb, analytic, _ = geom[:9]
+    s = AttnSaved(*saved)
     lib = _lib.load()
-    dt = _dtype_tag(x)
-    dev = x.device
-    C = x.shape[-1]
+    dt = _dtype_tag(s.x)
+    dev = s.x.device
     dy = dy.contiguous()
-    dx = torch.empty_like(x)
+    dx = torch.empty_like(s.x)
     d_ln_w, d_ln_b, d_w_qkv, d_b_qkv, d_w_out, d_b_out, d_tab, d_dense = _zero_grads(
-        (ln_w, ln_b, w_qkv, b_qkv, w_out, b_out, tab, dense if tab is None else None), dev, separate_grads)
-    fwd = _lib.LewinAttnFwdArgs(
-        B=B, H=H, W=W, C=C, nH=nH, shift=shift, windowed=int(windowed), use_rpb=int(use_rpb),
-        analytic_shift_mask=int(analytic), nW_mask=0 if mask is None else mask.shape[0],
-        save_for_backward=1, reserved=0,
-        x=_ptr(x), y=None, ln_w=_ptr(ln_w), ln_b=_ptr(ln_b), w_qkv=_ptr(w_qkv), b_qkv=_ptr(b_qkv),
-        w_out=_ptr(w_out), b_out=_ptr(b_out), rpb_table=_ptr(tab), rpb_dense=_ptr(dense),
-        index_sample=_ptr(idx), mask=_ptr(mask), drop_scale=_ptr(ds),
-        qkv=_ptr(qkv), ctx=_ptr(cbuf), top=_ptr(top), token_mask=_ptr(tm), Bm=0 if tm is None else tm.shape[0])
+        (s.ln_w, s.ln_b, s.w_qkv, s.b_qkv, s.w_out, s.b_out, s.rpb_table, s.rpb_dense if s.rpb_table is None else None), dev,
+        separate_grads)
     a = _lib.LewinAttnBwdArgs(
-        fwd=fwd, dy=_ptr(dy), dx=_ptr(dx), d_ln_w=_ptr(d_ln_w), d_ln_b=_ptr(d_ln_b),
+        fwd=_attn_args(geom, s, y=None, save=True), dy=_ptr(dy), dx=_ptr(dx), d_ln_w=_ptr(d_ln_w), d_ln_b=_ptr(d_ln_b),
         d_w_qkv=_ptr(d_w_qkv), d_b_qkv=_ptr(d_b_qkv), d_w_out=_ptr(d_w_out), d_b_out=_ptr(d_b_out),
         d_rpb_table=_ptr(d_tab), d_rpb_dense=_ptr(d_dense), deterministic=_deterministic())
     ws = _workspace(lib.lewin_attn_bwd_workspace_bytes(a, _lib.DTYPE_TAG[dt]), dev)
@@ -321,9 +325,24 @@ class _AttnFn(torch.autograd.Function):
         return _attn_backward(ctx.saved_tensors, ctx.geom, dy) + (None, None, None, None, None)
 
 
+# The tensors of a LeFF-half call as they cross the ABI, which its backward reads again: the fp32 parameters, the hidden
+# activations h1 / h2 and the pre-activations a1 / a2.
+LeffSaved = namedtuple("LeffSaved", "y ln_w ln_b w1 b1 w_dw b_dw w2 b2 drop_scale h1 h2 a1 a2")
+
+
+def _leff_args(geom, s, *, out, save):
+    """LewinLeffFwdArgs of a forward (out given) or backward (out = None) call on the tensors ``s`` (a LeffSaved)."""
+    B, H, W, fused = geom[:4]
+    return _lib.LewinLeffFwdArgs(
+        B=B, H=H, W=W, C=s.y.shape[-1], hidden=s.w1.shape[0], fused=int(fused), save_for_backward=int(save), ld_out=0,
+        y=_ptr(s.y), out=_ptr(out), ln_w=_ptr(s.ln_w), ln_b=_ptr(s.ln_b), w1=_ptr(s.w1), b1=_ptr(s.b1),
+        w_dw=_ptr(s.w_dw), b_dw=_ptr(s.b_dw), w2=_ptr(s.w2), b2=_ptr(s.b2), drop_scale=_ptr(s.drop_scale),
+        h1=_ptr(s.h1), h2=_ptr(s.h2), a1=_ptr(s.a1), a2=_ptr(s.a2))
+
+
 def _leff_forward(y, ln_w, ln_b, w1, b1, w_dw, b_dw, w2, b2, drop_scale, geom, out_view=None):
-    """One lewin_leff_fwd_* call.  Returns (out, saved): ``saved`` (None for an inference call) is what the backward call needs.
-    Shared by the autograd.Function below and the torch.library ops of compile_ops.py."""
+    """One lewin_leff_fwd_* call.  Returns (out, saved): ``saved`` (None for an inference call) is the LeffSaved the backward
+    call needs.  Shared by the autograd.Function below and the torch.library ops of compile_ops.py."""
     B, H, W, fused, need_grad = geom
     lib = _lib.load()
     dt = _dtype_tag(y)
@@ -338,14 +357,10 @@ def _leff_forward(y, ln_w, ln_b, w1, b1, w_dw, b_dw, w2, b2, drop_scale, geom, o
     h2 = h1                       # placeholder until the library says whether h2 exists in global memory for this call
     a1 = torch.empty_like(h1) if need_grad else None
     a2 = torch.empty_like(h1) if need_grad else None
-    ln_w_, ln_b_, w1_, b1_, wdw_, bdw_, w2_, b2_, ds_ = [_f32c(t) for t in (ln_w, ln_b, w1, b1, w_dw, b_dw, w2, b2, drop_scale)]
-    a = _lib.LewinLeffFwdArgs(
-        B=B, H=H, W=W, C=C, hidden=hidden, fused=int(fused), save_for_backward=int(need_grad), ld_out=0,
-        y=_ptr(y), out=_ptr(out), ln_w=_ptr(ln_w_), ln_b=_ptr(ln_b_), w1=_ptr(w1_), b1=_ptr(b1_),
-        w_dw=_ptr(wdw_), b_dw=_ptr(bdw_), w2=_ptr(w2_), b2=_ptr(b2_), drop_scale=_ptr(ds_),
-        h1=_ptr(h1), h2=_ptr(h2), a1=_ptr(a1), a2=_ptr(a2))
+    s = LeffSaved(y, *[_f32c(t) for t in (ln_w, ln_b, w1, b1, w_dw, b_dw, w2, b2, drop_scale)], h1, h2, a1, a2)
+    a = _leff_args(geom, s, out=out, save=need_grad)
     if dt == "bf16" and C >= 256 and not need_grad:
-        w1_b, w2_b = _bf16_image(w1_), _bf16_image(w2_)
+        w1_b, w2_b = _bf16_image(s.w1), _bf16_image(s.w2)
         a.w1_bf16, a.w2_bf16 = _ptr(w1_b), _ptr(w2_b)
     if out_view is not None and not need_grad and lib.lewin_leff_fwd_supports_ld_out(a, _lib.DTYPE_TAG[dt]):
         # the caller's column block of a wider buffer (the right half of the decoder's concat buffer): written in place
@@ -363,29 +378,22 @@ def _leff_forward(y, ln_w, ln_b, w1, b1, w_dw, b_dw, w2, b2, drop_scale, geom, o
     fn = getattr(lib, f"lewin_leff_fwd_{dt}")
     with torch.cuda.device(dev):
         _lib.check(fn(a, ws.data_ptr(), ws.numel(), _stream()), f"lewin_leff_fwd_{dt}")
-    return out, ((y, ln_w_, ln_b_, w1_, b1_, wdw_, bdw_, w2_, b2_, ds_, h1, h2, a1, a2) if need_grad else None)
+    return out, (s._replace(h2=h2) if need_grad else None)
 
 
 def _leff_backward(saved, geom, dout, separate_grads=False):
-    """One lewin_leff_bwd_* call on the tensors _leff_forward saved -> (dy, d_ln_w, d_ln_b, d_w1, d_b1, d_w_dw, d_b_dw, d_w2,
+    """One lewin_leff_bwd_* call on the LeffSaved of the forward -> (dy, d_ln_w, d_ln_b, d_w1, d_b1, d_w_dw, d_b_dw, d_w2,
     d_b2); entries of absent parameters are None."""
-    (y, ln_w, ln_b, w1, b1, wdw, bdw, w2, b2, ds, h1, h2, a1, a2) = saved
-    B, H, W, fused, _ = geom
+    s = LeffSaved(*saved)
     lib = _lib.load()
-    dt = _dtype_tag(y)
-    dev = y.device
-    C = y.shape[-1]
-    hidden = w1.shape[0]
+    dt = _dtype_tag(s.y)
+    dev = s.y.device
     dout = dout.contiguous()
-    dy = torch.empty_like(y)
-    d_ln_w, d_ln_b, d_w1, d_b1, d_wdw, d_bdw, d_w2, d_b2 = _zero_grads((ln_w, ln_b, w1, b1, wdw, bdw, w2, b2), dev, separate_grads)
-    fwd = _lib.LewinLeffFwdArgs(
-        B=B, H=H, W=W, C=C, hidden=hidden, fused=int(fused), save_for_backward=1, ld_out=0,
-        y=_ptr(y), out=None, ln_w=_ptr(ln_w), ln_b=_ptr(ln_b), w1=_ptr(w1), b1=_ptr(b1),
-        w_dw=_ptr(wdw), b_dw=_ptr(bdw), w2=_ptr(w2), b2=_ptr(b2), drop_scale=_ptr(ds),
-        h1=_ptr(h1), h2=_ptr(h2), a1=_ptr(a1), a2=_ptr(a2))
+    dy = torch.empty_like(s.y)
+    d_ln_w, d_ln_b, d_w1, d_b1, d_wdw, d_bdw, d_w2, d_b2 = _zero_grads(
+        (s.ln_w, s.ln_b, s.w1, s.b1, s.w_dw, s.b_dw, s.w2, s.b2), dev, separate_grads)
     a = _lib.LewinLeffBwdArgs(
-        fwd=fwd, dout=_ptr(dout), dy=_ptr(dy), d_ln_w=_ptr(d_ln_w), d_ln_b=_ptr(d_ln_b),
+        fwd=_leff_args(geom, s, out=None, save=True), dout=_ptr(dout), dy=_ptr(dy), d_ln_w=_ptr(d_ln_w), d_ln_b=_ptr(d_ln_b),
         d_w1=_ptr(d_w1), d_b1=_ptr(d_b1), d_w_dw=_ptr(d_wdw), d_b_dw=_ptr(d_bdw), d_w2=_ptr(d_w2), d_b2=_ptr(d_b2),
         deterministic=_deterministic())
     ws = _workspace(lib.lewin_leff_bwd_workspace_bytes(a, _lib.DTYPE_TAG[dt]), dev)
@@ -454,6 +462,15 @@ def lewin_leff(y, *, B, H, W, ln_w, ln_b, w1, b1, w_dw, b_dw, w2, b2, drop_scale
     return _LeffFn.apply(y, ln_w, ln_b, w1, b1, w_dw, b_dw, w2, b2, drop_scale, geom, out)
 
 
+def _core_args(geom, qkv, ctx, rpb_table, rpb_dense, index_sample, mask, top):
+    """LewinCoreFwdArgs of a core-only forward or backward call (qkv [B_, 64, 3C], head_dim = C / nH)."""
+    nH, use_rpb = geom
+    return _lib.LewinCoreFwdArgs(B_=qkv.shape[0], nH=nH, use_rpb=int(use_rpb), nW_mask=0 if mask is None else mask.shape[0],
+                                 head_dim=qkv.shape[-1] // 3 // nH, reserved=0,
+                                 qkv=_ptr(qkv), ctx=_ptr(ctx), rpb_table=_ptr(rpb_table), rpb_dense=_ptr(rpb_dense),
+                                 index_sample=_ptr(index_sample), mask=_ptr(mask), top=_ptr(top))
+
+
 class _CoreFn(torch.autograd.Function):
     """ProbAttention.forward (attn.py:287-342) on projected q|k|v; backward = lewin_probsparse_core_bwd_* for the saved selection."""
 
@@ -471,11 +488,8 @@ class _CoreFn(torch.autograd.Function):
         out = torch.empty((B_, L, C), dtype=qkv.dtype, device=dev)
         top = torch.empty((B_, nH, 25), dtype=torch.uint8, device=dev)
         tab_, dense_, mask_ = _f32c(rpb_table), _f32c(rpb_dense), _f32c(mask)
-        idx = prepare_index_sample(index_sample, dev)
-        a = _lib.LewinCoreFwdArgs(B_=B_, nH=nH, use_rpb=int(use_rpb), nW_mask=0 if mask_ is None else mask_.shape[0],
-                                  head_dim=C // nH, reserved=0,
-                                  qkv=_ptr(qkv), ctx=_ptr(out), rpb_table=_ptr(tab_), rpb_dense=_ptr(dense_),
-                                  index_sample=_ptr(idx), mask=_ptr(mask_), top=_ptr(top))
+        idx = prepare_index_sample(index_sample, dev)          # alive until the call: the struct holds only its address
+        a = _core_args(geom, qkv, out, tab_, dense_, idx, mask_, top)
         ws = _workspace(lib.lewin_probsparse_core_fwd_workspace_bytes(a, _lib.DTYPE_TAG[dt]), dev)
         fn = getattr(lib, f"lewin_probsparse_core_fwd_{dt}")
         with torch.cuda.device(dev):
@@ -488,19 +502,14 @@ class _CoreFn(torch.autograd.Function):
     @staticmethod
     def backward(ctx, dctx, _dtop):
         qkv, tab, dense, mask, top = ctx.saved_tensors
-        nH, use_rpb = ctx.geom
         lib = _lib.load()
         dt = ctx.dt
         dev = qkv.device
-        B_, L, C3 = qkv.shape
         dctx = dctx.contiguous()
         dqkv = torch.empty_like(qkv)
         d_tab, d_dense = _zero_grads((tab, dense if tab is None else None), dev)
-        fwd = _lib.LewinCoreFwdArgs(B_=B_, nH=nH, use_rpb=int(use_rpb), nW_mask=0 if mask is None else mask.shape[0],
-                                    head_dim=C3 // 3 // nH, reserved=0,
-                                    qkv=_ptr(qkv), ctx=_ptr(dctx), rpb_table=_ptr(tab), rpb_dense=_ptr(dense),
-                                    index_sample=None, mask=_ptr(mask), top=_ptr(top))
-        a = _lib.LewinCoreBwdArgs(fwd=fwd, dctx=_ptr(dctx), dqkv=_ptr(dqkv), d_rpb_table=_ptr(d_tab), d_rpb_dense=_ptr(d_dense),
+        a = _lib.LewinCoreBwdArgs(fwd=_core_args(ctx.geom, qkv, dctx, tab, dense, None, mask, top), dctx=_ptr(dctx),
+                                  dqkv=_ptr(dqkv), d_rpb_table=_ptr(d_tab), d_rpb_dense=_ptr(d_dense),
                                   deterministic=_deterministic())
         ws = _workspace(lib.lewin_probsparse_core_bwd_workspace_bytes(a, _lib.DTYPE_TAG[dt]), dev)
         fn = getattr(lib, f"lewin_probsparse_core_bwd_{dt}")
